@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (N > 1: launched under torchrun)
     python bench.py --impl reference --gpus N --steps K --warmup W
+    python bench.py --steps K --warmup W --dump-outputs DIR  (also writes the result records of the last timed step)
 
 Headline workload (BASELINE.json `metric`, configs[4] at its per-GPU share): the full VAD -> KWS -> S2I gated cascade
 (nnCntrlClass_exec, evb/src/nnCntrlClass.c:152-272) over 8,192 independent synthetic 16 kHz streams per GPU -- 65,536 at
@@ -11,18 +12,23 @@ N = 8 -- one step = 100 frames (1.0 s of audio) of every stream. The single-mode
 `configs` block of the same line.
 
 One JSON line on stdout (rank 0):
-  value         audio-seconds per second, PCM already resident in HBM; K steps timed with CUDA events on the engine's
-                stream, repeated until the timed regions add up to >= 0.5 s, median repetition, MAX over ranks
+  value         audio-seconds per second, PCM already resident in HBM; exactly K steps (after W warm-up steps, W raised to
+                at least 3) timed with CUDA events on the engine's stream, MAX over ranks
   e2e           the same metric through the C ABI call with HOST (pinned) buffers: H2D + kernels + D2H inside
   roofline      the dominant kernel (feat_kernel) against the resource that binds it (issue slots), the HBM line next to it
   cpu_baseline  the reference's own C (oracle/_ref, unmodified sources, gcc -O2) on this host's cores, same PCM, same
                 controller state per stream carried from step to step
   bit_exact_frame_pct   result records of a stream sample against that reference, taken outside the timed region
+
+--dump-outputs DIR writes what the headline path returned to its caller in the last timed step: every field of the
+[streams, frames] cascade result records of rank 0 (the only rank when N = 1) as DIR/<field>.npy in float32 (exact for
+these integer fields, 23 MB in all).
+The PCM is synthesised from fixed seeds and every step count is fixed by the arguments, so two builds run with the same
+arguments can be compared output for output.
 """
 import argparse
 import hashlib
 import json
-import math
 import multiprocessing as mp
 import os
 import subprocess
@@ -39,7 +45,6 @@ FRAME = 160
 FRAMES_PER_STEP = 100
 AUDIO_S_PER_FRAME = FRAME / 16000.0
 CASCADE_STREAMS_PER_GPU = 8192                   # 65,536 / 8: BASELINE.json configs[4]
-MIN_TIMED_S = 0.5
 MODEL_FILE = {0: "s2i.nnspm", 1: "vad.nnspm", 2: "kws_galaxy.nnspm"}
 # SURVEY.md section 8(d), algorithmic bytes per stream-frame of the whole path (one-frame-per-launch design):
 #   S2I 2 872, KWS 2 824, VAD 2 608; the cascade adds the PCM ring (write 320 + look-back read 320) to the S2I figure
@@ -284,8 +289,8 @@ def run_reference_arm(args, rank):
 
 # ---------------------------------------------------------------------------------------------
 class Timer:
-    """K steps between two CUDA events on the handle's stream, a barrier + synchronize on both sides; repeated until the
-    timed regions add up to MIN_TIMED_S; the time of a repetition is the MAX over ranks, the result their median."""
+    """W warm-up steps (W >= 3, see main), then exactly K steps between two CUDA events on the handle's stream, a barrier + synchronize on
+    both sides; the time is the MAX over ranks."""
 
     def __init__(self, nb, device, dist):
         self.nb, self.device, self.dist = nb, device, dist
@@ -315,25 +320,27 @@ class Timer:
         h.sync()
         return self.ev0.elapsed_ms_to(self.ev1)
 
-    def run(self, h, step, K, W, min_s=MIN_TIMED_S):
+    def run(self, h, step, K, W):
         for i in range(W):
             step(i)
-        first = self.allmax([self.once(h, step, K)])[0]
-        reps = int(min(200, max(1, math.ceil(min_s * 1e3 / max(first, 1e-3)))))
-        times = [first] + self.allmax([self.once(h, step, K) for _ in range(reps - 1)])
-        return float(np.median(times)), times
+        return self.allmax([self.once(h, step, K)])[0]
 
 
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=20)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--warmup", type=int, default=3, help="untimed steps before each timed region (at least 3 for the b200 implementation)")
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-side-configs", action="store_true")
-    ap.add_argument("--min-timed-s", type=float, default=MIN_TIMED_S, help="repeat the K-step timed region until it adds up to this (profiler runs: 0)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the cascade results of the last timed step as DIR/<field>.npy "
+                    "(b200 implementation only; under torchrun rank 0's streams only)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the results of the b200 implementation; the reference arm only times its steps")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -418,8 +425,14 @@ def main():
 
     sampler = ClockSampler(device)
     sampler.start()
-    ms_total, rep_times = tm.run(casc, step, K, W, min_s=args.min_timed_s)
+    ms_total = tm.run(casc, step, K, W)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:                  # dev_res holds the last timed step's records until the next step
+        last = dev_res.to_host()
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for f in last.dtype.names:
+            np.save(os.path.join(args.dump_outputs, f + ".npy"), last[f].astype(np.float32))
+        del last
     km = []
     for i in range(5):                                  # per-kernel durations: CUDA events the engine records around its launches
         step(i)
@@ -459,10 +472,7 @@ def main():
     e2e_loop(3)
     sampler = ClockSampler(device)
     sampler.start()
-    first = tm.allmax([e2e_once()])[0]
-    e2e_reps = int(min(50, max(1, math.ceil(args.min_timed_s / max(first, 1e-6)))))
-    e2e_times = [first] + tm.allmax([e2e_once() for _ in range(e2e_reps - 1)])
-    e2e_s = float(np.median(e2e_times))
+    e2e_s = tm.allmax([e2e_once()])[0]
     clocks_e2e = sampler.stop()
     clocks["e2e"] = {k: clocks_e2e[k] for k in ("sm_mhz", "reasons", "samples")}
     clocks["reasons"] = sorted(set(clocks["reasons"]) | set(clocks_e2e["reasons"]))
@@ -503,7 +513,7 @@ def main():
             res = nb.DeviceArray((Sg, T), nb.RESULT_DT, device)
             fn = lambda i: b.exec_device(d[i & 1], T * FRAME, T, res)
             tc0, kl0 = nb.tc5_launches(), nb.kernel_launches()
-            ms, _ = tm.run(b, fn, K, W, min_s=min(0.25, args.min_timed_s))
+            ms = tm.run(b, fn, K, W)
             tc5_share = (nb.tc5_launches() - tc0, nb.kernel_launches() - kl0)
             kk = []
             for i in range(3):
@@ -558,14 +568,13 @@ def main():
             "metric": METRIC, "value": value, "unit": "audio-s/s", "n_gpus": world, "steps": K, "warmup": W,
             "ms_per_step": ms_total / K, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
             "dtype": DTYPE, "data": "synthetic", "config": workload_config(world),
-            "timing": {"repetitions": len(rep_times), "timed_region_s": sum(rep_times) * 1e-3, "ms_per_repetition_median": ms_total,
-                       "ms_per_repetition_min": min(rep_times), "ms_per_repetition_max": max(rep_times),
-                       "rule": "each repetition = exactly `steps` steps between CUDA events, barrier + synchronize on both sides, "
-                               "MAX over ranks; value from the median repetition"},
+            "timing": {"timed_steps": K, "timed_region_s": ms_total * 1e-3,
+                       "rule": "`warmup` steps, then exactly `steps` steps between CUDA events, barrier + synchronize on both "
+                               "sides, MAX over ranks"},
             "bit_exact_frame_pct": bit_exact["pct"] if bit_exact else None, "bit_exact": bit_exact,
             "stage_frames_last_step": {"s2i": stage[0], "vad": stage[1], "kws": stage[2]},
             "e2e": {"value": audio_s / e2e_s, "unit": "audio-s/s", "h2d_bytes_per_step": h2d_bytes, "d2h_bytes_per_step": d2h_bytes,
-                    "ms_per_step": 1e3 * e2e_s / K, "repetitions": len(e2e_times), "timed_region_s": sum(e2e_times),
+                    "ms_per_step": 1e3 * e2e_s / K, "timed_region_s": e2e_s,
                     "call": "nnsp_b200_cascade_exec_host_async + _wait_host, two pinned buffer pairs, results of every step read on the host",
                     "blocking_call_value": (audio_s / world) / e2e_sync_s if world == 1 else None,
                     "link_gbs": link_gbs, "link_frac": (h2d_bytes * K / e2e_s / 1e9) / link_gbs,
