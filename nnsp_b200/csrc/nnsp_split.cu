@@ -1090,6 +1090,21 @@ __global__ void __launch_bounds__(256) vseq_kernel(VseqArgs a)
     }
 }
 
+/* debug tap of a tcgen05 layer 0 (batched NNSPClass): its int16 outputs back from the byte planes it wrote, decoded like
+ * the tap of seg_kernel. Runs right behind seg0_tc5_kernel, before anything reuses that plane buffer. */
+__global__ void tc5_tap_kernel(const uint8_t *planes, long long tile_bytes, int pa, int tile0, int s0, int ns, int T,
+                               int first, int n_inf, int H, int act_stride, int16_t *tap_act)
+{
+    const long long n = (long long)ns * n_inf * H;
+    for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+        const int u = (int)(i % H);
+        const long long pk = i / H;
+        const int k = (int)(pk % n_inf), p = (int)(pk / n_inf);
+        const uint8_t *x = planes + (size_t)(tile0 + (p >> 4)) * (size_t)tile_bytes + (size_t)k * 32 * pa + (p & 15) * pa + u;
+        tap_act[((long long)(s0 + p) * T + first + 2 * k) * act_stride + u] = (int16_t)(((int)(int8_t)x[0] << 8) | x[16 * pa]);
+    }
+}
+
 static bool tc5_wanted(int n_inf)
 {
     const char *e = getenv("NNSP_B200_TC5");
@@ -1131,8 +1146,9 @@ int launch_split_layers(const MmaDeviceModel &mm, const SplitGroup &q, int devic
         int l1 = li;
         while (l1 < D->numlayers && D->layer[l1].type == LAYER_FC) l1++;
         const bool tc5_batch = q.mode == 1 && !q.list && !q.tstart;                       /* the batched NNSPClass */
-        const bool tc5_round = q.mode == 2 && q.list && q.tstart && q.vseq;                /* first round of the cascade */
-        if (l1 > li && from_feat && l1 == 1 && (tc5_batch || tc5_round) && mm.tc5 && D->pa <= TC5_PAMAX && !tp.act && tc5_wanted(q.n_inf)) {
+        const bool tc5_round = q.mode == 2 && q.list && q.tstart && q.vseq && !tp.act;     /* first round of the cascade (never tapped: cascade_use_split) */
+        /* a tapped batch call takes the same layer-0 kernel as an untapped one: tc5_tap_kernel reads its outputs back */
+        if (l1 > li && from_feat && l1 == 1 && (tc5_batch || tc5_round) && mm.tc5 && D->pa <= TC5_PAMAX && tc5_wanted(q.n_inf)) {
             /* layer 0 on the tcgen05 tensor cores (nnsp_tc5.cuh) */
             if (tc5_round) {
                 VseqArgs v{};
@@ -1157,6 +1173,13 @@ int launch_split_layers(const MmaDeviceModel &mm, const SplitGroup &q, int devic
             seg0_tc5_kernel<<<grid, TC5_THREADS, sizeof(Tc5Smem) + 1024, st>>>(a);
             NNSP_LAUNCH_CHECK();
             g_tc5_launches.fetch_add(1, std::memory_order_relaxed);
+            if (tp.act) {
+                const long long n = (long long)q.ns * q.n_inf * D->layer[0].rows;
+                const int tgrid = (int)((n + 255) / 256 < 4 * sm_count(device) ? (n + 255) / 256 : 4 * sm_count(device));
+                tc5_tap_kernel<<<tgrid, 256, 0, st>>>(bufs[which], tile_bytes, D->pa, q.tile0, q.s0, q.ns, q.T, q.first, q.n_inf,
+                                                      D->layer[0].rows, D->act_stride, tp.act);
+                NNSP_LAUNCH_CHECK();
+            }
             ao += D->layer[0].rows;
             cur_in = bufs[which]; which ^= 1;
             from_feat = false;

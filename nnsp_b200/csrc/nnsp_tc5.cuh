@@ -23,10 +23,11 @@
  *   4 conversion warps (TMA bulk copies of the raw int16 rows through a 4-deep ring -> byte planes in entry layout), 1 warp
  *   whose lane 0 issues the MMAs -- its own warp because the issue of a queued tcgen05.mma blocks, which would stall the
  *   conversion behind it. Three A buffers / TMEM stages in flight.
- * Eligibility (launch_split_layers): a range selection (the batched NNSPClass; the cascade's rounds keep seg_kernel<2>),
- * layer 0 = fc 240 -> rows <= 80 with tanh and the exact 32-bit finish, followed by an LSTM, no activation tap,
- * and at least 45 % of the tiles' inference slots in use (tc5_wanted, nnsp_split.cu). NNSP_B200_TC5=0 keeps the mma.sync
- * kernel, =2 takes this one whenever the layer qualifies. */
+ * Eligibility (launch_split_layers): a range selection (the batched NNSPClass; the cascade's first round only under
+ * NNSP_B200_TC5=2, through vseq_kernel), layer 0 = fc 240 -> rows <= 80 with tanh and the exact 32-bit finish, followed by
+ * an LSTM, and at least 45 % of the tiles' inference slots in use (tc5_wanted, nnsp_split.cu). Taps do not change the
+ * choice: with an activation tap, tc5_tap_kernel decodes the output planes into it right after this kernel.
+ * NNSP_B200_TC5=0 keeps the mma.sync kernel, =2 takes this one whenever the layer qualifies. */
 #pragma once
 
 namespace nnsp {

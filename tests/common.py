@@ -87,6 +87,15 @@ NET_CRAFTED = [
     ("all_p127", 2, (240, 32, 32, 2), (0, 1, 0), (2, 1, 3), (7, 5, 7), (8, 15, 15), (14, 13, 15), 127),
     ("all_m128_q0", 0, (240, 40, 40, 41), (0, 1, 0), (1, 1, 3), (0, 0, 0), (8, 15, 15), (15, 15, 15), -128),   # qs = 15: no output shift
 ]
+# stacks the tcgen05 layer 0 takes (tanh fc 240 -> <= 80, exact 32-bit finish, an LSTM behind it) whose standardisation
+# saturates: Q15 feature rows (feat_rshift 15) with the header's random means and stdR put most feature values at -32768
+# or 32767, so the hi / lo byte split reaches hi = -128 and hi = 127, lo = 255; every weight -128 / +127 or random.
+#   ..., fill (None = random weights)
+NET_TC5_SATURATING = [
+    ("sat_feat_m128", 2, (240, 32, 32, 2), (0, 1, 0), (1, 1, 3), (7, 5, 7), (15, 15, 15), (14, 13, 15), -128),
+    ("sat_feat_p127", 2, (240, 32, 32, 2), (0, 1, 0), (1, 1, 3), (7, 5, 7), (15, 15, 15), (14, 13, 15), 127),
+    ("sat_feat_random", 1, (240, 24, 16, 2), (0, 1, 0), (1, 1, 3), (7, 6, 7), (15, 15, 15), (14, 13, 15), None),
+]
 
 
 def net_case_blob(case, acc32):

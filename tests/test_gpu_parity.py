@@ -39,15 +39,20 @@ def test_feature_stages_bit_exact(nb, oracle):
             assert (out[k][i] == ref[k]).all(), "stage %s differs for window %d" % (k, i)
 
 
-@pytest.mark.parametrize("path", ["split", "imma", "dp2a"])
+@pytest.mark.parametrize("path", ["split", "split_tc5", "imma", "dp2a"])
 @pytest.mark.parametrize("nn_id,acc32", [(1, False), (2, True), (0, False), (0, True), (1, True), (2, False)])
-def test_batch_matches_oracle_every_tap(nb, oracle, nn_id, acc32, path):
-    """All network paths: scan-split (default), tensor-core IMMA in the time loop, dp2a warp per stream."""
+def test_batch_matches_oracle_every_tap(nb, oracle, monkeypatch, nn_id, acc32, path):
+    """All network paths: scan-split (default) with layer 0 on the mma.sync kernel seg_kernel<feat> (NNSP_B200_TC5=0) and
+    on the tcgen05 kernel (=2), tensor-core IMMA in the time loop, dp2a warp per stream."""
     S, T = 53, 64                      # 53: a partial 16-stream tile at the end
+    if path.startswith("split"):
+        monkeypatch.setenv("NNSP_B200_TC5", "2" if path == "split_tc5" else "0")
     pcm = nb.synth_pcm(S, T)
     m = _model(nb, nn_id, acc32)
-    b = nb.NNSPBatch(m, S, nn_path=path)
+    b = nb.NNSPBatch(m, S, nn_path=path.split("_")[0])
+    n0 = nb.tc5_launches()
     res, taps = b.exec(pcm, taps=True)
+    assert nb.tc5_launches() - n0 == (1 if path == "split_tc5" else 0)       # which layer-0 kernel ran
     m_or = oracle.model(nn_id, acc32)
     for s in range(S):
         _compare_stream(oracle, m_or, pcm[s], res[s], taps, s)
