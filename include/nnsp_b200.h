@@ -61,6 +61,12 @@ const char *nnsp_b200_last_error(void);
 long long nnsp_b200_kernel_launches(void);
 /* how many of them were the tcgen05 (5th-generation tensor core) layer-0 kernel of the batched network path */
 long long nnsp_b200_tc5_launches(void);
+/* how many of them were the cascade's per-stream network kernels, by kind: 0 the sequential kernel in its narrow shape
+ * (every layer at most 80 wide, LSTM state at most 80, at most 48 outputs), 1 the sequential kernel in its wide shape,
+ * 2 the two-warps-per-stream replay kernel behind the stage-sorted rounds (-1 for any other kind). Launches, not work:
+ * after the stage-sorted rounds the replay (kind 2, or kind 0 / 1 when the replay kernel is not used) is launched once
+ * per call and returns at once when no stream is left for it. */
+long long nnsp_b200_cascade_kernel_launches(int kind);
 
 /* ------------------------------------------------------------------------------------ */
 /* Models                                                                               */

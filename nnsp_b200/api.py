@@ -559,3 +559,12 @@ def kernel_launches():
 
 def tc5_launches():
     return lib().nnsp_b200_tc5_launches()
+
+
+CASCADE_KERNELS = ("narrow", "wide", "replay")
+
+
+def cascade_kernel_launches():
+    """launches of the cascade's per-stream network kernels so far: {"narrow": cascade_kernel<CsNarrow>, "wide":
+    cascade_kernel<CsWide>, "replay": cascade_replay_kernel}"""
+    return {k: lib().nnsp_b200_cascade_kernel_launches(i) for i, k in enumerate(CASCADE_KERNELS)}

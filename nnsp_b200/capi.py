@@ -35,7 +35,7 @@ _lib = None
 
 # every symbol include/nnsp_b200.h declares (tests/test_abi.py checks the list against the header)
 SYMBOLS = """nnsp_b200_version nnsp_b200_strerror nnsp_b200_last_error nnsp_b200_kernel_launches nnsp_b200_tc5_launches
-nnsp_b200_model_from_net nnsp_b200_model_from_table_text nnsp_b200_model_to_table_text nnsp_b200_model_from_blob nnsp_b200_model_to_blob nnsp_b200_model_set_acc32
+nnsp_b200_cascade_kernel_launches nnsp_b200_model_from_net nnsp_b200_model_from_table_text nnsp_b200_model_to_table_text nnsp_b200_model_from_blob nnsp_b200_model_to_blob nnsp_b200_model_set_acc32
 nnsp_b200_model_info nnsp_b200_model_free nnsp_b200_batch_create nnsp_b200_batch_reset nnsp_b200_batch_exec
 nnsp_b200_batch_exec_host nnsp_b200_batch_exec_host_async nnsp_b200_batch_wait_host nnsp_b200_batch_sync nnsp_b200_batch_last_kernel_ms nnsp_b200_batch_dims
 nnsp_b200_batch_stream nnsp_b200_batch_set_nn_path nnsp_b200_batch_get_nn_path nnsp_b200_batch_destroy nnsp_b200_cascade_default_params nnsp_b200_cascade_create
@@ -65,6 +65,8 @@ def lib():
     L.nnsp_b200_last_error.restype = C.c_char_p
     L.nnsp_b200_kernel_launches.restype = ll
     L.nnsp_b200_tc5_launches.restype = ll
+    L.nnsp_b200_cascade_kernel_launches.restype = ll
+    L.nnsp_b200_cascade_kernel_launches.argtypes = [ci]
     L.nnsp_b200_model_from_net.argtypes = [vp, vp, vp, ci, C.POINTER(vp)]
     L.nnsp_b200_model_from_table_text.argtypes = [C.c_char_p, C.c_size_t, ci, ci, C.POINTER(vp)]
     L.nnsp_b200_model_to_table_text.argtypes = [vp, C.c_char_p, C.c_char_p, C.c_size_t, C.POINTER(C.c_size_t)]

@@ -336,6 +336,9 @@ struct ReplaySmem {
     CsNarrow::WS ws[CR_GROUPS];
     int slot[CR_GROUPS];
 };
+/* both kernels stage the same weight images behind their structs: every cascade the narrow sequential kernel takes fits
+ * the replay kernel, so cascade_kernel<CsNarrow> replays only when NNSP_B200_REPLAY_COOP=0 asks for it */
+static_assert(sizeof(ReplaySmem) <= sizeof(CascadeSmem<CsNarrow>), "the replay kernel must fit wherever the narrow kernel does");
 
 __global__ void __launch_bounds__(CR_THREADS, 1)
 cascade_replay_kernel(CascadeArgs a, int off_w, int off_b)
@@ -1162,13 +1165,16 @@ static int cascade_launch(nnsp_b200_cascade *c, const int16_t *pcm, long long st
     int blocks = (ns + cs_warps - 1) / cs_warps;
     const int cap = sm_count(c->device);
     if (blocks > cap) blocks = cap;
+    int kind;                                   /* nnsp_b200_cascade_kernel_launches */
     if (a.replay_list && c->narrow && c->replay_coop) {
         /* NNSP_CR_GW warps per stream; as many CTAs as the worst case needs (ns streams), at most one per SM */
         int rb = (ns + CR_GROUPS - 1) / CR_GROUPS;
         if (rb > cap) rb = cap;
         cascade_replay_kernel<<<rb, CR_THREADS, c->smem_replay, st>>>(a, c->off_w_replay, c->off_w_replay + (c->off_b - c->off_w));
-    } else if (c->narrow) cascade_kernel<CsNarrow><<<blocks, 32 * CsNarrow::WARPS, c->smem_total, st>>>(a, c->off_w, c->off_b);
-    else cascade_kernel<CsWide><<<blocks, 32 * CsWide::WARPS, c->smem_total, st>>>(a, c->off_w, c->off_b);
+        kind = 2;
+    } else if (c->narrow) { cascade_kernel<CsNarrow><<<blocks, 32 * CsNarrow::WARPS, c->smem_total, st>>>(a, c->off_w, c->off_b); kind = 0; }
+    else { cascade_kernel<CsWide><<<blocks, 32 * CsWide::WARPS, c->smem_total, st>>>(a, c->off_w, c->off_b); kind = 1; }
+    g_cascade_net_launches[kind].fetch_add(1, std::memory_order_relaxed);
     NNSP_LAUNCH_CHECK();
     if (timed) {
         if (!piped) NNSP_CUDA(cudaEventRecord(tl[2], st));      /* one stream: the chain starts where the front end ended */

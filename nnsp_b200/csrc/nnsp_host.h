@@ -11,6 +11,7 @@
 namespace nnsp {
 
 extern std::atomic<long long> g_launches, g_tc5_launches;
+extern std::atomic<long long> g_cascade_net_launches[3];   /* cascade_kernel<CsNarrow>, cascade_kernel<CsWide>, cascade_replay_kernel */
 
 #define NNSP_CUDA(expr)                                                                       \
     do {                                                                                      \

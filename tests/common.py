@@ -96,6 +96,15 @@ NET_TC5_SATURATING = [
     ("sat_feat_p127", 2, (240, 32, 32, 2), (0, 1, 0), (1, 1, 3), (7, 5, 7), (15, 15, 15), (14, 13, 15), 127),
     ("sat_feat_random", 1, (240, 24, 16, 2), (0, 1, 0), (1, 1, 3), (7, 6, 7), (15, 15, 15), (14, 13, 15), None),
 ]
+# stacks on either side of the rule that gives the cascade's sequential kernel its narrow shape (every layer at most 80
+# wide, LSTM state at most 80, at most 48 outputs): exactly 80 / 48, then each limit crossed alone. The two LSTMs of
+# kws_wide_h81 hold 40 + 41 units: a state offset that is a multiple of 4 keeps the scan-split form (41 + 40 would not).
+NET_CASCADE_EDGES = [
+    ("s2i_narrow_edge", 0, (240, 80, 80, 48), (0, 1, 0), (1, 1, 3), (7, 5, 6), (8, 15, 15), (14, 14, 14)),
+    ("s2i_wide_rows81", 0, (240, 81, 80, 48), (0, 1, 0), (1, 1, 3), (7, 5, 6), (8, 15, 15), (14, 14, 14)),
+    ("s2i_wide_out49", 0, (240, 80, 80, 49), (0, 1, 0), (1, 1, 3), (7, 5, 6), (8, 15, 15), (14, 14, 14)),
+    ("kws_wide_h81", 2, (240, 40, 40, 41, 2), (0, 1, 1, 0), (1, 1, 1, 3), (7, 5, 5, 6), (8, 15, 15, 15), (14, 13, 13, 15)),
+]
 
 
 def net_case_blob(case, acc32):
@@ -126,3 +135,27 @@ def adversarial_states(rng, n, h_stride):
     c[1] = 2 ** 31 - 1; c[2] = -2 ** 31 + 1
     h[3] = 32767; h[4] = -32768
     return h, c
+
+
+def chunks(k, pattern=(100,)):
+    """lengths of the calls that cover k frames, cycling through `pattern`, the last one cut to length"""
+    out, i = [], 0
+    while sum(out) < k:
+        out.append(min(pattern[i % len(pattern)], k - sum(out)))
+        i += 1
+    return out
+
+
+def cascade_events(res, valid):
+    """per stream and frame t of the oracle cascade records: a new instance starts at t (stage change, or the stage's
+    instance was reset at t - 1), a detection at t, a time-out at t (the controller moved on without a detection, or the
+    s2i-only counter wrapped). res: [S][T] records, valid: [S][T]."""
+    sid, pos, det = res["stage_id"].astype(int), res["pos_after"].astype(int), res["detected"] != 0
+    new = np.zeros(sid.shape, bool)
+    new[:, 1:] = (sid[:, 1:] != sid[:, :-1]) | (valid[:, :-1] == 0)
+    pos_before = np.concatenate([np.zeros((len(pos), 1), int), pos[:, :-1]], axis=1)
+    cnt = res["cnt_timeout"].astype(int)
+    wrapped = np.zeros(sid.shape, bool)
+    wrapped[:, 1:] = (sid[:, 1:] == sid[:, :-1]) & (cnt[:, 1:] < cnt[:, :-1])
+    timeout = ~det & (sid != 1) & ((pos != pos_before) | wrapped)       # 1: VAD, which has no time-out
+    return new, det, timeout

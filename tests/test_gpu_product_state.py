@@ -19,10 +19,11 @@ import ctypes as C
 import numpy as np
 import pytest
 
+from common import cascade_events, chunks
+
 pytestmark = pytest.mark.gpu
 MODEL_FILE = {0: "s2i.nnspm", 1: "vad.nnspm", 2: "kws_galaxy.nnspm"}
 S2I, VAD, KWS = 0, 1, 2
-CALL = 100                                     # longest call of a prefix: the bench shape
 CASC_TAPS = (("logmel", "logmel"), ("feat", "feat"), ("hstate", "h"), ("cstate", "c"), ("post", "post"))
 BATCH_TAPS = CASC_TAPS + (("act", "act"), ("logits", "logits"))
 PIPE_LENS = [50, 50, 3, 47, 100, 50, 1, 49, 50, 100]     # prefix calls of the pipelined arm (cycled, cut to length)
@@ -48,14 +49,6 @@ def test_cascade_sets_cover_every_stage_and_event():
     assert all(any(e in c[6] for c in CASC_SETS) for e in ("fix", "detection", "timeout"))
 
 
-def _chunks(k, pattern=(CALL,)):
-    out, i = [], 0
-    while sum(out) < k:
-        out.append(min(pattern[i % len(pattern)], k - sum(out)))
-        i += 1
-    return out
-
-
 def _first_diff(a, b):
     bad = (a != b).reshape(a.shape[0], a.shape[1], -1).any(axis=2)
     s, t = (int(x[0]) for x in np.nonzero(bad))
@@ -75,21 +68,6 @@ def _stream_params(nb, c):
             p[names.index(n)] = rng.integers(lo, hi + 1)
         rows.append(p)
     return np.stack(rows)
-
-
-def cascade_events(res, valid):
-    """per stream and frame t of the oracle records: a new instance starts at t (stage change, or the stage's instance was
-    reset at t - 1), a detection at t, a time-out at t (the controller moved on without a detection, or the s2i-only
-    counter wrapped). res: [S][T] records, valid: [S][T]."""
-    sid, pos, det = res["stage_id"].astype(int), res["pos_after"].astype(int), res["detected"] != 0
-    new = np.zeros(sid.shape, bool)
-    new[:, 1:] = (sid[:, 1:] != sid[:, :-1]) | (valid[:, :-1] == 0)
-    pos_before = np.concatenate([np.zeros((len(pos), 1), int), pos[:, :-1]], axis=1)
-    cnt = res["cnt_timeout"].astype(int)
-    wrapped = np.zeros(sid.shape, bool)
-    wrapped[:, 1:] = (sid[:, 1:] == sid[:, :-1]) & (cnt[:, 1:] < cnt[:, :-1])
-    timeout = ~det & (sid != VAD) & ((pos != pos_before) | wrapped)
-    return new, det, timeout
 
 
 @pytest.fixture(scope="module")
@@ -157,7 +135,7 @@ def test_cascade_sorted_pass_state_at_every_cut(nb, oracle, cascade_models, monk
     for k in cuts:
         c = make()
         parts, t = [], 0
-        for n in _chunks(k):
+        for n in chunks(k):
             parts.append(c.exec(pcm[:, t * 160:(t + n) * 160]))
             t += n
         res2, taps = c.exec(pcm[:, k * 160:(k + 2) * 160], taps=True)
@@ -169,7 +147,7 @@ def test_cascade_sorted_pass_state_at_every_cut(nb, oracle, cascade_models, monk
     row = pcm.shape[1]
     for k in cuts[::7]:
         c = make()
-        lens, t = _chunks(k, PIPE_LENS), 0
+        lens, t = chunks(k, PIPE_LENS), 0
         outs = [nb.DeviceArray((S, n), nb.CASCADE_RESULT_DT) for n in lens]
         for n, o in zip(lens, outs):
             c.exec_device(C.c_void_p(d_pcm.ptr.value + 2 * t * 160), row, n, o)
@@ -210,7 +188,7 @@ def test_batch_state_at_every_cut(nb, oracle, monkeypatch, nn_id, acc32, arm):
         assert b.nn_path == "split"
         parts, t = [], 0
         n0 = nb.tc5_launches()
-        for n in _chunks(k):
+        for n in chunks(k):
             parts.append(b.exec(pcm[:, t * 160:(t + n) * 160]))
             t += n
         tc5_calls += nb.tc5_launches() - n0
@@ -227,7 +205,7 @@ def test_batch_state_at_every_cut(nb, oracle, monkeypatch, nn_id, acc32, arm):
                 raise AssertionError("cut %d: stream %d frame %d tap %s: gpu %s oracle %s" % (k, s, k + t, g, a[s, t][:6], o[s, t][:6]))
     # prefix calls with an inference: k = 1 .. 140 hold 140 of them plus one per cut past 100; the library's rule takes the
     # tcgen05 kernel for the calls of >= 29 inferences only
-    with_inf = sum(len(_chunks(k)) for k in range(1, K + 1))
+    with_inf = sum(len(chunks(k)) for k in range(1, K + 1))
     if arm == "tc5_forced":
         assert tc5_calls == with_inf
     else:
