@@ -20,6 +20,7 @@
  *   nnsp_b200_cascade_create ........ nnCntrlClass_init         evb/src/nnCntrlClass.c:56-128
  *   nnsp_b200_cascade_reset ......... nnCntrlClass_reset        evb/src/nnCntrlClass.c:130-150
  *   nnsp_b200_cascade_exec[_host] ... nnCntrlClass_exec         evb/src/nnCntrlClass.c:152-272
+ *   nnsp_b200_cascade_exec_*ragged* . the same, called a different number of times on each instance
  *   nnsp_b200_ingest_audadc ......... audio_frame_callback      evb/src/main_nnsp.cc:58-65 (mask + glitch fix)
  *   nnsp_b200_feature_stages ........ stftModule_analyze/spec2pspec/melSpecProc/log10_vec
  *                                     ns-nnsp/src/spectrogram_module.c:33-77, melSpecProc.c:6-27,
@@ -215,6 +216,25 @@ int nnsp_b200_cascade_exec_host(nnsp_b200_cascade *c, const int16_t *pcm, long l
 /* asynchronous twin of the host-buffer call: see nnsp_b200_batch_exec_host_async */
 int nnsp_b200_cascade_exec_host_async(nnsp_b200_cascade *c, const int16_t *pcm, long long stream_stride,
                                       int n_frames, nnsp_b200_cascade_result *results, long long *ticket);
+/* Ragged calls: stream s advances by n_frames[s] frames (0 <= n_frames[s] <= max_frames), exactly as if nnCntrlClass_exec
+ * had been called n_frames[s] times on its instance -- a server passes what each stream has buffered, 0 for an idle slot.
+ * PCM layout as nnsp_b200_cascade_exec with T = max_frames; no sample of a frame t >= n_frames[s] is used. Records
+ * and tap rows of frames t >= n_frames[s] are written as "no frame": stage_id = -1 and every other field 0 (taps: zero
+ * rows). A stream with n_frames[s] == 0 keeps its whole state (counters, time-outs, PCM and log-mel history).
+ *   exec_ragged: n_frames_dev is a device array of n_streams counts, owned and pipelined like pcm_dev; values outside
+ *     [0, max_frames] are clamped on the device. No sample of a frame t >= n_frames[s] is read. A call whose counts all
+ *     equal max_frames is nnsp_b200_cascade_exec: same bytes, the same sequence of kernel launches.
+ *   exec_host_ragged_async: n_frames is host memory (same lifetime rules as pcm); a value outside [0, max_frames] returns
+ *     NNSP_B200_ERR_ARG before anything is queued. Follows nnsp_b200_cascade_set_host_format, slices and pipelines like
+ *     nnsp_b200_cascade_exec_host_async and completes in ticket order (nnsp_b200_cascade_wait_host). Like the uniform
+ *     call it copies every stream's max_frames frames (and conditions them, for AUDADC words); only the feature and
+ *     history kernels read PCM, and they read none past a stream's count. */
+int nnsp_b200_cascade_exec_ragged(nnsp_b200_cascade *c, const int16_t *pcm_dev, long long stream_stride, int max_frames,
+                                  const int32_t *n_frames_dev, nnsp_b200_cascade_result *results_dev,
+                                  const nnsp_b200_taps *taps);
+int nnsp_b200_cascade_exec_host_ragged_async(nnsp_b200_cascade *c, const int16_t *pcm, long long stream_stride,
+                                             int max_frames, const int32_t *n_frames, nnsp_b200_cascade_result *results,
+                                             long long *ticket);
 int nnsp_b200_cascade_wait_host(nnsp_b200_cascade *c, long long ticket);
 int nnsp_b200_cascade_sync(nnsp_b200_cascade *c);
 int nnsp_b200_cascade_last_kernel_ms(nnsp_b200_cascade *c, float ms[3]);

@@ -272,6 +272,7 @@ class Cascade:
             for k, v in params.items():
                 setattr(p, k, v)
         self.params = p
+        self._counts_in_flight = {}          # ticket -> host counts of a ragged host call, kept alive until it completes
         self.h = C.c_void_p()
         check(L.nnsp_b200_cascade_create(arr, seq_a, len(seq), C.byref(p), self.S, device, C.byref(self.h)), "cascade_create")
 
@@ -317,6 +318,37 @@ class Cascade:
                 v.free()
         return (res, out) if taps else res
 
+    def exec_ragged_device(self, pcm_dev, stride, max_frames, n_frames_dev, results_dev=None, taps=None):
+        """Asynchronous ragged call on device buffers: stream s advances by n_frames_dev[s] (int32, on the device) frames"""
+        p = pcm_dev.ptr if isinstance(pcm_dev, DeviceArray) else pcm_dev
+        n = n_frames_dev.ptr if isinstance(n_frames_dev, DeviceArray) else n_frames_dev
+        r = results_dev.ptr if isinstance(results_dev, DeviceArray) else results_dev
+        check(lib().nnsp_b200_cascade_exec_ragged(self.h, p, stride, max_frames, n, r, C.byref(taps) if taps is not None else None),
+              "cascade_exec_ragged")
+
+    def exec_ragged(self, pcm, n_frames, taps=False):
+        """pcm: int16 [S, T*160]; stream s advances by n_frames[s] (0..T) of its frames, as if nnCntrlClass_exec ran n_frames[s]
+        times on it. Records (and tap rows) of frames t >= n_frames[s] are "no frame": stage_id -1, every other field 0."""
+        pcm = np.ascontiguousarray(pcm, np.int16)
+        T = pcm.shape[1] // FRAME
+        counts = np.ascontiguousarray(n_frames, np.int32)
+        assert counts.shape == (self.S,)
+        d_pcm = DeviceArray.from_host(pcm, self.device)
+        d_cnt = DeviceArray.from_host(counts, self.device)
+        d_res = DeviceArray((self.S, T), CASCADE_RESULT_DT, self.device)
+        tp, arrs = (None, None)
+        if taps:
+            tp, arrs = _make_taps(self.S, T, 1, 128, 1, self.device)
+        self.exec_ragged_device(d_pcm, pcm.shape[1], T, d_cnt, d_res, tp)
+        self.sync()
+        res = d_res.to_host()
+        out = {k: v.to_host() for k, v in arrs.items()} if taps else None
+        d_pcm.free(); d_cnt.free(); d_res.free()
+        if arrs:
+            for v in arrs.values():
+                v.free()
+        return (res, out) if taps else res
+
     def set_host_format(self, fmt):
         check(lib().nnsp_b200_cascade_set_host_format(self.h, NNSPBatch.HOST_FORMAT[fmt]), "cascade_set_host_format")
 
@@ -338,8 +370,26 @@ class Cascade:
                                                       results.ctypes.data_as(C.c_void_p), C.byref(ticket)), "cascade_exec_host_async")
         return ticket.value
 
+    def exec_host_ragged_async(self, pcm, n_frames, results):
+        """exec_host_async with a frame count per stream (0..T): `pcm` (int16, or uint32 AUDADC words after
+        set_host_format('audadc')) and `results` (pinned) must stay untouched until wait_host(ticket). Counts outside
+        0..T raise NnspError and queue nothing."""
+        assert pcm.dtype in (np.int16, np.uint32) and pcm.flags.c_contiguous and pcm.shape[0] == self.S
+        T = pcm.shape[1] // FRAME
+        assert results.dtype == CASCADE_RESULT_DT and results.flags.c_contiguous and results.shape == (self.S, T)
+        counts = np.ascontiguousarray(n_frames, np.int32)
+        assert counts.shape == (self.S,)
+        ticket = C.c_longlong(0)
+        check(lib().nnsp_b200_cascade_exec_host_ragged_async(self.h, pcm.ctypes.data_as(C.c_void_p), pcm.shape[1], T,
+                                                             counts.ctypes.data_as(C.c_void_p), results.ctypes.data_as(C.c_void_p),
+                                                             C.byref(ticket)), "cascade_exec_host_ragged_async")
+        self._counts_in_flight[ticket.value] = counts
+        return ticket.value
+
     def wait_host(self, ticket):
         check(lib().nnsp_b200_cascade_wait_host(self.h, ticket), "cascade_wait_host")
+        for t in [t for t in self._counts_in_flight if t <= ticket]:      # calls complete in ticket order
+            del self._counts_in_flight[t]
 
     def last_kernel_ms(self):
         ms = (C.c_float * 3)()

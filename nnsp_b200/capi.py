@@ -46,7 +46,8 @@ nnsp_b200_host_free_pinned nnsp_b200_memcpy_h2d nnsp_b200_memcpy_d2h nnsp_b200_m
 nnsp_b200_event_record nnsp_b200_event_elapsed_ms nnsp_b200_event_destroy nnsp_b200_int_peak nnsp_b200_net_eval
 nnsp_b200_group_create_batch nnsp_b200_group_create_cascade nnsp_b200_group_size nnsp_b200_group_range nnsp_b200_group_reset nnsp_b200_group_set_stream_params
 nnsp_b200_group_exec_host nnsp_b200_group_exec_host_async nnsp_b200_group_wait nnsp_b200_group_destroy
-nnsp_b200_batch_set_host_format nnsp_b200_cascade_set_host_format nnsp_b200_wav_info nnsp_b200_wav_read_frames nnsp_b200_wav_load_streams nnsp_b200_cascade_timeline""".split()
+nnsp_b200_batch_set_host_format nnsp_b200_cascade_set_host_format nnsp_b200_wav_info nnsp_b200_wav_read_frames nnsp_b200_wav_load_streams nnsp_b200_cascade_timeline
+nnsp_b200_cascade_exec_ragged nnsp_b200_cascade_exec_host_ragged_async""".split()
 
 
 def lib():
@@ -100,6 +101,8 @@ def lib():
         L.nnsp_b200_cascade_exec.argtypes = [vp, vp, ll, ci, vp, C.POINTER(Taps)]
         L.nnsp_b200_cascade_exec_host.argtypes = [vp, vp, ll, ci, vp]
         L.nnsp_b200_cascade_exec_host_async.argtypes = [vp, vp, ll, ci, vp, C.POINTER(ll)]
+        L.nnsp_b200_cascade_exec_ragged.argtypes = [vp, vp, ll, ci, vp, vp, C.POINTER(Taps)]
+        L.nnsp_b200_cascade_exec_host_ragged_async.argtypes = [vp, vp, ll, ci, vp, vp, C.POINTER(ll)]
         L.nnsp_b200_cascade_wait_host.argtypes = [vp, ll]
         L.nnsp_b200_cascade_sync.argtypes = [vp]
         L.nnsp_b200_cascade_last_kernel_ms.argtypes = [vp, C.POINTER(C.c_float * 3)]

@@ -69,7 +69,16 @@ struct CascadeArgs {
     const int *t0;                    /* per stream: first frame this kernel still has to process (null: 0) */
     const int *replay_list;           /* with t0: the streams that still have frames left, handed out dynamically ... */
     int *replay_ctl;                  /* ... [0] = how many, [1] = cursor                                         */
+    const int32_t *nfr;               /* ragged call: stream s runs frames [0, stream_frames(nfr, s, T)) (null: all T) */
 };
+
+/* frames [Ts, T) of stream s in a ragged call: "no frame" records -- stage_id -1, every other field 0 -- by the threads
+ * i0, i0 + step, ... (12-byte records, written as 4-byte words) */
+__device__ __forceinline__ void write_no_frames(nnsp_b200_cascade_result *results, long long s, int Ts, int T, int i0, int step)
+{
+    uint32_t *out = reinterpret_cast<uint32_t *>(results + s * T);
+    for (int i = 3 * Ts + i0; i < 3 * T; i += step) out[i] = (i % 3 == 0) ? 0xffu : 0u;
+}
 
 __device__ __forceinline__ CascThr load_thr(const CascadeDev &cd, long long s)
 {
@@ -164,8 +173,18 @@ cascade_kernel(CascadeArgs a, int off_w, int off_b)
             if (si >= a.ns) break;
             s = a.s0 + si;
         }
+        const int Ts = stream_frames(a.nfr, s, T);                    /* this stream's frames [0, Ts) of the call */
+        if (!a.replay_list && Ts < T) {                               /* ragged call: nothing for the frames past them */
+            if (a.results) write_no_frames(a.results, s, Ts, T, lane, 32);
+            const long long f0 = (long long)s * T + Ts, nf = T - Ts;
+            if (a.taps.logmel) for (long long i = lane; i < nf * 40; i += 32) a.taps.logmel[f0 * 40 + i] = 0;
+            if (a.taps.feat) for (long long i = lane; i < nf * 40; i += 32) a.taps.feat[f0 * 40 + i] = 0;
+            if (a.taps.hstate) for (long long i = lane; i < nf * HS; i += 32) a.taps.hstate[f0 * HS + i] = 0;
+            if (a.taps.cstate) for (long long i = lane; i < nf * HS; i += 32) a.taps.cstate[f0 * HS + i] = 0;
+            if (a.taps.post) for (long long i = lane; i < nf * SC_N; i += 32) a.taps.post[f0 * SC_N + i] = 0;
+        }
         const int t_begin = a.t0 ? a.t0[s] : 0;                       /* frames before it were done by the stage-sorted pass */
-        if (t_begin >= a.T) continue;
+        if (t_begin >= Ts) continue;
         for (int i = lane; i < 240; i += 32) ws->ctx[i] = a.st.ctx[(long long)s * 240 + i];
         for (int i = lane; i < HW; i += 32) { ws->h[i] = a.st.h[(long long)s * HS + i]; ws->c[i] = a.st.c[(long long)s * HS + i]; }
         if (lane < SC_N) ws->scal[lane] = a.st.scal[(long long)s * SC_N + lane];
@@ -179,7 +198,7 @@ cascade_kernel(CascadeArgs a, int off_w, int off_b)
         const int32_t *lm_now = a.logmel + (long long)s * T * NNSP_B200_NMEL;
         const int32_t *lm_old = a.st.lmhist + ((long long)s * cd.dmax + cd.dmax) * NNSP_B200_NMEL;   /* lm_old[r*40], r < 0 */
 
-        for (int t = t_begin; t < T; t++) {
+        for (int t = t_begin; t < Ts; t++) {
             const long long ft = (long long)s * T + t;
             const int id = cd.seq[pos];
             const DevModel &M = sm.model[id];
@@ -408,8 +427,8 @@ cascade_replay_kernel(CascadeArgs a, int off_w, int off_b)
         group_sync<CR_GW>(bid);                                              /* everyone has read the slot before it is rewritten */
         if (idx >= a.replay_ctl[0]) break;
         const int s = a.replay_list[idx];
-        const int t_begin = a.t0[s];
-        if (t_begin >= T) continue;
+        const int t_begin = a.t0[s], Ts = stream_frames(a.nfr, s, T);
+        if (t_begin >= Ts) continue;
         for (int i = gt; i < 240; i += CR_GT) ws->ctx[i] = a.st.ctx[(long long)s * 240 + i];
         for (int i = gt; i < HW; i += CR_GT) { ws->h[i] = a.st.h[(long long)s * HS + i]; ws->c[i] = a.st.c[(long long)s * HS + i]; }
         if (gt < SC_N) ws->scal[gt] = a.st.scal[(long long)s * SC_N + gt];
@@ -423,7 +442,7 @@ cascade_replay_kernel(CascadeArgs a, int off_w, int off_b)
         const int32_t *lm_now = a.logmel + (long long)s * T * NNSP_B200_NMEL;
         const int32_t *lm_old = a.st.lmhist + ((long long)s * cd.dmax + cd.dmax) * NNSP_B200_NMEL;
 
-        for (int t = t_begin; t < T; t++) {
+        for (int t = t_begin; t < Ts; t++) {
             const long long ft = (long long)s * T + t;
             const int id = cd.seq[pos];
             const DevModel &M = sm.model[id];
@@ -563,7 +582,7 @@ struct RoundArrays {                  /* per stream, valid during one call */
 };
 
 __global__ void cascade_classify_kernel(StreamState st, CascadeDev cd, int s0, int ns, int S, int *list, int *ctl, RoundArrays ra,
-                                        int *fix_list)
+                                        int *fix_list, const int32_t *nfr, int T)
 {
     const int si = blockIdx.x * blockDim.x + threadIdx.x;
     if (si >= ns) return;
@@ -574,6 +593,7 @@ __global__ void cascade_classify_kernel(StreamState st, CascadeDev cd, int s0, i
     ra.tstart[s] = (st.scal[s * SC_N + SC_SLIDES] == 1) ? 0 : 1;     /* nn_speech.c:84: the stride-2 gate */
     ra.age0[s] = age;
     ra.t0[s] = -1;
+    if (stream_frames(nfr, s, T) == 0) return;                       /* ragged call, idle stream: in no group */
     list[(long long)id * S + s0 + atomicAdd(&ctl[id], 1)] = (int)s;
     if (age < 2) fix_list[s0 + atomicAdd(&ctl[CTL_FIX], 1)] = (int)s;
 }
@@ -583,12 +603,13 @@ __global__ void cascade_offsets_kernel(int *ctl)
     for (int g = 0; g < 3; g++) { ctl[3 + g] = o; o += (ctl[g] + 15) >> 4; }
 }
 
-/* round r >= 1: the streams queued by the previous round's walk, sorted by (model they entered, start frame) so that a
- * 16-stream tile holds streams of similar length; one CTA, counting sort over 3 x 256 buckets */
+/* round r >= 1: the streams queued by the previous round's walk, sorted by (model they entered, frames left) so that a
+ * 16-stream tile holds streams of similar length; one CTA, counting sort over 3 x 256 buckets. The key T - (frames left)
+ * is the start frame unless the call is ragged. */
 constexpr int CSORT_THREADS = 1024, CSORT_BUCKETS = 1024, CRG_NB = 256;
 __global__ void __launch_bounds__(CSORT_THREADS) cascade_regroup_kernel(StreamState st, CascadeDev cd, const int *__restrict__ pend,
                                                                        const int *__restrict__ ctl_prev, int *ctl, int *list, int S, int s0,
-                                                                       RoundArrays ra, int T)
+                                                                       RoundArrays ra, int T, const int32_t *nfr)
 {
     __shared__ int hist[3 * CRG_NB];
     __shared__ int gstart[4];
@@ -598,7 +619,7 @@ __global__ void __launch_bounds__(CSORT_THREADS) cascade_regroup_kernel(StreamSt
     __syncthreads();
     auto bucket = [&](int s) {
         const int id = cd.seq[st.casc[(long long)s * CS_N + CS_POS]];
-        const long long b = (long long)ra.tstart[s] * CRG_NB / (T + 1);
+        const long long b = (long long)(ra.tstart[s] + T - stream_frames(nfr, s, T)) * CRG_NB / (T + 1);
         return id * CRG_NB + (int)(b < 0 ? 0 : (b >= CRG_NB ? CRG_NB - 1 : b));
     };
     for (int i = threadIdx.x; i < n; i += CSORT_THREADS) atomicAdd(&hist[bucket(pend[i])], 1);
@@ -636,6 +657,7 @@ struct FixArgs {
     RoundArrays ra;
     CascadeDev cd;
     int T;
+    const int32_t *nfr;              /* ragged call: no row past the stream's own frames */
 };
 struct FixSmem { FeatSmemTables ft; FrameScratch fs[16]; };
 __global__ void __launch_bounds__(256) cascade_fix_kernel(FixArgs a)
@@ -653,7 +675,7 @@ __global__ void __launch_bounds__(256) cascade_fix_kernel(FixArgs a)
         const int id = cd.seq[a.st.casc[s * CS_N + CS_POS]];
         const int d = (id == NNSP_B200_ID_VAD) ? 0 : (id == NNSP_B200_ID_KWS ? cd.P.frs_vbufBk_kws : cd.P.frs_vbufBk_s2i);
         const int t = a.ra.tb[s] + la - a.ra.age0[s];                 /* frame of the call with life index la */
-        const bool valid = la >= a.ra.age0[s] && t < a.T;
+        const bool valid = la >= a.ra.age0[s] && t < stream_frames(a.nfr, s, a.T);
         const int tf = t - d, base = (tf - 2) * NNSP_B200_FRAME, first_live = (2 - la) * NNSP_B200_FRAME;
         const int16_t *ps = a.pcm + s * a.stride;
         const int16_t *hs = a.st.hist + s * hist_len + hist_len;       /* hs[g], g < 0: frames before the call */
@@ -667,11 +689,11 @@ __global__ void __launch_bounds__(256) cascade_fix_kernel(FixArgs a)
 }
 
 /* The replay is latency-bound -- one warp walks one stream frame by frame, so the kernel lasts at least as long as the
- * longest remainder. Handing the streams out longest-first (earliest t0 first) keeps a long one from being started
- * last: a counting sort of the list by t0, one CTA. */
+ * longest remainder. Handing the streams out longest-first (earliest t0 first; in a ragged call, least T - frames left)
+ * keeps a long one from being started last: a counting sort of the list, one CTA. */
 __global__ void __launch_bounds__(CSORT_THREADS) cascade_sort_replay_kernel(const int *__restrict__ list_in, int *__restrict__ list_out,
                                                                            const int *__restrict__ count_in, int *__restrict__ ctl_out,
-                                                                           const int *__restrict__ t0, int T)
+                                                                           const int *__restrict__ t0, int T, const int32_t *__restrict__ nfr)
 {
     __shared__ int hist[CSORT_BUCKETS];
     const int n = *count_in;
@@ -679,7 +701,10 @@ __global__ void __launch_bounds__(CSORT_THREADS) cascade_sort_replay_kernel(cons
     if (n == 0) return;
     for (int i = threadIdx.x; i < CSORT_BUCKETS; i += CSORT_THREADS) hist[i] = 0;
     __syncthreads();
-    auto bucket = [&](int s) { const long long b = (long long)t0[s] * CSORT_BUCKETS / (T + 1); return (int)(b < 0 ? 0 : (b >= CSORT_BUCKETS ? CSORT_BUCKETS - 1 : b)); };
+    auto bucket = [&](int s) {
+        const long long b = (long long)(t0[s] + T - stream_frames(nfr, s, T)) * CSORT_BUCKETS / (T + 1);
+        return (int)(b < 0 ? 0 : (b >= CSORT_BUCKETS ? CSORT_BUCKETS - 1 : b));
+    };
     for (int i = threadIdx.x; i < n; i += CSORT_THREADS) atomicAdd(&hist[bucket(list_in[i])], 1);
     __syncthreads();
     if (threadIdx.x < 32) {                                            /* exclusive scan of 1024 counts by one warp */
@@ -709,6 +734,7 @@ struct CascadePostArgs {
     int s0, ns, T;
     nnsp_b200_cascade_result *results;
     CascadeDev cd;
+    const int32_t *nfr;              /* ragged call: stream s ends at frame stream_frames(nfr, s, T) */
 };
 
 /* log-mel row the instance of stream s reads at frame f of the call (f >= its tb): a fix row during its first two frames */
@@ -726,6 +752,7 @@ __device__ __forceinline__ const int32_t *cascade_lm_row(const CascadePostArgs &
  * (every lane redundantly, on broadcast decision records) only steps through the INFERENCES of the round to find the
  * first detection -- s2i_post_proc / binary_post_proc on the decision records, nn_speech.c:146-227 -- takes the earlier of
  * that and the first time-out that leaves the instance, and then writes all result records of the round in parallel. */
+template <bool RAGGED>                                                 /* RAGGED: a.nfr != null; false: the uniform call's code */
 __global__ void __launch_bounds__(32 * CPOST_WARPS) cascade_post_kernel(CascadePostArgs a)
 {
     const CascadeDev &cd = a.cd;
@@ -734,7 +761,11 @@ __global__ void __launch_bounds__(32 * CPOST_WARPS) cascade_post_kernel(CascadeP
     const int si = blockIdx.x * CPOST_WARPS + (threadIdx.x >> 5);
     if (si >= nsel) return;
     const long long s = a.list ? a.list[si] : (long long)a.s0 + si;
-    const int T = a.T;
+    const int T = a.T, Ts = RAGGED ? stream_frames(a.nfr, s, T) : T;  /* the stream's frames of the call: [0, Ts) */
+    if (RAGGED) {
+        if (!a.list && a.results && Ts < T) write_no_frames(a.results, s, Ts, T, lane, 32);   /* round 0 */
+        if (Ts == 0) return;                                          /* idle stream: its state stays as it is */
+    }
     const int tb = a.ra.tb[s], ts = a.ra.tstart[s], age0 = a.ra.age0[s];
     const int pos = a.st.casc[s * CS_N + CS_POS];
     int cnt_kws = a.st.casc[s * CS_N + CS_CNT_KWS], cnt_s2i = a.st.casc[s * CS_N + CS_CNT_S2I];
@@ -759,7 +790,7 @@ __global__ void __launch_bounds__(32 * CPOST_WARPS) cascade_post_kernel(CascadeP
     const bool has_to = id != NNSP_B200_ID_VAD;
     const int timeout = (id == NNSP_B200_ID_S2I) ? thr.timeout_s2i : thr.timeout_kws;
     const int c0 = (id == NNSP_B200_ID_S2I) ? cnt_s2i : cnt_kws;
-    int to_next = pos, t_to = T;                                      /* first frame whose counter reads time-out - 1 */
+    int to_next = pos, t_to = Ts;                                     /* first frame whose counter reads time-out - 1 */
     bool to_exit = false;
     if (has_to) {
         int n = (timeout - 1 - c0) % timeout;                          /* c0 may exceed a time-out that was shortened at run time */
@@ -769,7 +800,7 @@ __global__ void __launch_bounds__(32 * CPOST_WARPS) cascade_post_kernel(CascadeP
         else { to_next = (pos - 1) % cd.len_seq; if (to_next < 0) to_next += cd.len_seq; }
         to_exit = cd.seq[to_next] != id;                              /* otherwise the time-out changes nothing (:198, :234) */
     }
-    const int t_lim = (to_exit && t_to < T) ? t_to : T - 1;           /* last frame this instance can see in this call */
+    const int t_lim = (to_exit && t_to < Ts) ? t_to : Ts - 1;         /* last frame this instance can see in this call */
     /* ---- first detection: a stale trigger on the frame before the first inference, else the first inference that fires */
     int t_det = -1;
     if (ts > tb && tb <= t_lim && trig) t_det = tb;                   /* nn_speech.c:126: odd frames return the previous trigger */
@@ -810,8 +841,8 @@ __global__ void __launch_bounds__(32 * CPOST_WARPS) cascade_post_kernel(CascadeP
     int t_exit = -1, next_pos_exit = pos;
     bool by_det = false;
     if (t_det >= 0) { t_exit = t_det; by_det = true; next_pos_exit = (pos + 1) % cd.len_seq; }   /* :189-205, :224-228, :256-266 */
-    else if (to_exit && t_to < T) { t_exit = t_to; next_pos_exit = to_next; }
-    const int t_last = (t_exit >= 0) ? t_exit : T - 1;
+    else if (to_exit && t_to < Ts) { t_exit = t_to; next_pos_exit = to_next; }
+    const int t_last = (t_exit >= 0) ? t_exit : Ts - 1;
     /* ---- result records of frames tb .. t_last, in parallel */
     if (a.results) {
         uint32_t *out = reinterpret_cast<uint32_t *>(a.results + s * T);                   /* 12-byte records, 4-byte aligned */
@@ -853,10 +884,10 @@ __global__ void __launch_bounds__(32 * CPOST_WARPS) cascade_post_kernel(CascadeP
             a.st.casc[s * CS_N + CS_AGE] = 0;
             a.ra.t0[s] = t_exit + 1;
             a.ra.tb[s] = t_exit + 1; a.ra.tstart[s] = t_exit + 1; a.ra.age0[s] = 0;   /* a fresh instance: slides == 1 (nn_speech.c:62) */
-            if (t_exit + 1 < T) a.next_list[a.s0 + atomicAdd(a.next_count, 1)] = (int)s;
+            if (t_exit + 1 < Ts) a.next_list[a.s0 + atomicAdd(a.next_count, 1)] = (int)s;   /* at Ts - 1: next call */
         }
     } else {
-        const int n = T - tb;                                          /* frames the instance lived in this call */
+        const int n = Ts - tb;                                         /* frames the instance lived in this call */
         if (has_to) { const int c = (c0 + n) % timeout; if (id == NNSP_B200_ID_S2I) cnt_s2i = c; else cnt_kws = c; }
         slides ^= n & 1;                                               /* nn_speech.c:125 */
         if (lane == 0) {
@@ -880,7 +911,7 @@ __global__ void __launch_bounds__(32 * CPOST_WARPS) cascade_post_kernel(CascadeP
 }
 
 /* context of the instances that lived through the call (t0 == T + 1): the newest six standardised rows of (the rows the
- * instance had when its life in this call began ++ the rows of its frames tb .. T-1, read with its look-back); a warp
+ * instance had when its life in this call began ++ the rows of its frames tb .. Ts-1, read with its look-back); a warp
  * per stream */
 __global__ void __launch_bounds__(256) cascade_ctx_kernel(CascadePostArgs a)
 {
@@ -892,7 +923,7 @@ __global__ void __launch_bounds__(256) cascade_ctx_kernel(CascadePostArgs a)
     const CascadeDev &cd = a.cd;
     const int id = cd.seq[a.st.casc[s * CS_N + CS_POS]];
     const int d = (id == NNSP_B200_ID_VAD) ? 0 : (id == NNSP_B200_ID_KWS ? cd.P.frs_vbufBk_kws : cd.P.frs_vbufBk_s2i);
-    const int tb = a.ra.tb[s], age0 = a.ra.age0[s];
+    const int tb = a.ra.tb[s], age0 = a.ra.age0[s], Ts = stream_frames(a.nfr, s, T);
     const MmaModel &M = *a.model[id];
     int16_t *ctx = a.st.ctx + s * 240;
     int16_t v[8];
@@ -901,7 +932,7 @@ __global__ void __launch_bounds__(256) cascade_ctx_kernel(CascadePostArgs a)
         const int e = lane + 32 * k;
         v[k] = 0;
         if (e < 240) {
-            const int j = e / 40, i = e - j * 40, f = T - 6 + j;
+            const int j = e / 40, i = e - j * 40, f = Ts - 6 + j;
             v[k] = (f >= tb) ? standardise(cascade_lm_row(a, s, f, d, tb, age0)[i], M.mean[i], M.stdR[i], M.feat_rshift)
                              : ctx[(6 + f - tb) * 40 + i];
         }
@@ -1004,6 +1035,7 @@ struct nnsp_b200_cascade {
     int host_last_T = 0;                       /* frames per stream of the latest host-buffer call */
     int host_fmt = NNSP_B200_HOST_PCM16;       /* int16 PCM or raw 32-bit AUDADC words (conditioned on the device) */
     uint32_t *d_raw = nullptr;
+    int32_t *d_nfr = nullptr;                  /* ragged host-buffer calls: the per-stream counts, two buffers of [S] like d_pcm */
 };
 
 constexpr int CS_MAX_SLICES = 8;
@@ -1063,12 +1095,13 @@ static int cascade_ensure_logmel(nnsp_b200_cascade *c, int T)
 static int cascade_launch(nnsp_b200_cascade *c, const int16_t *pcm, long long stride, int T, int s0, int ns,
                           nnsp_b200_cascade_result *results, const nnsp_b200_taps *taps, cudaStream_t st, bool timed,
                           int slice = 0, int32_t *logmel = nullptr, cudaStream_t st_nn = nullptr, cudaEvent_t ev_feat = nullptr,
-                          cudaEvent_t ev_prev_nn = nullptr)
+                          cudaEvent_t ev_prev_nn = nullptr, const int32_t *nfr = nullptr)
 {
     const int hist_frames = c->cd.dmax + 2;
     if (!logmel) logmel = c->logmel;
     const bool piped = st_nn != nullptr;
     FeatLaunch fl{ pcm, stride, c->st.hist, hist_frames, s0, ns, T, logmel };
+    fl.nfr = nfr;
     cudaEvent_t *tl = c->tl[c->tl_count % 8];
     if (timed) NNSP_CUDA(cudaEventRecord(tl[0], st));
     int rc = launch_feature(c->tables, fl, c->device, st);
@@ -1079,14 +1112,14 @@ static int cascade_launch(nnsp_b200_cascade *c, const int16_t *pcm, long long st
         NNSP_CUDA(cudaStreamWaitEvent(st_nn, ev_feat, 0));
         /* the spare history buffer is the one the previous call's replay may still read: roll into it only then */
         if (ev_prev_nn) NNSP_CUDA(cudaStreamWaitEvent(st, ev_prev_nn, 0));
-        if ((rc = launch_hist_roll(pcm, stride / 2, c->st.hist, c->hist2, hist_frames, NNSP_B200_FRAME / 2, s0, ns, T, st))) return rc;
+        if ((rc = launch_hist_roll(pcm, stride / 2, c->st.hist, c->hist2, hist_frames, NNSP_B200_FRAME / 2, s0, ns, T, st, nfr))) return rc;
         st = st_nn;
         if (timed) NNSP_CUDA(cudaEventRecord(tl[2], st));
     }
     CascadeArgs a{};
     for (int i = 0; i < 3; i++) { a.model[i] = c->dm[i].d; a.wimg[i] = c->dm[i].wimg; a.bimg[i] = c->dm[i].bimg; }
     a.tables = c->tables; a.st = c->st; a.stale = c->stale; a.pcm = pcm; a.stride = stride; a.logmel = logmel;
-    a.s0 = s0; a.ns = ns; a.T = T; a.results = results; a.cd = c->cd;
+    a.s0 = s0; a.ns = ns; a.T = T; a.results = results; a.cd = c->cd; a.nfr = nfr;
     if (taps) a.taps = *taps;
     if (cascade_use_split(c, taps)) {
         /* stage-sorted rounds (see the kernels above). Everything is sized for the worst case and reads its true size
@@ -1096,24 +1129,24 @@ static int cascade_launch(nnsp_b200_cascade *c, const int16_t *pcm, long long st
         const int n_inf_max = (T + 1) / 2;
         const int cap = sm_count(c->device);
         NNSP_CUDA(cudaMemsetAsync(ctl, 0, CTL_INTS * sizeof(int), st));
-        cascade_classify_kernel<<<(ns + 255) / 256, 256, 0, st>>>(c->st, c->cd, s0, ns, c->S, c->grp_list, ctl, c->ra, c->fix_list);
+        cascade_classify_kernel<<<(ns + 255) / 256, 256, 0, st>>>(c->st, c->cd, s0, ns, c->S, c->grp_list, ctl, c->ra, c->fix_list, nfr, T);
         NNSP_LAUNCH_CHECK();
         cascade_offsets_kernel<<<1, 1, 0, st>>>(ctl);
         NNSP_LAUNCH_CHECK();
         CascadePostArgs p{};
         for (int i = 0; i < 3; i++) p.model[i] = c->mm[i].d;
         p.st = c->st; p.stale = c->stale; p.logmel = logmel; p.dec = c->dec; p.dec_stride = n_inf_max; p.ra = c->ra;
-        p.s0 = s0; p.ns = ns; p.T = T; p.results = results; p.cd = c->cd;
+        p.s0 = s0; p.ns = ns; p.T = T; p.results = results; p.cd = c->cd; p.nfr = nfr;
         for (int r = 0; r < c->rounds; r++) {
             int *ctl_r = ctl + CTL_ROUND * r, *ctl_prev = ctl + CTL_ROUND * (r - 1);
             const int *queued = r ? c->pend[r & 1] + s0 : nullptr;        /* streams the previous round's walk queued */
             if (r) {
-                cascade_regroup_kernel<<<1, CSORT_THREADS, 0, st>>>(c->st, c->cd, queued, ctl_prev, ctl_r, c->grp_list, c->S, s0, c->ra, T);
+                cascade_regroup_kernel<<<1, CSORT_THREADS, 0, st>>>(c->st, c->cd, queued, ctl_prev, ctl_r, c->grp_list, c->S, s0, c->ra, T, nfr);
                 NNSP_LAUNCH_CHECK();
             }
             {   /* log-mel rows of the first two frames of fresh instances */
                 FixArgs f{};
-                f.tables = c->tables; f.st = c->st; f.pcm = pcm; f.stride = stride; f.ra = c->ra; f.cd = c->cd; f.T = T;
+                f.tables = c->tables; f.st = c->st; f.pcm = pcm; f.stride = stride; f.ra = c->ra; f.cd = c->cd; f.T = T; f.nfr = nfr;
                 f.list = r ? queued : c->fix_list + s0;
                 f.count = r ? ctl_prev + CTL_NEXT : ctl + CTL_FIX;
                 int fb = (ns + 7) / 8;
@@ -1138,7 +1171,7 @@ static int cascade_launch(nnsp_b200_cascade *c, const int16_t *pcm, long long st
                 q.planes0 = c->planes[0]; q.planes1 = c->planes[1];
                 q.dec = c->dec; q.dec_stride = n_inf_max;
                 q.thresh_prob = 0; q.thr_prob = &c->thr->prob[id]; q.thr_stride = (int)(sizeof(CascThr) / sizeof(int16_t));   /* per stream: thr[s].prob[id] */
-                q.tstart = c->ra.tstart; q.tb = c->ra.tb; q.age0 = c->ra.age0; q.lmfix = c->ra.lmfix;
+                q.tstart = c->ra.tstart; q.tb = c->ra.tb; q.age0 = c->ra.age0; q.lmfix = c->ra.lmfix; q.nfr = nfr;
                 if (r == 0 && c->vseq) { q.vseq = c->vseq; q.vseq_rows = c->vseq_rows; }
                 cudaStream_t gs = c->gs[lane_set][k];
                 NNSP_CUDA(cudaStreamWaitEvent(gs, c->ev_fork[lane_set], 0));
@@ -1149,7 +1182,8 @@ static int cascade_launch(nnsp_b200_cascade *c, const int16_t *pcm, long long st
             /* walk the controller over the decisions; a stream that changes stage is cut there and queued for the next round */
             p.list = queued; p.count = r ? ctl_prev + CTL_NEXT : nullptr;
             p.next_list = c->pend[(r + 1) & 1]; p.next_count = ctl_r + CTL_NEXT;
-            cascade_post_kernel<<<(ns + CPOST_WARPS - 1) / CPOST_WARPS, 32 * CPOST_WARPS, 0, st>>>(p);
+            if (nfr) cascade_post_kernel<true><<<(ns + CPOST_WARPS - 1) / CPOST_WARPS, 32 * CPOST_WARPS, 0, st>>>(p);
+            else cascade_post_kernel<false><<<(ns + CPOST_WARPS - 1) / CPOST_WARPS, 32 * CPOST_WARPS, 0, st>>>(p);
             NNSP_LAUNCH_CHECK();
         }
         cascade_ctx_kernel<<<(ns * 32 + 255) / 256, 256, 0, st>>>(p);
@@ -1157,7 +1191,7 @@ static int cascade_launch(nnsp_b200_cascade *c, const int16_t *pcm, long long st
         /* what is still queued after the last round goes to the sequential kernel, longest remainder first */
         a.t0 = c->ra.t0;
         cascade_sort_replay_kernel<<<1, CSORT_THREADS, 0, st>>>(c->pend[c->rounds & 1] + s0, c->replay_sorted + s0,
-                                                                ctl + CTL_ROUND * (c->rounds - 1) + CTL_NEXT, ctl + CTL_REPLAY, c->ra.t0, T);
+                                                                ctl + CTL_ROUND * (c->rounds - 1) + CTL_NEXT, ctl + CTL_REPLAY, c->ra.t0, T, nfr);
         NNSP_LAUNCH_CHECK();
         a.replay_list = c->replay_sorted + s0; a.replay_ctl = ctl + CTL_REPLAY;
     }
@@ -1181,9 +1215,9 @@ static int cascade_launch(nnsp_b200_cascade *c, const int16_t *pcm, long long st
         NNSP_CUDA(cudaEventRecord(tl[3], st));
         c->ev_valid = true; c->last_piped = piped; c->tl_count++;
     }
-    if (!piped && (rc = launch_hist_update(pcm, stride / 2, c->st.hist, hist_frames, NNSP_B200_FRAME / 2, s0, ns, T, st))) return rc;
+    if (!piped && (rc = launch_hist_update(pcm, stride / 2, c->st.hist, hist_frames, NNSP_B200_FRAME / 2, s0, ns, T, st, nfr))) return rc;
     if (c->cd.dmax > 0)
-        rc = launch_hist_update(logmel, (long long)T * NNSP_B200_NMEL, c->st.lmhist, c->cd.dmax, NNSP_B200_NMEL, s0, ns, T, st);
+        rc = launch_hist_update(logmel, (long long)T * NNSP_B200_NMEL, c->st.lmhist, c->cd.dmax, NNSP_B200_NMEL, s0, ns, T, st, nfr);
     return rc;
 }
 
@@ -1395,8 +1429,9 @@ static int cascade_check_pcm(const void *pcm, long long stride, int T)
     return NNSP_B200_OK;
 }
 
-int nnsp_b200_cascade_exec(nnsp_b200_cascade *c, const int16_t *pcm_dev, long long stream_stride, int n_frames,
-                           nnsp_b200_cascade_result *results_dev, const nnsp_b200_taps *taps)
+/* nfr: per-stream frame counts on the device (ragged call), or null */
+static int cascade_exec_dev(nnsp_b200_cascade *c, const int16_t *pcm_dev, long long stream_stride, int n_frames,
+                            const int32_t *nfr, nnsp_b200_cascade_result *results_dev, const nnsp_b200_taps *taps)
 {
     if (!c) return NNSP_B200_ERR_ARG;
     int rc = cascade_check_pcm(pcm_dev, stream_stride, n_frames);
@@ -1412,7 +1447,7 @@ int nnsp_b200_cascade_exec(nnsp_b200_cascade *c, const int16_t *pcm_dev, long lo
         const int i = (int)(c->pipe++ & 1u);
         if (c->nn_pending[i]) NNSP_CUDA(cudaStreamWaitEvent(c->stream, c->ev_nn[i], 0));   /* log-mel buffer i / PCM history in use two calls ago */
         rc = cascade_launch(c, pcm_dev, stream_stride, n_frames, 0, c->S, results_dev, nullptr, c->stream, true, 0,
-                            i ? c->logmel2 : c->logmel, c->nn_stream, c->ev_feat[i], c->nn_pending[i ^ 1] ? c->ev_nn[i ^ 1] : nullptr);
+                            i ? c->logmel2 : c->logmel, c->nn_stream, c->ev_feat[i], c->nn_pending[i ^ 1] ? c->ev_nn[i ^ 1] : nullptr, nfr);
         if (rc) return rc;
         NNSP_CUDA(cudaEventRecord(c->ev_nn[i], c->nn_stream));
         c->nn_pending[i] = true;
@@ -1420,13 +1455,27 @@ int nnsp_b200_cascade_exec(nnsp_b200_cascade *c, const int16_t *pcm_dev, long lo
         return NNSP_B200_OK;
     }
     if ((rc = cascade_join_nn(c, c->stream))) return rc;
-    return cascade_launch(c, pcm_dev, stream_stride, n_frames, 0, c->S, results_dev, taps, c->stream, true);
+    return cascade_launch(c, pcm_dev, stream_stride, n_frames, 0, c->S, results_dev, taps, c->stream, true, 0, nullptr, nullptr,
+                          nullptr, nullptr, nfr);
+}
+
+int nnsp_b200_cascade_exec(nnsp_b200_cascade *c, const int16_t *pcm_dev, long long stream_stride, int n_frames,
+                           nnsp_b200_cascade_result *results_dev, const nnsp_b200_taps *taps)
+{
+    return cascade_exec_dev(c, pcm_dev, stream_stride, n_frames, nullptr, results_dev, taps);
+}
+
+int nnsp_b200_cascade_exec_ragged(nnsp_b200_cascade *c, const int16_t *pcm_dev, long long stream_stride, int max_frames,
+                                  const int32_t *n_frames_dev, nnsp_b200_cascade_result *results_dev, const nnsp_b200_taps *taps)
+{
+    if (!n_frames_dev) { nnsp_set_error("cascade_exec_ragged: null n_frames"); return NNSP_B200_ERR_ARG; }
+    return cascade_exec_dev(c, pcm_dev, stream_stride, max_frames, n_frames_dev, results_dev, taps);
 }
 
 /* one host-buffer call queued on the pipeline streams (slice k always on stream k % 3: consecutive calls are ordered
  * slice by slice by stream order alone); nothing here waits for it */
 static int cascade_enqueue_host(nnsp_b200_cascade *c, const int16_t *pcm, long long stream_stride, int n_frames,
-                                nnsp_b200_cascade_result *results)
+                                nnsp_b200_cascade_result *results, const int32_t *nfr = nullptr)
 {
     int rc = cascade_check_pcm(pcm, stream_stride, n_frames);
     if (rc) return rc;
@@ -1464,10 +1513,15 @@ static int cascade_enqueue_host(nnsp_b200_cascade *c, const int16_t *pcm, long l
         NNSP_CUDA(cudaDeviceSynchronize());
         NNSP_CUDA(cudaMalloc(&c->d_raw, (size_t)c->S * c->d_pcm_frames * NNSP_B200_FRAME * sizeof(uint32_t)));
     }
+    if (nfr && !c->d_nfr) {
+        NNSP_CUDA(cudaDeviceSynchronize());
+        NNSP_CUDA(cudaMalloc(&c->d_nfr, (size_t)2 * c->S * sizeof(int32_t)));
+    }
     c->host_inflight = true;
     const int nsl = c->S >= 4096 ? 8 : (c->S >= 256 ? 4 : 1);
     const int buf = (int)(c->host_calls++ & 1);
     int16_t *dpcm = c->d_pcm + (size_t)buf * c->S * c->d_pcm_frames * NNSP_B200_FRAME;
+    int32_t *dnfr = nfr ? c->d_nfr + (size_t)buf * c->S : nullptr;     /* the counts of a ragged call, buffered like the PCM */
     auto slice = [&](int k, int *s0, int *s1) {
         *s0 = (int)(((long long)c->S * k / nsl) & ~15LL);
         *s1 = (k == nsl - 1) ? c->S : (int)(((long long)c->S * (k + 1) / nsl) & ~15LL);
@@ -1485,6 +1539,8 @@ static int cascade_enqueue_host(nnsp_b200_cascade *c, const int16_t *pcm, long l
                 NNSP_CUDA(cudaMemcpy2DAsync(dpcm + (size_t)s0 * dstride, dstride * sizeof(int16_t),
                                             pcm + (size_t)s0 * stream_stride, stream_stride * sizeof(int16_t),
                                             dstride * sizeof(int16_t), (size_t)(s1 - s0), cudaMemcpyHostToDevice, c->h2d_stream));
+            if (dnfr)
+                NNSP_CUDA(cudaMemcpyAsync(dnfr + s0, nfr + s0, (size_t)(s1 - s0) * sizeof(int32_t), cudaMemcpyHostToDevice, c->h2d_stream));
             NNSP_CUDA(cudaEventRecord(c->ev_h2d[buf][k], c->h2d_stream));
         }
     for (int k = 0; k < nsl; k++) {
@@ -1498,9 +1554,12 @@ static int cascade_enqueue_host(nnsp_b200_cascade *c, const int16_t *pcm, long l
                                         raw + (size_t)s0 * stream_stride, stream_stride * sizeof(uint32_t),
                                         dstride * sizeof(uint32_t), (size_t)(s1 - s0), cudaMemcpyHostToDevice, st));
             if ((rc = launch_ingest(c->d_raw + (size_t)s0 * dstride, dpcm + (size_t)s0 * dstride, (long long)(s1 - s0) * T, c->device, st))) return rc;
+            if (dnfr)
+                NNSP_CUDA(cudaMemcpyAsync(dnfr + s0, nfr + s0, (size_t)(s1 - s0) * sizeof(int32_t), cudaMemcpyHostToDevice, st));
         } else
             NNSP_CUDA(cudaStreamWaitEvent(st, c->ev_h2d[buf][k], 0));
-        rc = cascade_launch(c, dpcm, dstride, T, s0, s1 - s0, results ? c->d_res : nullptr, nullptr, st, false, k);
+        rc = cascade_launch(c, dpcm, dstride, T, s0, s1 - s0, results ? c->d_res : nullptr, nullptr, st, false, k,
+                            nullptr, nullptr, nullptr, nullptr, dnfr);
         if (rc) return rc;
         NNSP_CUDA(cudaEventRecord(c->ev_read[buf][k], st));         /* every reader of the slice's PCM has joined st by now */
         c->read_valid[buf][k] = true;
@@ -1527,6 +1586,24 @@ int nnsp_b200_cascade_exec_host_async(nnsp_b200_cascade *c, const int16_t *pcm, 
 {
     if (!c) return NNSP_B200_ERR_ARG;
     int rc = cascade_enqueue_host(c, pcm, stream_stride, n_frames, results);
+    if (rc) return rc;
+    const long long t = ++c->host_seq;
+    for (int j = 0; j < 3; j++) NNSP_CUDA(cudaEventRecord(c->host_ev[t % CS_HOST_RING][j], c->xs[j]));
+    if (ticket) *ticket = t;
+    return NNSP_B200_OK;
+}
+
+int nnsp_b200_cascade_exec_host_ragged_async(nnsp_b200_cascade *c, const int16_t *pcm, long long stream_stride, int max_frames,
+                                             const int32_t *n_frames, nnsp_b200_cascade_result *results, long long *ticket)
+{
+    if (!c) return NNSP_B200_ERR_ARG;
+    if (!n_frames) { nnsp_set_error("cascade_exec_host_ragged_async: null n_frames"); return NNSP_B200_ERR_ARG; }
+    for (int s = 0; s < c->S; s++)                                   /* checked before anything is queued */
+        if (n_frames[s] < 0 || n_frames[s] > max_frames) {
+            nnsp_set_error("cascade_exec_host_ragged_async: n_frames[%d] = %d is outside [0, %d]", s, (int)n_frames[s], max_frames);
+            return NNSP_B200_ERR_ARG;
+        }
+    int rc = cascade_enqueue_host(c, pcm, stream_stride, max_frames, results, n_frames);
     if (rc) return rc;
     const long long t = ++c->host_seq;
     for (int j = 0; j < 3; j++) NNSP_CUDA(cudaEventRecord(c->host_ev[t % CS_HOST_RING][j], c->xs[j]));
@@ -1614,7 +1691,7 @@ void nnsp_b200_cascade_destroy(nnsp_b200_cascade *c)
     for (int i = 0; i < 3; i++) if (c->have[i]) free_model(&c->dm[i]);
     cudaFree(c->st.ctx); cudaFree(c->st.h); cudaFree(c->st.c); cudaFree(c->st.scal); cudaFree(c->st.casc);
     cudaFree(c->st.hist); cudaFree(c->st.lmhist); cudaFree(c->stale); cudaFree(c->thr); cudaFree(c->vseq);
-    cudaFree(c->logmel); cudaFree(c->logmel2); cudaFree(c->hist2); cudaFree(c->d_pcm); cudaFree(c->d_res); cudaFree(c->d_raw);
+    cudaFree(c->logmel); cudaFree(c->logmel2); cudaFree(c->hist2); cudaFree(c->d_pcm); cudaFree(c->d_res); cudaFree(c->d_raw); cudaFree(c->d_nfr);
     if (c->nn_stream) cudaStreamDestroy(c->nn_stream);
     for (auto e : c->ev_feat) if (e) cudaEventDestroy(e);
     for (auto e : c->ev_nn) if (e) cudaEventDestroy(e);

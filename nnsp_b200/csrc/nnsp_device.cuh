@@ -9,6 +9,15 @@ namespace nnsp {
 enum { LAYER_FC = 0, LAYER_LSTM = 1 };
 enum { ACT_RELU6 = 0, ACT_TANH = 1, ACT_SIGMOID = 2, ACT_LINEAR = 3 };
 
+/* Frames stream s advances in a call of T frames. nfr: the per-stream counts of a ragged cascade call
+ * (nnsp_b200_cascade_exec_ragged), clamped to [0, T]; null for every other call, which advances every stream by T. */
+__device__ __forceinline__ int stream_frames(const int32_t *nfr, long long s, int T)
+{
+    if (!nfr) return T;
+    const int n = __ldg(nfr + s);
+    return n < 0 ? 0 : (n > T ? T : n);
+}
+
 /* ---- Q15 products ------------------------------------------------------------------- */
 /* (a*b) >> 15 with a 64-bit intermediate and floor: the ">>= 15" of complex.c:66-69. The
  * int32 saturation that follows in the reference cannot fire for int16 PCM input: with the

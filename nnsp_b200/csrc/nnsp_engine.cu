@@ -258,10 +258,15 @@ struct FeatSmem {
     int32_t norm[84];              /* mean[40], stdR[40], rshift: only when the kernel standardises */
 };
 
+/* RAGGED (a ragged cascade call, nfr != null): stream s has stream_frames(nfr, s, T) frames; a later frame reads no PCM
+ * and writes no row, and a warp whose two frames are both past their streams' counts skips the pair. The uniform
+ * instantiation is the kernel as it was before ragged calls existed, instruction for instruction. */
+template <bool RAGGED>
 __global__ void __launch_bounds__(FEAT_THREADS, FEAT_CTAS_PER_SM)
 feat_kernel(const DevTables *__restrict__ tables, const int16_t *__restrict__ pcm, long long stride,
             const int16_t *__restrict__ hist, int hist_frames, int s0, int ns, int T,
-            int32_t *__restrict__ logmel, const int32_t *__restrict__ norm, int16_t *__restrict__ feat16)
+            int32_t *__restrict__ logmel, const int32_t *__restrict__ norm, int16_t *__restrict__ feat16,
+            const int32_t *__restrict__ nfr)
 {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     FeatSmem &sm = *reinterpret_cast<FeatSmem *>(smem_raw);
@@ -275,16 +280,23 @@ feat_kernel(const DevTables *__restrict__ tables, const int16_t *__restrict__ pc
     const int hist_len = hist_frames * NNSP_B200_FRAME;
     for (long long f0 = ((long long)blockIdx.x * FEAT_WARPS + warp) * 2; f0 < F; f0 += (long long)gridDim.x * FEAT_WARPS * 2) {
         const long long f = f0 + half;
-        const bool valid = f < F;
+        bool valid = f < F;
         const long long fc = valid ? f : 0;
         const int s = s0 + (int)(fc / T), t = (int)(fc % T);
+        if (RAGGED) {
+            valid = valid && t < stream_frames(nfr, s, T);
+            if (!__any_sync(0xffffffffu, valid)) continue;              /* warp-uniform: neither frame is live */
+        }
         /* the 480-sample window starts two frames back: word L + 16a of it comes from this call's PCM or, for
          * the first two frames, from the carried history (both 4-byte aligned; immediates after unrolling) */
         const int base = (t - 2) * NNSP_B200_FRAME;                        /* first sample of the window */
         const unsigned int *pw = reinterpret_cast<const unsigned int *>(pcm + (long long)s * stride + base) + L;
         const unsigned int *hw = reinterpret_cast<const unsigned int *>(hist + (long long)s * hist_len + hist_len + base) + L;
         const int pth = (2 - t) * (NNSP_B200_FRAME / 2);                   /* pairs below pth precede the call */
-        auto load_pair = [&](int a, int p) -> uint32_t { return (p < pth) ? __ldg(hw + 16 * a) : __ldg(pw + 16 * a); };
+        auto load_pair = [&](int a, int p) -> uint32_t {
+            if (RAGGED && !valid) return 0u;
+            return (p < pth) ? __ldg(hw + 16 * a) : __ldg(pw + 16 * a);
+        };
         const long long row = ((long long)s * T + t) * NNSP_B200_NMEL;
         frame_logmel<false>(sm.tb, fs, L, load_pair, logmel + row, valid, FeatDump{}, snorm, feat16 + row);
     }
@@ -296,7 +308,8 @@ int launch_feature(const DevTables *tb, const FeatLaunch &a, int device, cudaStr
     static std::mutex attr_mu;                         /* host threads may drive separate handles on one device */
     std::unique_lock<std::mutex> attr_lk(attr_mu);
     if (!attr_set[device]) {
-        NNSP_CUDA(cudaFuncSetAttribute(feat_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(FeatSmem)));
+        NNSP_CUDA(cudaFuncSetAttribute(feat_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(FeatSmem)));
+        NNSP_CUDA(cudaFuncSetAttribute(feat_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(FeatSmem)));
         attr_set[device] = true;
     }
     attr_lk.unlock();
@@ -320,22 +333,34 @@ int launch_feature(const DevTables *tb, const FeatLaunch &a, int device, cudaStr
     static const int pad = [] { const char *e = getenv("NNSP_B200_FEAT_SMEM_PAD"); return e ? atoi(e) : 0; }();   /* measurement knob: fewer resident CTAs */
     if (pad > 0) {
         static bool pad_set[64] = { false };
-        if (!pad_set[device]) { NNSP_CUDA(cudaFuncSetAttribute(feat_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(FeatSmem) + pad)); pad_set[device] = true; }
+        if (!pad_set[device]) {
+            NNSP_CUDA(cudaFuncSetAttribute(feat_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(FeatSmem) + pad));
+            NNSP_CUDA(cudaFuncSetAttribute(feat_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(FeatSmem) + pad));
+            pad_set[device] = true;
+        }
     }
-    feat_kernel<<<(unsigned)blocks, FEAT_THREADS, sizeof(FeatSmem) + (pad > 0 ? pad : 0), st>>>(tb, a.pcm, a.stride, a.hist, a.hist_frames,
-                                                                            a.s0, a.ns, a.T, a.logmel, a.norm, a.feat16);
+    const size_t smem = sizeof(FeatSmem) + (pad > 0 ? pad : 0);
+    if (a.nfr)
+        feat_kernel<true><<<(unsigned)blocks, FEAT_THREADS, smem, st>>>(tb, a.pcm, a.stride, a.hist, a.hist_frames, a.s0, a.ns, a.T,
+                                                                       a.logmel, a.norm, a.feat16, a.nfr);
+    else
+        feat_kernel<false><<<(unsigned)blocks, FEAT_THREADS, smem, st>>>(tb, a.pcm, a.stride, a.hist, a.hist_frames, a.s0, a.ns, a.T,
+                                                                        a.logmel, a.norm, a.feat16, nullptr);
     NNSP_LAUNCH_CHECK();
     return NNSP_B200_OK;
 }
 
 /* keep the newest hist_frames frames of (previous history ++ this call) for the next call; a "frame" is
- * wpf 32-bit words (80 for PCM, 40 for log-mel rows) */
+ * wpf 32-bit words (80 for PCM, 40 for log-mel rows). A ragged cascade call appends stream s's own frame count. */
+template <bool RAGGED>
 __global__ void hist_kernel(const unsigned int *__restrict__ src, long long stride_words, unsigned int *__restrict__ hist,
-                            int hist_frames, int wpf, int s0, int ns, int T)
+                            int hist_frames, int wpf, int s0, int ns, int T_call, const int32_t *__restrict__ nfr)
 {
     const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
     if (warp >= ns) return;
     const int s = s0 + warp;
+    const int T = RAGGED ? stream_frames(nfr, s, T_call) : T_call;
+    if (RAGGED && T == 0) return;
     const int words = hist_frames * wpf;
     const int keep = hist_frames - T;                                  /* frames of old history that survive (T < hist_frames) */
     unsigned int *h = hist + (long long)s * words;
@@ -359,12 +384,15 @@ __global__ void hist_kernel(const unsigned int *__restrict__ src, long long stri
 }
 
 /* out of place: hist_out <- newest hist_frames frames of (hist_in ++ src[0..T)) */
+template <bool RAGGED>
 __global__ void hist_roll_kernel(const unsigned int *__restrict__ src, long long stride_words, const unsigned int *__restrict__ hist_in,
-                                 unsigned int *__restrict__ hist_out, int hist_frames, int wpf, int s0, int ns, int T)
+                                 unsigned int *__restrict__ hist_out, int hist_frames, int wpf, int s0, int ns, int T_call,
+                                 const int32_t *__restrict__ nfr)
 {
     const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
     if (warp >= ns) return;
     const long long s = s0 + warp;
+    const int T = RAGGED ? stream_frames(nfr, s, T_call) : T_call;            /* 0: hist_out is hist_in */
     const int words = hist_frames * wpf, keep = (hist_frames - T) * wpf;       /* words of the old history that survive */
     const unsigned int *hi = hist_in + s * words, *p = src + s * stride_words;
     unsigned int *ho = hist_out + s * words;
@@ -373,23 +401,23 @@ __global__ void hist_roll_kernel(const unsigned int *__restrict__ src, long long
 }
 
 int launch_hist_roll(const void *src, long long stride_words, const void *hist_in, void *hist_out, int hist_frames,
-                     int words_per_frame, int s0, int ns, int T, cudaStream_t st)
+                     int words_per_frame, int s0, int ns, int T, cudaStream_t st, const int32_t *nfr)
 {
     if (ns <= 0 || T <= 0 || hist_frames <= 0) return NNSP_B200_OK;
     const int threads = 256, blocks = (ns * 32 + threads - 1) / threads;
-    hist_roll_kernel<<<blocks, threads, 0, st>>>((const unsigned int *)src, stride_words, (const unsigned int *)hist_in,
-                                                 (unsigned int *)hist_out, hist_frames, words_per_frame, s0, ns, T);
+    (nfr ? hist_roll_kernel<true> : hist_roll_kernel<false>)<<<blocks, threads, 0, st>>>((const unsigned int *)src, stride_words, (const unsigned int *)hist_in,
+                                                 (unsigned int *)hist_out, hist_frames, words_per_frame, s0, ns, T, nfr);
     NNSP_LAUNCH_CHECK();
     return NNSP_B200_OK;
 }
 
 int launch_hist_update(const void *src, long long stride_words, void *hist, int hist_frames, int words_per_frame,
-                       int s0, int ns, int T, cudaStream_t st)
+                       int s0, int ns, int T, cudaStream_t st, const int32_t *nfr)
 {
     if (ns <= 0 || T <= 0 || hist_frames <= 0) return NNSP_B200_OK;
     const int threads = 256, blocks = (ns * 32 + threads - 1) / threads;
-    hist_kernel<<<blocks, threads, 0, st>>>((const unsigned int *)src, stride_words, (unsigned int *)hist, hist_frames,
-                                            words_per_frame, s0, ns, T);
+    (nfr ? hist_kernel<true> : hist_kernel<false>)<<<blocks, threads, 0, st>>>((const unsigned int *)src, stride_words, (unsigned int *)hist, hist_frames,
+                                            words_per_frame, s0, ns, T, nfr);
     NNSP_LAUNCH_CHECK();
     return NNSP_B200_OK;
 }

@@ -54,15 +54,18 @@ struct FeatLaunch {
     int32_t *logmel;                          /* [S][T][40] */
     const int32_t *norm = nullptr;            /* device: mean[40], stdR[40], rshift -> write feat16 instead of logmel */
     int16_t *feat16 = nullptr;                /* [S][T][40] standardised rows (feature_module.c:67-73) */
+    const int32_t *nfr = nullptr;             /* ragged cascade call: stream s has stream_frames(nfr, s, T) frames; the rows
+                                                 of its later frames are neither computed nor written, their PCM not read */
 };
 int launch_feature(const DevTables *tb, const FeatLaunch &a, int device, cudaStream_t st);
-/* hist <- newest hist_frames frames of (hist ++ src[0..T)); frames are words_per_frame 32-bit words */
+/* hist <- newest hist_frames frames of (hist ++ src[0..T)); frames are words_per_frame 32-bit words. nfr (ragged
+ * cascade call): stream s appends only its first stream_frames(nfr, s, T) frames, none when that is 0 */
 int launch_hist_update(const void *src, long long stride_words, void *hist, int hist_frames, int words_per_frame,
-                       int s0, int ns, int T, cudaStream_t st);
+                       int s0, int ns, int T, cudaStream_t st, const int32_t *nfr = nullptr);
 /* the same, out of place (hist_in and hist_out distinct): lets the next call's front end start while kernels of this
  * call still read the old history */
 int launch_hist_roll(const void *src, long long stride_words, const void *hist_in, void *hist_out, int hist_frames,
-                     int words_per_frame, int s0, int ns, int T, cudaStream_t st);
+                     int words_per_frame, int s0, int ns, int T, cudaStream_t st, const int32_t *nfr = nullptr);
 
 
 /* audio_frame_callback's conditioning (evb/src/main_nnsp.cc:58-65) of n_frames consecutive 160-sample frames, raw 32-bit
@@ -123,6 +126,9 @@ struct SplitGroup {
     /* cascade, first round: scratch for the streams' standardised window rows, [S][vseq_rows][40] (vseq_kernel); with it
      * layer 0 runs on the tcgen05 kernel. Null: seg_kernel<2> standardises while staging (later rounds, few streams) */
     int16_t *vseq = nullptr; int vseq_rows = 0;
+    /* ragged cascade call (null otherwise): stream s ends at frame stream_frames(nfr, s, T), so a row of a round has
+     * (Ts - tstart[s] + 1) / 2 inferences */
+    const int32_t *nfr = nullptr;
 };
 int launch_split_layers(const MmaDeviceModel &mm, const SplitGroup &q, int device, cudaStream_t st);
 int split_supported(const MmaDeviceModel &mm);

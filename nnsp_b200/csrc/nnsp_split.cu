@@ -196,6 +196,7 @@ struct SegArgs {
     const int16_t *thr_prob; int thr_stride;   /* per-stream thresholds (cascade), else null */
     const int *tstart, *tb, *age0;  /* cascade rounds: per-stream first inference frame, life begin, age there (SplitGroup) */
     const int32_t *lmfix;           /* [S][2][40] log-mel rows of an instance's first two frames */
+    const int32_t *nfr;             /* ragged cascade call: per-stream end frame (SplitGroup) */
 };
 
 /* Where the outputs of one fc layer of one (tile, inference) row block go. */
@@ -335,7 +336,7 @@ __global__ void __launch_bounds__(SEG_THREADS, SEG_MINB)
 seg_kernel(SegArgs a)
 {
     constexpr bool FROM_FEAT = MODE != 0;
-    __shared__ int sids[16], s_ts[16], s_tb[16], s_ag[16], s_ninf;
+    __shared__ int sids[16], s_ts[16], s_te[16], s_tb[16], s_ag[16], s_ninf;
     extern __shared__ __align__(128) unsigned char smem[];
     const bool per_row = a.tstart != nullptr;                     /* cascade rounds: every row has its own start frame */
     {   /* nothing selected (a later round of the cascade, an empty group) or more CTAs than work items: leave before the prologue */
@@ -414,7 +415,9 @@ seg_kernel(SegArgs a)
                 int ts = a.first, tbv = 0, ag = 2;
                 if (per_row && tid < nvalid) { ts = a.tstart[sid]; tbv = a.tb[sid]; ag = a.age0[sid]; }
                 sids[tid] = sid; s_ts[tid] = ts; s_tb[tid] = tbv; s_ag[tid] = ag;
-                int ni = (tid < nvalid) ? (per_row ? (ts < T ? (T - ts + 1) >> 1 : 0) : a.n_inf) : 0;
+                const int Ts = per_row && tid < nvalid ? stream_frames(a.nfr, sid, T) : T;
+                s_te[tid] = Ts;
+                int ni = (tid < nvalid) ? (per_row ? (ts < Ts ? (Ts - ts + 1) >> 1 : 0) : a.n_inf) : 0;
                 for (int o = 8; o; o >>= 1) ni = max(ni, __shfl_xor_sync(0x0000ffffu, ni, o));
                 if (tid == 0) s_ninf = ni;
             }
@@ -479,7 +482,7 @@ seg_kernel(SegArgs a)
                                 if (life < 0) {                                      /* before that: the instance's stored context rows 1..5 */
                                     const uint2 c = *reinterpret_cast<const uint2 *>(a.ctx + s * 240 + (6 + life) * 40 + x * 4);
                                     v[u] = make_int4((int16_t)(c.x & 0xffff), (int32_t)c.x >> 16, (int16_t)(c.y & 0xffff), (int32_t)c.y >> 16);
-                                } else if (f < T) {
+                                } else if (f < s_te[r]) {                            /* frames past the row's own end stage as zeros */
                                     const int la = life + s_ag[r], fr = f - a.dback;
                                     const int32_t *row = (la < 2) ? a.lmfix + (s * 2 + la) * NNSP_B200_NMEL     /* STFT buffer still partly zero */
                                                        : (fr >= 0) ? a.logmel + (s * T + fr) * NNSP_B200_NMEL
@@ -601,6 +604,7 @@ struct ScanArgs {
     int16_t *tap_act, *tap_h;
     int32_t *tap_c;
     const int *tstart;              /* cascade rounds: per-stream first inference frame (null: every row has n_inf inferences) */
+    const int32_t *nfr;             /* ragged cascade call: per-stream end frame (SplitGroup) */
 };
 
 __device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity)
@@ -699,7 +703,10 @@ scan_kernel(ScanArgs a)
         /* inferences of this row: the tile runs as many steps as its longest row; a row's state is final after its own
          * last step and is stored right there (cascade rounds start streams at different frames) */
         int ni = 0;
-        if (r < nvalid) { ni = a.n_inf; if (per_row) { const int ts = a.tstart[sid]; ni = ts < a.T ? (a.T - ts + 1) >> 1 : 0; } }
+        if (r < nvalid) {
+            ni = a.n_inf;
+            if (per_row) { const int ts = a.tstart[sid], Ts = stream_frames(a.nfr, sid, a.T); ni = ts < Ts ? (Ts - ts + 1) >> 1 : 0; }
+        }
         s_last[r] = ni - 1;
         for (int o = 8; o; o >>= 1) ni = max(ni, __shfl_xor_sync(0x0000ffffu, ni, o));
         if (r == 0) s_ninf = ni;
@@ -1059,6 +1066,7 @@ struct VseqArgs {
     const int16_t *ctx;
     int T, dmax, dback, rows;
     int16_t *vseq;
+    const int32_t *nfr;
 };
 __global__ void __launch_bounds__(256) vseq_kernel(VseqArgs a)
 {
@@ -1068,8 +1076,8 @@ __global__ void __launch_bounds__(256) vseq_kernel(VseqArgs a)
     for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (long long)gridDim.x * blockDim.x) {
         const int p = (int)(e / (a.rows * 10)), rem = (int)(e - (long long)p * a.rows * 10), v = rem / 10, x = rem - v * 10;
         const long long s = a.list[p];
-        const int ts = a.tstart[s];
-        const int ninf = ts < a.T ? (a.T - ts + 1) >> 1 : 0;
+        const int ts = a.tstart[s], Ts = stream_frames(a.nfr, s, a.T);
+        const int ninf = ts < Ts ? (Ts - ts + 1) >> 1 : 0;
         if (v >= 2 * ninf + 4 || ninf == 0) continue;
         const int f = ts - 5 + v, life = f - a.tb[s];
         int16_t w[4] = { 0, 0, 0, 0 };
@@ -1154,7 +1162,7 @@ int launch_split_layers(const MmaDeviceModel &mm, const SplitGroup &q, int devic
                 VseqArgs v{};
                 v.model = mm.d; v.list = q.list; v.count = q.count; v.tstart = q.tstart; v.tb = q.tb; v.age0 = q.age0;
                 v.logmel = q.logmel; v.lmhist = q.lmhist; v.lmfix = q.lmfix; v.ctx = q.ctx;
-                v.T = q.T; v.dmax = q.dmax; v.dback = q.dback; v.rows = q.vseq_rows; v.vseq = q.vseq;
+                v.T = q.T; v.dmax = q.dmax; v.dback = q.dback; v.rows = q.vseq_rows; v.vseq = q.vseq; v.nfr = q.nfr;
                 long long work = (long long)q.max_streams * q.vseq_rows * 10;
                 int grid = (int)((work + 255) / 256);
                 grid = grid < 1 ? 1 : (grid > 8 * sm_count(device) ? 8 * sm_count(device) : grid);
@@ -1167,7 +1175,7 @@ int launch_split_layers(const MmaDeviceModel &mm, const SplitGroup &q, int devic
             a.T = q.T; a.first = q.first; a.n_inf = q.n_inf; a.nchunks = (q.n_inf + TC5_KC - 1) / TC5_KC;
             a.pa = D->pa; a.tile_bytes = tile_bytes;
             a.feat16 = q.feat16; a.ctx = q.ctx; a.out_planes = bufs[which];
-            if (tc5_round) { a.list = q.list; a.count = q.count; a.tile_off = q.tile_off; a.tstart = q.tstart; a.vseq = q.vseq; a.vf = q.vseq_rows; }
+            if (tc5_round) { a.list = q.list; a.count = q.count; a.tile_off = q.tile_off; a.tstart = q.tstart; a.vseq = q.vseq; a.vf = q.vseq_rows; a.nfr = q.nfr; }
             const int nitems = (((tc5_round ? q.max_streams : q.ns) + 1) / 2) * a.nchunks;
             const int grid = nitems < sm_count(device) ? nitems : sm_count(device);
             seg0_tc5_kernel<<<grid, TC5_THREADS, sizeof(Tc5Smem) + 1024, st>>>(a);
@@ -1198,7 +1206,7 @@ int launch_split_layers(const MmaDeviceModel &mm, const SplitGroup &q, int devic
             a.ctx = q.ctx; a.in_planes = cur_in;
             a.out_planes = (l1 < D->numlayers) ? bufs[which] : nullptr;
             a.dec = q.dec; a.tap_act = tp.act; a.tap_logits = tp.logits; a.ao0 = ao; a.thresh_prob = q.thresh_prob; a.thr_prob = q.thr_prob; a.thr_stride = q.thr_stride;
-            a.tstart = q.tstart; a.tb = q.tb; a.age0 = q.age0; a.lmfix = q.lmfix;
+            a.tstart = q.tstart; a.tb = q.tb; a.age0 = q.age0; a.lmfix = q.lmfix; a.nfr = q.nfr;
             int per_sm = (int)((227 * 1024) / (lay.total + 1024));
             per_sm = per_sm < 1 ? 1 : (per_sm > SEG_MINB ? SEG_MINB : per_sm);     /* __launch_bounds__(256, SEG_MINB) */
             int grid = sm_count(device) * per_sm;
@@ -1220,7 +1228,7 @@ int launch_split_layers(const MmaDeviceModel &mm, const SplitGroup &q, int devic
             a.ho = ho; a.hs = q.h_stride; a.ao = ao; a.act_stride = D->act_stride; a.tap_out = (li < D->numlayers - 1);
             a.sel = sel; a.T = q.T; a.first = q.first; a.n_inf = q.n_inf; a.tile_bytes = tile_bytes;
             a.xin = cur_in; a.hout = bufs[which]; a.h = q.h; a.c = q.c;
-            a.tap_act = tp.act; a.tap_h = tp.hstate; a.tap_c = tp.cstate; a.tstart = q.tstart;
+            a.tap_act = tp.act; a.tap_h = tp.hstate; a.tap_c = tp.cstate; a.tstart = q.tstart; a.nfr = q.nfr;
             const size_t smem = scan_smem(D, L);
             /* the shipped layers get their k-step counts compiled in: VAD 28 -> 28 (1 k-step), KWS 64 -> 64 (2), S2I 72 -> 72 (3) */
             const int kq = (L.kt == L.ktr) ? L.kt : 0;

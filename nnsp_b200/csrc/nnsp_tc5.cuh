@@ -71,11 +71,13 @@ struct Tc5Args {
     const int16_t *ctx;             /* [S][240] */
     uint8_t *out_planes;
     /* cascade rounds (vseq != null): the selection is a device-side list (count, plane tile offset as in StreamSel), stream s
-     * has its own first inference frame tstart[s], hence (T - tstart[s] + 1) / 2 inferences, and its window rows were
+     * has its own first inference frame tstart[s], hence (Ts - tstart[s] + 1) / 2 inferences (Ts: its end frame, T unless
+     * the call is ragged), and its window rows were
      * written by vseq_kernel: vseq[s][v] = row of frame tstart[s] - 5 + v, already standardised, context rows included */
     const int *list, *count, *tile_off, *tstart;
     const int16_t *vseq;
     int vf;                         /* rows per stream in vseq */
+    const int32_t *nfr;             /* ragged cascade call: stream s ends at frame stream_frames(nfr, s, T) (null: at T) */
 };
 __device__ __forceinline__ int tc5_nsel(const Tc5Args &a) { return a.list ? *a.count : a.ns; }
 __device__ __forceinline__ long long tc5_sid(const Tc5Args &a, int p) { return a.list ? a.list[p] : (long long)a.s0 + p; }
@@ -84,7 +86,11 @@ __device__ __forceinline__ int tc5_nk(const Tc5Args &a, int p, int nsel, int k0)
 {
     if (p >= nsel) return 0;
     int ninf = a.n_inf;
-    if (a.vseq) { const int ts = a.tstart[tc5_sid(a, p)]; ninf = ts < a.T ? (a.T - ts + 1) >> 1 : 0; }
+    if (a.vseq) {
+        const long long s = tc5_sid(a, p);
+        const int ts = a.tstart[s], Ts = stream_frames(a.nfr, s, a.T);
+        ninf = ts < Ts ? (Ts - ts + 1) >> 1 : 0;
+    }
     return max(0, min(TC5_KC, ninf - k0));
 }
 
@@ -189,23 +195,23 @@ seg0_tc5_kernel(Tc5Args a)
             const int chunk = item / npairs, pair = item - chunk * npairs;
             const int k0 = chunk * TC5_KC;
             const int f_lo = a.first - 5 + 2 * k0, nctx = (!a.vseq && f_lo < 0) ? -f_lo : 0;
-            int nfr[TC5_STREAMS];
+            int nrow[TC5_STREAMS];
             uint32_t bytes = 0;
             for (int q = 0; q < TC5_STREAMS; q++) {
                 const int nk = tc5_nk(a, 2 * pair + q, nsel, k0);
-                nfr[q] = nk > 0 ? 2 * nk + 4 : 0;
-                bytes += (uint32_t)(nfr[q] * 80);
+                nrow[q] = nk > 0 ? 2 * nk + 4 : 0;
+                bytes += (uint32_t)(nrow[q] * 80);
             }
             asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" :: "r"(smem_u32(&sm.raw_full[rb])), "r"(bytes) : "memory");
             for (int q = 0; q < TC5_STREAMS; q++) {
-                if (!nfr[q]) continue;
+                if (!nrow[q]) continue;
                 const long long s = tc5_sid(a, 2 * pair + q);
                 if (nctx)
                     asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
                                  :: "r"(smem_u32(&sm.raw[rb][q][0])), "l"(a.ctx + s * 240 + (6 + f_lo) * 40), "r"((uint32_t)(nctx * 80)), "r"(smem_u32(&sm.raw_full[rb])) : "memory");
                 const int16_t *src = a.vseq ? a.vseq + (s * a.vf + 2 * k0) * 40 : a.feat16 + (s * T + f_lo + nctx) * 40;
                 asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                             :: "r"(smem_u32(&sm.raw[rb][q][nctx * 40])), "l"(src), "r"((uint32_t)((nfr[q] - nctx) * 80)), "r"(smem_u32(&sm.raw_full[rb])) : "memory");
+                             :: "r"(smem_u32(&sm.raw[rb][q][nctx * 40])), "l"(src), "r"((uint32_t)((nrow[q] - nctx) * 80)), "r"(smem_u32(&sm.raw_full[rb])) : "memory");
             }
         };
         if (ptid == 0)
@@ -219,9 +225,9 @@ seg0_tc5_kernel(Tc5Args a)
             if (use >= 1) tc5_wait(&sm.mma_done[b], (uint32_t)((use - 1) & 1));                  /* the MMAs that read a[b] are complete */
             tc5_wait(&sm.raw_full[rb], (uint32_t)((n / TC5_RING) & 1));
             const int chunk = item / npairs, pair = item - chunk * npairs;
-            const int nfr = 2 * max(tc5_nk(a, 2 * pair, nsel, chunk * TC5_KC), tc5_nk(a, 2 * pair + 1, nsel, chunk * TC5_KC)) + 4;   /* rows past a stream's own count are stale: their slots are dropped */
-            for (int e = ptid; e < TC5_STREAMS * nfr; e += TC5_CONV_THREADS) {
-                const int q = e / nfr, fr = e - q * nfr;
+            const int nrow = 2 * max(tc5_nk(a, 2 * pair, nsel, chunk * TC5_KC), tc5_nk(a, 2 * pair + 1, nsel, chunk * TC5_KC)) + 4;   /* rows past a stream's own count are stale: their slots are dropped */
+            for (int e = ptid; e < TC5_STREAMS * nrow; e += TC5_CONV_THREADS) {
+                const int q = e / nrow, fr = e - q * nrow;
                 const uint4 *src = reinterpret_cast<const uint4 *>(&sm.raw[rb][q][fr * 40]);
                 const uint4 v0 = src[0], v1 = src[1], v2 = src[2], v3 = src[3], v4 = src[4];
                 uint4 h0, l0, h1, l1;
