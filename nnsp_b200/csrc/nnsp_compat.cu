@@ -103,13 +103,19 @@ __global__ void __launch_bounds__(32) legacy_kernel(LegacyIO *io, const DevTable
     if (lane < SC_N) io->scal[lane] = ws->scal[lane];
 }
 
+/* an uploaded model and the bytes of the NeuralNetClass it was built from */
+struct LegacyModel {
+    NeuralNetClass net;
+    DeviceModel *dm;
+};
+
 struct LegacyCtx {
     int device = 0;
     bool ready = false;
     const DevTables *tables = nullptr;
     LegacyIO *h_io = nullptr, *d_io = nullptr;
     cudaStream_t stream = nullptr;
-    std::map<const void *, DeviceModel *> models;          /* keyed by NeuralNetClass* */
+    std::map<const void *, LegacyModel> models;            /* keyed by NeuralNetClass* */
 };
 static LegacyCtx g_lg;
 static std::mutex g_lg_mu;
@@ -137,10 +143,20 @@ static void legacy_init()
     g_lg.ready = true;
 }
 
+/* The reference reads the NeuralNetClass on every call, so an application may fill one struct with another table
+ * between calls. The cached upload is reused only while the struct's bytes are the ones it was built from; tables
+ * rewritten in place behind unchanged pointers are not detected. The first call on a struct builds the entry: from
+ * NeuralNetClass_exe with nn_id -1 and zero statistics, which legacy_kernel never reads (LegacyIO carries them). */
 static DeviceModel *legacy_model(const NeuralNetClass *net, const int32_t *mean, const int32_t *stdR, int nn_id)
 {
     auto it = g_lg.models.find(net);
-    if (it != g_lg.models.end()) return it->second;
+    if (it != g_lg.models.end()) {
+        if (!memcmp(&it->second.net, net, sizeof *net)) return it->second.dm;
+        cudaSetDevice(g_lg.device);
+        free_model(it->second.dm);
+        delete it->second.dm;
+        g_lg.models.erase(it);
+    }
     static const int32_t zeros[40] = { 0 };
     nnsp_b200_model *m = nullptr;
     if (nnsp_b200_model_from_net(net, mean ? mean : zeros, stdR ? stdR : zeros, nn_id, &m)) legacy_die("nnsp_b200_model_from_net");
@@ -148,7 +164,9 @@ static DeviceModel *legacy_model(const NeuralNetClass *net, const int32_t *mean,
     cudaSetDevice(g_lg.device);
     if (upload_model(m, dm) || cudaDeviceSynchronize() != cudaSuccess) legacy_die("model upload");
     nnsp_b200_model_free(m);
-    g_lg.models[net] = dm;
+    LegacyModel &e = g_lg.models[net];
+    memcpy(&e.net, net, sizeof e.net);
+    e.dm = dm;
     return dm;
 }
 

@@ -381,7 +381,7 @@ int nnsp_b200_model_to_table_text(const nnsp_b200_model *m, const char *nn_name,
 {
     if (!m || !nn_name || !*nn_name || strlen(nn_name) > 40) return NNSP_B200_ERR_ARG;
     sink s = { buf, cap, 0 };
-    static const char *act_enum[] = { "relu6", "ftanh", "fsigmoid", "linear" };
+    static const char *act_enum[] = { "relu6", "ftanh", "sigmoid", "linear" };   /* ACTIVATION_TYPE, activation.h:16-22 */
     static const char *act_fn[] = { "relu6_fix", "tanh_fix", "sigmoid_fix", "linear_fix" };
     const int nl = m->numlayers;
     put(&s, "#include <stdint.h>\n#include \"neural_nets.h\"\n#include \"activation.h\"\n#include \"affine.h\"\n"

@@ -89,22 +89,30 @@ def test_reference_table_files_parse_to_the_compiled_models(nb):
 
 def test_emitted_text_is_valid_c_for_the_reference_headers(nb):
     """The writer's output compiles against the drop-in headers (same declarations as the reference's) and the
-    linked table, read back through nnsp_b200_model_from_net, is the same model."""
+    linked table, read back through nnsp_b200_model_from_net, is the same model. With -DDEF_ACC32BIT_OPT only the
+    layer_func addresses (tags in libnnsp_b200.so, referenced from another shared object) make it the acc32 model.
+    Besides the shipped models, a synthetic stack with sigmoid layers: the ACTIVATION_TYPE enumerator is `sigmoid`."""
     nb = nb
     import ctypes as C
-    raw = open(os.path.join(nb.MODEL_DIR, "kws_galaxy.nnspm"), "rb").read()
-    m = nb.Model.from_blob(raw)
+    tables = [(name, nn_id, open(os.path.join(nb.MODEL_DIR, blob), "rb").read()) for name, (_, nn_id, blob) in FILES.items()]
+    tables.append(("two_lstm_sigmoid", 2, make_blob(2, (240, 24, 20, 12, 9, 2), (0, 1, 0, 1, 0), [2, 1, 2, 1, 3], [6, 5, 5, 5, 6],
+                                                    [8, 15, 15, 15, 15], [13, 13, 15, 14, 15], seed=3)))
     with tempfile.TemporaryDirectory() as d:
-        src = os.path.join(d, "def_nn2_kws_galaxy.c")
-        open(src, "wb").write(m.to_table_text("kws_galaxy"))
-        so = os.path.join(d, "tbl.so")
-        r = subprocess.run(["gcc", "-shared", "-fPIC", "-w", "-I", os.path.join(ROOT, "include", "nnsp_compat"), "-I", os.path.join(ROOT, "include"),
-                            src, "-o", so, "-L", os.path.join(ROOT, "nnsp_b200"), "-lnnsp_b200", "-Wl,-rpath," + os.path.join(ROOT, "nnsp_b200")],
-                           capture_output=True, text=True)
-        assert r.returncode == 0, r.stderr
-        T = C.CDLL(so)
-        net = C.addressof(C.c_char.in_dll(T, "net_kws_galaxy"))
-        mean = C.addressof(C.c_char.in_dll(T, "feature_mean_kws_galaxy"))
-        stdr = C.addressof(C.c_char.in_dll(T, "feature_stdR_kws_galaxy"))
-        m2 = nb.Model.from_net(net, mean, stdr, 2)
-        assert m2.to_blob() == raw
+        for (name, nn_id, raw), acc32 in [(t, a) for t in tables for a in (False, True)]:
+            src = os.path.join(d, "def_nn%d_%s.c" % (nn_id, name))
+            text = nb.Model.from_blob(raw).to_table_text(name)
+            open(src, "wb").write(text)
+            so = os.path.join(d, "tbl_%s_%d.so" % (name, acc32))
+            r = subprocess.run(["gcc", "-shared", "-fPIC", "-w", "-I", os.path.join(ROOT, "include", "nnsp_compat"), "-I", os.path.join(ROOT, "include")]
+                               + (["-DDEF_ACC32BIT_OPT"] if acc32 else [])
+                               + [src, "-o", so, "-L", os.path.join(ROOT, "nnsp_b200"), "-lnnsp_b200", "-Wl,-rpath," + os.path.join(ROOT, "nnsp_b200")],
+                               capture_output=True, text=True)
+            assert r.returncode == 0, r.stderr
+            T = C.CDLL(so)
+            net = C.addressof(C.c_char.in_dll(T, "net_" + name))
+            mean = C.addressof(C.c_char.in_dll(T, "feature_mean_" + name))
+            stdr = C.addressof(C.c_char.in_dll(T, "feature_stdR_" + name))
+            m2 = nb.Model.from_net(net, mean, stdr, nn_id)
+            assert m2.acc32 == acc32, (name, acc32)
+            assert m2.to_blob() == nb.Model.from_blob(raw, acc32=acc32).to_blob(), (name, acc32)
+            assert (m2.to_blob() == raw) != acc32, (name, acc32)       # the acc32 flag is part of the container
