@@ -68,6 +68,11 @@ long long nnsp_b200_tc5_launches(void);
  * after the stage-sorted rounds the replay (kind 2, or kind 0 / 1 when the replay kernel is not used) is launched once
  * per call and returns at once when no stream is left for it. */
 long long nnsp_b200_cascade_kernel_launches(int kind);
+/* how many of them were the LSTM scan kernel of the split network path (batched NNSPClass, net_eval, the cascade's
+ * stage-sorted rounds), by specialisation (unit groups NT, CTAs per SM, k-steps compiled in, 0 = read at run time), in
+ * the order the dispatch tries them: 0 <4,4,1>, 1 <4,4,0>, 2 <8,2,2>, 3 <9,2,3>, 4 <9,2,0>, 5 <16,1,0> (-1 for any other
+ * kind). Which one runs depends only on the LSTM layer's shape, so a test can tell which code path evaluated a model. */
+long long nnsp_b200_scan_kernel_launches(int kind);
 
 /* ------------------------------------------------------------------------------------ */
 /* Models                                                                               */

@@ -618,3 +618,12 @@ def cascade_kernel_launches():
     """launches of the cascade's per-stream network kernels so far: {"narrow": cascade_kernel<CsNarrow>, "wide":
     cascade_kernel<CsWide>, "replay": cascade_replay_kernel}"""
     return {k: lib().nnsp_b200_cascade_kernel_launches(i) for i, k in enumerate(CASCADE_KERNELS)}
+
+
+SCAN_KERNELS = ("4,4,1", "4,4,0", "8,2,2", "9,2,3", "9,2,0", "16,1,0")
+
+
+def scan_kernel_launches():
+    """launches of the split path's LSTM scan kernel so far, by specialisation scan_kernel<NT, MINB, KT>: {"4,4,1": n, ...}
+    in dispatch order (KT 0: k-step counts read at run time)"""
+    return {k: lib().nnsp_b200_scan_kernel_launches(i) for i, k in enumerate(SCAN_KERNELS)}

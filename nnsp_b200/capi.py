@@ -47,7 +47,7 @@ nnsp_b200_event_record nnsp_b200_event_elapsed_ms nnsp_b200_event_destroy nnsp_b
 nnsp_b200_group_create_batch nnsp_b200_group_create_cascade nnsp_b200_group_size nnsp_b200_group_range nnsp_b200_group_reset nnsp_b200_group_set_stream_params
 nnsp_b200_group_exec_host nnsp_b200_group_exec_host_async nnsp_b200_group_wait nnsp_b200_group_destroy
 nnsp_b200_batch_set_host_format nnsp_b200_cascade_set_host_format nnsp_b200_wav_info nnsp_b200_wav_read_frames nnsp_b200_wav_load_streams nnsp_b200_cascade_timeline
-nnsp_b200_cascade_exec_ragged nnsp_b200_cascade_exec_host_ragged_async""".split()
+nnsp_b200_cascade_exec_ragged nnsp_b200_cascade_exec_host_ragged_async nnsp_b200_scan_kernel_launches""".split()
 
 
 def lib():
@@ -68,6 +68,8 @@ def lib():
     L.nnsp_b200_tc5_launches.restype = ll
     L.nnsp_b200_cascade_kernel_launches.restype = ll
     L.nnsp_b200_cascade_kernel_launches.argtypes = [ci]
+    L.nnsp_b200_scan_kernel_launches.restype = ll
+    L.nnsp_b200_scan_kernel_launches.argtypes = [ci]
     L.nnsp_b200_model_from_net.argtypes = [vp, vp, vp, ci, C.POINTER(vp)]
     L.nnsp_b200_model_from_table_text.argtypes = [C.c_char_p, C.c_size_t, ci, ci, C.POINTER(vp)]
     L.nnsp_b200_model_to_table_text.argtypes = [vp, C.c_char_p, C.c_char_p, C.c_size_t, C.POINTER(C.c_size_t)]

@@ -23,6 +23,7 @@ namespace nnsp {
 
 std::atomic<long long> g_launches{0}, g_tc5_launches{0};
 std::atomic<long long> g_cascade_net_launches[3] = {};
+std::atomic<long long> g_scan_launches[6] = {};
 
 /* ======================================================================================== */
 /* device bookkeeping                                                                         */
@@ -848,6 +849,7 @@ const char *nnsp_b200_version(void) { return "nnsp-b200 0.1 (sm_100a)"; }
 long long nnsp_b200_kernel_launches(void) { return g_launches.load(); }
 long long nnsp_b200_tc5_launches(void) { return g_tc5_launches.load(); }
 long long nnsp_b200_cascade_kernel_launches(int kind) { return (kind >= 0 && kind < 3) ? g_cascade_net_launches[kind].load() : -1; }
+long long nnsp_b200_scan_kernel_launches(int kind) { return (kind >= 0 && kind < 6) ? g_scan_launches[kind].load() : -1; }
 
 int nnsp_b200_device_count(void)
 {

@@ -12,6 +12,7 @@ namespace nnsp {
 
 extern std::atomic<long long> g_launches, g_tc5_launches;
 extern std::atomic<long long> g_cascade_net_launches[3];   /* cascade_kernel<CsNarrow>, cascade_kernel<CsWide>, cascade_replay_kernel */
+extern std::atomic<long long> g_scan_launches[6];          /* scan_kernel<4,4,1>, <4,4,0>, <8,2,2>, <9,2,3>, <9,2,0>, <16,1,0> */
 
 #define NNSP_CUDA(expr)                                                                       \
     do {                                                                                      \

@@ -172,9 +172,9 @@ int nnsp_model_validate(const struct nnsp_b200_model *m)
             return NNSP_B200_ERR_UNSUPPORTED;
         }
         const int last = (i == m->numlayers - 1);
-        if ((!last && L->rows > NNSP_B200_MAX_WIDTH) || (last && L->rows > NNSP_B200_MAX_WIDTH) ||
-            (last && L->act == NNSP_ACT_LINEAR && L->rows > NNSP_B200_MAX_OUT)) {
-            nnsp_set_error("layer %d: width %d exceeds engine limit", i, L->rows);
+        const int limit = (last && L->act == NNSP_ACT_LINEAR && NNSP_B200_MAX_OUT < NNSP_B200_MAX_WIDTH) ? NNSP_B200_MAX_OUT : NNSP_B200_MAX_WIDTH;
+        if (L->rows > limit) {
+            nnsp_set_error("layer %d: width %d exceeds the engine limit of %d units", i, L->rows, limit);
             return NNSP_B200_ERR_UNSUPPORTED;
         }
         if (L->qk < 0 || L->qk > 15 || L->qi < 0 || L->qi > 15 || L->qb < 0 || L->qb > 15 ||

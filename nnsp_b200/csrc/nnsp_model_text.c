@@ -298,6 +298,11 @@ int nnsp_b200_model_from_table_text(const char *text, size_t nbytes, int nn_id, 
                 if (f == 3) net.qbit_kernel[i] = q; else if (f == 4) net.qbit_input[i] = q; else net.qbit_bias[i] = q;
             }
         }
+        /* qbit_input[nl]: the qbit_input_rec of a last LSTM layer (neural_nets.c:108); 0 when the initialiser stops at nl */
+        if (f == 4 && nl < NNSP_B200_MAX_LAYERS && list_item(item, nl, sub, sizeof sub) && *sub) {
+            last_word(sub, word, sizeof word);
+            net.qbit_input[nl] = (int8_t)strtol(word, NULL, 0);
+        }
     }
     /* fields 7, 8: state pointers (owned by the engine here). 9: act_func, 10: layer_func, 11..13: tables */
     for (int i = 0; i < nl; i++) {
@@ -384,6 +389,15 @@ int nnsp_b200_model_to_table_text(const nnsp_b200_model *m, const char *nn_name,
     static const char *act_enum[] = { "relu6", "ftanh", "sigmoid", "linear" };   /* ACTIVATION_TYPE, activation.h:16-22 */
     static const char *act_fn[] = { "relu6_fix", "tanh_fix", "sigmoid_fix", "linear_fix" };
     const int nl = m->numlayers;
+    const nnsp_layer *Ll = &m->layer[nl - 1];
+    /* A last LSTM layer reads its qbit_input_rec from qbit_input[nl] (neural_nets.c:108). With 10 layers that entry lies
+     * past the array, on qbit_bias[0] (what nnsp_b200_model_from_net reads too): a table cannot hold any other value. */
+    const int emit_qi_next = Ll->type == NNSP_LAYER_LSTM && nl < NNSP_B200_MAX_LAYERS;
+    if (Ll->type == NNSP_LAYER_LSTM && nl == NNSP_B200_MAX_LAYERS && Ll->qi_next != m->layer[0].qb) {
+        nnsp_set_error("model to table text: the last of %d layers is an LSTM whose qbit_input_rec %d differs from "
+                       "qbit_bias[0] %d; a %d-layer table reads qbit_bias[0] there", nl, Ll->qi_next, m->layer[0].qb, nl);
+        return NNSP_B200_ERR_UNSUPPORTED;
+    }
     put(&s, "#include <stdint.h>\n#include \"neural_nets.h\"\n#include \"activation.h\"\n#include \"affine.h\"\n"
             "#include \"affine_acc32b.h\"\n#include \"lstm.h\"\n/*************stats***********/\n");
     put(&s, "const int32_t feature_mean_%s[] = {", nn_name);
@@ -424,6 +438,7 @@ int nnsp_b200_model_to_table_text(const nnsp_b200_model *m, const char *nn_name,
     for (int i = 0; i < nl; i++) put(&s, "%d,", m->layer[i].qk);
     put(&s, "}, // fractional bits (kernel)\n\n\t{");
     for (int i = 0; i < nl; i++) put(&s, "%d,", m->layer[i].qi);
+    if (emit_qi_next) put(&s, "%d,", Ll->qi_next);
     put(&s, "}, // qbit_i\n\n\t{");
     for (int i = 0; i < nl; i++) put(&s, "%d,", m->layer[i].qb);
     put(&s, "}, // fractional bits (bias)\n\n\t{");

@@ -101,6 +101,15 @@ __device__ __forceinline__ int32_t activate16(int act, int32_t pre, const int16_
     }
 }
 
+/* dot_rows reads the old h of an LSTM as 8-byte words from ws->h + ho. A second LSTM behind a first one whose width is
+ * not a multiple of 4 starts at an offset that is not, and its rounded-up last word may reach past ws->h. Such a layer
+ * reads a copy instead: its old h in `row` (the layer's output buffer, which the cell loop writes only after every gate
+ * product), zero-padded to the k4rec words read. A caller syncs the threads that share `row` before reading it. */
+__device__ __forceinline__ void stage_h_row(int16_t *row, const int16_t *h, int rows, int k4rec, int t, int nt)
+{
+    for (int k = t; k < 4 * k4rec; k += nt) row[k] = (k < rows) ? h[k] : (int16_t)0;
+}
+
 /* One network evaluation for the warp's stream. ws->ctx is the input; LSTM state in ws->h/c.
  * tap_act / tap_logits (global, may be null) receive the layer outputs of this frame. */
 template <class WS>
@@ -121,6 +130,7 @@ __device__ __forceinline__ void net_forward(const DevModel &M, const uint32_t *_
         if (L.type == LAYER_LSTM) {
             const uint32_t *Wr = wimg + L.wrec_off;
             const int16_t *hh = ws->h + ho;
+            if (ho & 3) { stage_h_row(y, hh, L.rows, L.k4rec, lane, 32); __syncwarp(); hh = y; }
             for (int r = 0; r < rounds; r += 4) {
                 const int nr = min(4, rounds - r), r0 = r * 32 + lane;
                 int32_t ax[4] = { 0, 0, 0, 0 }, ah[4] = { 0, 0, 0, 0 };
@@ -205,6 +215,7 @@ __device__ __forceinline__ void net_forward_group(const DevModel &M, const uint3
         if (L.type == LAYER_LSTM) {
             const uint32_t *Wr = wimg + L.wrec_off;
             const int16_t *hh = ws->h + ho;
+            if (ho & 3) { stage_h_row(y, hh, L.rows, L.k4rec, gt, 32 * GW); group_sync<GW>(bar_id); hh = y; }
             for (int r = rs; r < re; r += 4) {
                 const int nr = min(4, re - r), r0 = r * 32 + lane;
                 int32_t ax[4] = { 0, 0, 0, 0 }, ah[4] = { 0, 0, 0, 0 };

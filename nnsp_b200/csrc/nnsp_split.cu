@@ -1031,8 +1031,9 @@ size_t split_plane_bytes(const MmaDeviceModel &mm, int n_streams, int n_inf)
     return (size_t)((n_streams + 15) / 16) * (size_t)n_inf * 32 * mm.h->pa;
 }
 
+/* kind: the index nnsp_b200_scan_kernel_launches counts this specialisation under */
 template <int NW, int MINB, int KT>
-static int launch_scan(const ScanArgs &a, int ntiles, size_t smem, int device, cudaStream_t st)
+static int launch_scan(int kind, const ScanArgs &a, int ntiles, size_t smem, int device, cudaStream_t st)
 {
     static bool attr_done[64] = { false };
     static std::mutex attr_mu;                         /* host threads may drive separate handles on one device */
@@ -1045,6 +1046,7 @@ static int launch_scan(const ScanArgs &a, int ntiles, size_t smem, int device, c
     attr_lk.unlock();
     scan_kernel<NW, MINB, KT><<<ntiles, 32 * NW, smem, st>>>(a);
     NNSP_LAUNCH_CHECK();
+    g_scan_launches[kind].fetch_add(1, std::memory_order_relaxed);
     return NNSP_B200_OK;
 }
 
@@ -1232,13 +1234,13 @@ int launch_split_layers(const MmaDeviceModel &mm, const SplitGroup &q, int devic
             const size_t smem = scan_smem(D, L);
             /* the shipped layers get their k-step counts compiled in: VAD 28 -> 28 (1 k-step), KWS 64 -> 64 (2), S2I 72 -> 72 (3) */
             const int kq = (L.kt == L.ktr) ? L.kt : 0;
-            if (L.nt <= 4) rc = (kq == 1) ? launch_scan<4, 4, 1>(a, ntiles, smem, device, st) : launch_scan<4, 4, 0>(a, ntiles, smem, device, st);
+            if (L.nt <= 4) rc = (kq == 1) ? launch_scan<4, 4, 1>(0, a, ntiles, smem, device, st) : launch_scan<4, 4, 0>(1, a, ntiles, smem, device, st);
             /* 64-unit layers (KWS): eight unit groups take eight warps, not nine (-2 % of the network time; capping the
              * registers for three CTAs per SM spills and gains nothing: profiles/r2_cascade_overlap.txt) */
-            else if (L.nt <= 8 && kq == 2) rc = launch_scan<8, 2, 2>(a, ntiles, smem, device, st);
-            else if (L.nt <= 9) rc = (kq == 2) ? launch_scan<9, 2, 2>(a, ntiles, smem, device, st)
-                                   : (kq == 3) ? launch_scan<9, 2, 3>(a, ntiles, smem, device, st) : launch_scan<9, 2, 0>(a, ntiles, smem, device, st);
-            else rc = launch_scan<16, 1, 0>(a, ntiles, smem, device, st);
+            else if (L.nt <= 8 && kq == 2) rc = launch_scan<8, 2, 2>(2, a, ntiles, smem, device, st);
+            /* kq is 3 or 0 here: nt 9 is H in 65..72 (ktr 3), and H in 33..64 with kq 2 took the branch above */
+            else if (L.nt <= 9) rc = (kq == 3) ? launch_scan<9, 2, 3>(3, a, ntiles, smem, device, st) : launch_scan<9, 2, 0>(4, a, ntiles, smem, device, st);
+            else rc = launch_scan<16, 1, 0>(5, a, ntiles, smem, device, st);
             if (rc) return rc;
             cur_in = bufs[which]; which ^= 1;
             ao += L.rows; ho += L.rows;

@@ -23,11 +23,11 @@ from collections import Counter
 import numpy as np
 import pytest
 
-from common import NET_CASCADE_EDGES, NET_CASES, NET_CRAFTED, NET_TC5_SATURATING, cascade_events, chunks, net_case_blob, net_case_dims
+from common import NET_CASCADE_EDGES, NET_CASES, NET_CRAFTED, NET_LIMITS, NET_TC5_SATURATING, cascade_events, chunks, net_case_blob, net_case_dims
 
 S2I, VAD, KWS = 0, 1, 2
 MODEL_FILE = {S2I: "s2i.nnspm", VAD: "vad.nnspm", KWS: "kws_galaxy.nnspm"}
-STACKS = {c[0]: c for c in NET_CASES + NET_CRAFTED + NET_TC5_SATURATING + NET_CASCADE_EDGES}
+STACKS = {c[0]: c for c in NET_CASES + NET_CRAFTED + NET_TC5_SATURATING + NET_CASCADE_EDGES + NET_LIMITS}
 # short time-outs and look-backs, detections after one frame over a low threshold: a stage change every ~10 frames
 PARAMS = dict(thresh_timeout_kws=40, thresh_timeout_s2i=30, frs_vbufBk_kws=20, frs_vbufBk_s2i=3, thresh_cnts_vad=1,
               thresh_prob_vad=100, thresh_prob_kws=100, thresh_cnts_kws=1)
@@ -49,6 +49,9 @@ TRIOS = [
     ("wide_lstm100", ("lstm_wide", "sat_feat_random", "sat_feat_p127"), False, True, True, (False, True), EV, PARAMS),
     ("no_split_wide", ("lstm_requant", "fc_only", "two_lstm"), False, False, False, (False, True), EV, PARAMS),
     ("no_split_narrow", ("all_m128_q0", "bias_shift_18", "two_lstm"), True, False, False, (False,), (), PARAMS),   # acc32: VAD never fires
+    # a second KWS LSTM at state offset 6 / 41 (not a multiple of 4): no scan-split form, the sequential kernel in each shape
+    ("off6_narrow", ("s2i_narrow_edge", "fc_only", "lstm_off6"), True, False, False, (False, True), EV, PARAMS),
+    ("off41_wide", ("lstm_wide", "ten_layers", "lstm_off41"), False, False, False, (False, True), EV, PARAMS),
     # the shipped KWS model stays under any probability threshold on this audio: a count threshold of 0 lets it through
     ("shipped", None, True, True, True, (False, True), EV, dict(PARAMS, thresh_cnts_kws=0)),
 ]

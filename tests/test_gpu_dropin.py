@@ -14,7 +14,7 @@ from concurrent.futures import ThreadPoolExecutor
 import numpy as np
 import pytest
 
-from common import (GOLDEN_NETS, MODEL_NAME, NET_CASCADE_EDGES, NET_CASES, NET_CRAFTED, NET_TC5_SATURATING, ROOT, golden,
+from common import (GOLDEN_NETS, MODEL_NAME, NET_CASCADE_EDGES, NET_CASES, NET_CRAFTED, NET_LIMITS, NET_TC5_SATURATING, ROOT, golden,
                     net_case_blob, net_case_dims, res4, sha)
 from oracle.pyoracle import RESULT_DT, Taps
 
@@ -22,7 +22,7 @@ pytestmark = pytest.mark.gpu
 G = golden()
 MODEL_FILE = {0: "s2i.nnspm", 1: "vad.nnspm", 2: "kws_galaxy.nnspm"}
 ACC = {False: "acc64", True: "acc32"}
-SYNTH = NET_CASES + NET_CRAFTED + NET_CASCADE_EDGES + NET_TC5_SATURATING
+SYNTH = NET_CASES + NET_CRAFTED + NET_CASCADE_EDGES + NET_TC5_SATURATING + NET_LIMITS
 WAVS = ("speech", "galaxy", "galaxy_s2i")
 
 

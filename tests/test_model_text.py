@@ -1,6 +1,7 @@
 """The reference's on-disk model format -- generated C source `evb/src/def_nn{id}_{name}.c`
 (python/c_code_table_converter.py:143-347, layout python/nnsp_pack/c_weight_man.py:5-124) -- read and
 written as text by libnnsp_b200 (nnsp_model_text.c), no C compiler on the load path. Host logic only."""
+import ctypes as C
 import hashlib
 import os
 import struct
@@ -10,7 +11,7 @@ import tempfile
 import numpy as np
 import pytest
 
-from common import ROOT, have_reference_tree, make_blob
+from common import NET_LIMITS, ROOT, have_reference_tree, make_blob, net_case_blob, widen_text
 
 REF_SRC = "/root/reference/evb/src"
 FILES = {"s2i": ("def_nn0_s2i.c", 0, "s2i.nnspm"), "vad": ("def_nn1_vad.c", 1, "vad.nnspm"),
@@ -45,6 +46,71 @@ def test_text_round_trip_odd_shapes(nb, sizes, types):
     text = m.to_table_text("kws_odd")
     m2 = nb.Model.from_table_text(text)
     assert m2.to_blob() == raw
+
+
+@pytest.mark.parametrize("acc32", [False, True])
+@pytest.mark.parametrize("case", NET_LIMITS, ids=[c[0] for c in NET_LIMITS])
+def test_text_round_trip_at_the_model_limits(nb, case, acc32):
+    """10 layers, 128 units and outputs, unaligned LSTM offsets; a last LSTM keeps its qbit_input_rec (qbit_input[nl],
+    which a 10-layer table reads from qbit_bias[0])"""
+    raw = net_case_blob(case, acc32)
+    m = nb.Model.from_blob(raw)
+    text = m.to_table_text("kws_lim")
+    assert nb.Model.from_table_text(text, nn_id=case[1]).to_blob() == raw
+
+
+def test_text_writer_refuses_a_last_lstm_qbit_input_rec_a_table_cannot_hold(nb):
+    """with 10 layers the table has no qbit_input[10]: a last LSTM reads qbit_bias[0] there, so any other value is refused
+    rather than written as a different model; with fewer layers the value is written and read back"""
+    from nnsp_b200 import capi
+    case = [c for c in NET_LIMITS if c[0] == "ten_layers_last_lstm"][0]
+    name, nn_id, sizes, types, acts, qk, qi, qb = case[:8]
+    assert qi[10] == qb[0]
+    bad = make_blob(nn_id, sizes, types, list(acts), list(qk), list(qi[:10]) + [qb[0] - 1], list(qb))
+    m = nb.Model.from_blob(bad)
+    n = C.c_size_t()
+    L = capi.lib()
+    assert L.nnsp_b200_model_to_table_text(m.h, b"vad", None, 0, C.byref(n)) == -4          # NNSP_B200_ERR_UNSUPPORTED
+    assert b"qbit_bias[0]" in L.nnsp_b200_last_error()
+    with pytest.raises(nb.NnspError, match="qbit_bias"):
+        m.to_table_text("vad")
+    # 3 layers, last LSTM with qbit_input_rec 12: the 4th qi entry of the table
+    raw = make_blob(1, (240, 16, 8, 2), (0, 0, 1), [1, 1, 1], [7, 5, 6], [8, 15, 15, 12], [14, 13, 14])
+    text = nb.Model.from_blob(raw).to_table_text("vad")
+    assert b"{8,15,15,12,}, // qbit_i" in text
+    assert nb.Model.from_table_text(text).to_blob() == raw
+
+
+@pytest.mark.parametrize("last_fc", [True, False])
+def test_width_and_output_limits(nb, last_fc):
+    """128 units in a hidden layer and 128 outputs are accepted, 129 refused with the limit named, from the container and
+    from table text alike"""
+    from nnsp_b200 import capi
+    L = capi.lib()
+    for hidden, n_out, ok in ((128, 128, True), (129, 64, False), (64, 129, False)):
+        types = (0, 1, 0) if last_fc else (0, 0, 1)
+        sizes = (240, hidden, 64, n_out) if last_fc else (240, 64, hidden, n_out)
+        raw = make_blob(0, sizes, types, [1, 1, 3 if last_fc else 1], [7, 5, 6], [8, 15, 15], [14, 13, 15])
+        h = C.c_void_p()
+        rc = L.nnsp_b200_model_from_blob(raw, len(raw), C.byref(h))
+        assert (rc == 0) == ok, (sizes, rc)
+        if ok:
+            text = nb.Model.from_blob(raw).to_table_text("s2i")
+            assert nb.Model.from_table_text(text).to_blob() == raw
+            L.nnsp_b200_model_free(h)
+            continue
+        assert rc == -4 and b"exceeds" in L.nnsp_b200_last_error() and b"128" in L.nnsp_b200_last_error(), (sizes, rc)
+        # the same shape as table text: write the 128-wide model, widen one layer in the text
+        small = tuple(v if i == 0 else min(v, 128) for i, v in enumerate(sizes))
+        text = nb.Model.from_blob(make_blob(0, small, types, [1, 1, 3 if last_fc else 1], [7, 5, 6], [8, 15, 15], [14, 13, 15])).to_table_text("s2i")
+        wide = widen_text(text, small, sizes)
+        hh = C.c_void_p()
+        assert L.nnsp_b200_model_from_table_text(wide, len(wide), 0, 0, C.byref(hh)) == -4, sizes
+        assert b"exceeds" in L.nnsp_b200_last_error() and b"128" in L.nnsp_b200_last_error()
+        # the rewrite itself is sound: applied to the 128-wide sizes it gives a table the reader takes
+        ok_text = widen_text(text, small, small)
+        assert L.nnsp_b200_model_from_table_text(ok_text, len(ok_text), 0, 0, C.byref(hh)) == 0
+        L.nnsp_b200_model_free(hh)
 
 
 def test_text_reader_rejects_malformed_tables(nb):
