@@ -203,6 +203,28 @@ int nnsp_b200_cascade_create(const nnsp_b200_model *const models[3], const int *
                              const nnsp_b200_cascade_params *params, int n_streams, int device,
                              nnsp_b200_cascade **out);
 int nnsp_b200_cascade_reset(nnsp_b200_cascade *c);
+/* Reset individual streams of a live handle, e.g. to hand a server slot to a new caller without touching the others.
+ *   NNSP_B200_RESET_INSTANCE: nnCntrlClass_reset (nnCntrlClass.c:130-150) of that stream's controller, what
+ *     nnsp_b200_cascade_reset does to every stream: PCM ring and log-mel history cleared, every instance reset, time-out
+ *     counters zeroed; the stage position and context row 5 of every instance are kept (DESIGN.md section 2, quirks 2, 3).
+ *   NNSP_B200_RESET_FRESH: nnCntrlClass_init + reset, the state nnsp_b200_cascade_create leaves.
+ * `streams` is host memory, copied before the call returns. An id outside [0, n_streams), n < 0 or an unknown mode returns
+ * NNSP_B200_ERR_ARG and records nothing; n == 0 does nothing. The call does not wait for the device: the listed streams
+ * start the NEXT exec call of any kind (device, ragged, host, host-async, tapped) from the reset state. Calls issued
+ * before it keep their results and the state they leave; a reset issued between two asynchronous host tickets affects
+ * only the second. Resets compose in call order: a stream listed twice before a call is reset FRESH if either listing
+ * was FRESH, and nnsp_b200_cascade_reset issued while resets are pending leaves what it would leave had they come first.
+ * Per-stream parameters (nnsp_b200_cascade_set_stream_params) are configuration and survive both modes. A reset stream
+ * given n_frames[s] == 0 in a ragged call stays in its reset state. A call with no pending reset launches and copies
+ * exactly what it would without this function and never waits for the device. A call with some uploads the list and
+ * resets those streams on the device before its kernels read them; before it reuses the list's staging buffer it waits
+ * on the host until the device has run the list copies of the reset-carrying call before last, which are queued behind
+ * the work issued before them on their stream (pipelined device calls: the chain two calls back; host calls: the same
+ * slice of the previous ticket). A caller that resets before every call thus runs at most about two calls ahead of the
+ * device. */
+#define NNSP_B200_RESET_INSTANCE 0
+#define NNSP_B200_RESET_FRESH    1
+int nnsp_b200_cascade_reset_streams(nnsp_b200_cascade *c, const int32_t *streams, int n, int mode);
 /* ParamCntrlClass belongs to a controller instance (nnCntrlClass.h:12-29), i.e. to a stream: params[i] becomes the
  * parameter set of stream first_stream + i (thresholds, counts, time-outs; the two look-back depths must equal the
  * handle's, they size its history buffers). Waits for the handle's work in flight; takes effect with the next call and
@@ -276,6 +298,10 @@ int nnsp_b200_group_range(const nnsp_b200_group *g, int member, int *device, int
 int nnsp_b200_group_reset(nnsp_b200_group *g);
 /* nnsp_b200_cascade_set_stream_params in the group's stream numbering (cascade groups); waits for the calls issued so far */
 int nnsp_b200_group_set_stream_params(nnsp_b200_group *g, int first_stream, int n_streams, const nnsp_b200_cascade_params *params);
+/* nnsp_b200_cascade_reset_streams in the group's stream numbering (cascade groups; a batch group returns
+ * NNSP_B200_ERR_ARG). Checked and copied before it returns, queued in order with the group's calls in each member's
+ * command queue: the listed streams start the next call issued after it from the reset state. Does not wait. */
+int nnsp_b200_group_reset_streams(nnsp_b200_group *g, const int32_t *streams, int n, int mode);
 int nnsp_b200_group_exec_host(nnsp_b200_group *g, const int16_t *pcm, long long stream_stride, int n_frames, void *results);
 int nnsp_b200_group_exec_host_async(nnsp_b200_group *g, const int16_t *pcm, long long stream_stride, int n_frames,
                                     void *results, long long *ticket);

@@ -287,6 +287,14 @@ class Cascade:
     def reset(self):
         check(lib().nnsp_b200_cascade_reset(self.h), "cascade_reset")
 
+    def reset_streams(self, streams, fresh=False):
+        """Reset the listed streams before the next call of any kind, without waiting for the device: nnCntrlClass_reset of
+        their controllers (stage position and context row 5 of every instance kept), or with fresh=True the state a new
+        handle starts from. Per-stream parameters are kept either way."""
+        s = np.ascontiguousarray(streams, np.int32).ravel()
+        check(lib().nnsp_b200_cascade_reset_streams(self.h, s.ctypes.data_as(C.c_void_p), len(s), 1 if fresh else 0),
+              "cascade_reset_streams")
+
     def set_stream_params(self, first_stream, params):
         """params: [n][10] int16, rows in the field order of ParamCntrlClass (what params_array() returns for the handle)"""
         p = np.ascontiguousarray(params, np.int16).reshape(-1, len(capi.CascadeParams._fields_))
@@ -453,6 +461,12 @@ class Group:
 
     def reset(self):
         check(lib().nnsp_b200_group_reset(self.h), "group_reset")
+
+    def reset_streams(self, streams, fresh=False):
+        """cascade groups: Cascade.reset_streams in the group's stream numbering, queued in order with the group's calls"""
+        s = np.ascontiguousarray(streams, np.int32).ravel()
+        check(lib().nnsp_b200_group_reset_streams(self.h, s.ctypes.data_as(C.c_void_p), len(s), 1 if fresh else 0),
+              "group_reset_streams")
 
     def set_stream_params(self, first_stream, params):
         """cascade groups: params [n][10] int16 in the field order of ParamCntrlClass, global stream numbering"""

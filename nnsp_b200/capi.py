@@ -47,7 +47,8 @@ nnsp_b200_event_record nnsp_b200_event_elapsed_ms nnsp_b200_event_destroy nnsp_b
 nnsp_b200_group_create_batch nnsp_b200_group_create_cascade nnsp_b200_group_size nnsp_b200_group_range nnsp_b200_group_reset nnsp_b200_group_set_stream_params
 nnsp_b200_group_exec_host nnsp_b200_group_exec_host_async nnsp_b200_group_wait nnsp_b200_group_destroy
 nnsp_b200_batch_set_host_format nnsp_b200_cascade_set_host_format nnsp_b200_wav_info nnsp_b200_wav_read_frames nnsp_b200_wav_load_streams nnsp_b200_cascade_timeline
-nnsp_b200_cascade_exec_ragged nnsp_b200_cascade_exec_host_ragged_async nnsp_b200_scan_kernel_launches""".split()
+nnsp_b200_cascade_exec_ragged nnsp_b200_cascade_exec_host_ragged_async nnsp_b200_scan_kernel_launches
+nnsp_b200_cascade_reset_streams nnsp_b200_group_reset_streams""".split()
 
 
 def lib():
@@ -100,6 +101,7 @@ def lib():
         L.nnsp_b200_cascade_create.argtypes = [C.POINTER(vp), C.POINTER(ci), ci, C.POINTER(CascadeParams), ci, ci, C.POINTER(vp)]
         L.nnsp_b200_cascade_reset.argtypes = [vp]
         L.nnsp_b200_cascade_set_stream_params.argtypes = [vp, ci, ci, vp]
+        L.nnsp_b200_cascade_reset_streams.argtypes = [vp, vp, ci, ci]
         L.nnsp_b200_cascade_exec.argtypes = [vp, vp, ll, ci, vp, C.POINTER(Taps)]
         L.nnsp_b200_cascade_exec_host.argtypes = [vp, vp, ll, ci, vp]
         L.nnsp_b200_cascade_exec_host_async.argtypes = [vp, vp, ll, ci, vp, C.POINTER(ll)]
@@ -135,6 +137,7 @@ def lib():
     L.nnsp_b200_group_range.argtypes = [vp, ci, C.POINTER(ci), C.POINTER(ci), C.POINTER(ci)]
     L.nnsp_b200_group_reset.argtypes = [vp]
     L.nnsp_b200_group_set_stream_params.argtypes = [vp, ci, ci, vp]
+    L.nnsp_b200_group_reset_streams.argtypes = [vp, vp, ci, ci]
     L.nnsp_b200_group_exec_host.argtypes = [vp, vp, ll, ci, vp]
     L.nnsp_b200_group_exec_host_async.argtypes = [vp, vp, ll, ci, vp, C.POINTER(ll)]
     L.nnsp_b200_group_wait.argtypes = [vp, ll]

@@ -15,6 +15,7 @@
  *                    dataBuffer -- recompute it on the spot; standardise, network, post-processing,
  *                    controller transition, reset-on-exit
  *   hist kernels   : newest d_max+2 PCM frames and d_max log-mel rows for the next call */
+#include <algorithm>
 #include <cstdlib>
 #include <cuda_runtime.h>
 #include <vector>
@@ -946,28 +947,37 @@ struct ResetModels { const DevModel *m[3]; int seq[CS_MAXSEQ]; };
 
 /* nnCntrlClass_reset (nnCntrlClass.c:130-150): every instance reset, ring cleared, timeout counters
  * zeroed; current_pos_seq is NOT rewound (only nnCntrlClass_init sets it, :125) and every instance keeps
- * its context row 5. fresh != 0 (create = init + reset on zeroed structs) also rewinds and clears those. */
+ * its context row 5. fresh != 0 (create = init + reset on zeroed structs) also rewinds and clears those.
+ * list == null: streams 0 .. S-1, one per CTA, all with `fresh`; else the streams list[0 .. gridDim.x), each entry
+ * (stream << 1 | fresh). `parts` says what is written: the PCM ring, which the front end reads, and the controller /
+ * instance state with the log-mel history, which the chain reads -- a pipelined call resets them on different streams. */
+constexpr int RESET_RING = 1, RESET_STATE = 2;
 __global__ void cascade_reset_kernel(ResetModels rm, StreamState st, int16_t *stale, int S,
-                                     int hist_words, int lm_words, int fresh)
+                                     int hist_words, int lm_words, int fresh, const int *list, int parts)
 {
-    const int s = blockIdx.x;
+    int s = blockIdx.x;
+    if (list) { const int e = list[blockIdx.x]; s = e >> 1; fresh = e & 1; }
     if (s >= S) return;
     const int HS = NNSP_B200_MAX_WIDTH;
-    const int pos = fresh ? 0 : st.casc[(long long)s * CS_N + CS_POS];
-    const DevModel *M = rm.m[rm.seq[pos]];
-    __syncthreads();
-    for (int i = threadIdx.x; i < 200; i += blockDim.x) st.ctx[(long long)s * 240 + i] = M->silence[i % 40];
-    if (fresh) {
-        for (int i = threadIdx.x; i < 40; i += blockDim.x) st.ctx[(long long)s * 240 + 200 + i] = 0;
-        for (int i = threadIdx.x; i < 120; i += blockDim.x) stale[(long long)s * 120 + i] = 0;
+    if (parts & RESET_STATE) {
+        const int pos = fresh ? 0 : st.casc[(long long)s * CS_N + CS_POS];
+        const DevModel *M = rm.m[rm.seq[pos]];
+        __syncthreads();
+        for (int i = threadIdx.x; i < 200; i += blockDim.x) st.ctx[(long long)s * 240 + i] = M->silence[i % 40];
+        if (fresh) {
+            for (int i = threadIdx.x; i < 40; i += blockDim.x) st.ctx[(long long)s * 240 + 200 + i] = 0;
+            for (int i = threadIdx.x; i < 120; i += blockDim.x) stale[(long long)s * 120 + i] = 0;
+        }
+        for (int i = threadIdx.x; i < HS; i += blockDim.x) { st.h[(long long)s * HS + i] = 0; st.c[(long long)s * HS + i] = 0; }
+        for (int i = threadIdx.x; i < SC_N; i += blockDim.x) st.scal[(long long)s * SC_N + i] = (i == SC_SLIDES) ? 1 : 0;
+        for (int i = threadIdx.x; i < CS_N; i += blockDim.x) st.casc[(long long)s * CS_N + i] = (i == CS_POS) ? (uint16_t)pos : (uint16_t)0;
+        int32_t *lm = st.lmhist + (long long)s * lm_words;
+        for (int i = threadIdx.x; i < lm_words; i += blockDim.x) lm[i] = LOGMEL_OF_ZERO;       /* log-mel of an all-zero window */
     }
-    for (int i = threadIdx.x; i < HS; i += blockDim.x) { st.h[(long long)s * HS + i] = 0; st.c[(long long)s * HS + i] = 0; }
-    for (int i = threadIdx.x; i < SC_N; i += blockDim.x) st.scal[(long long)s * SC_N + i] = (i == SC_SLIDES) ? 1 : 0;
-    for (int i = threadIdx.x; i < CS_N; i += blockDim.x) st.casc[(long long)s * CS_N + i] = (i == CS_POS) ? (uint16_t)pos : (uint16_t)0;
-    unsigned int *h = reinterpret_cast<unsigned int *>(st.hist) + (long long)s * hist_words;
-    for (int i = threadIdx.x; i < hist_words; i += blockDim.x) h[i] = 0;                       /* PcmBufClass_reset, PcmBufClass.c:19-28 */
-    int32_t *lm = st.lmhist + (long long)s * lm_words;
-    for (int i = threadIdx.x; i < lm_words; i += blockDim.x) lm[i] = LOGMEL_OF_ZERO;           /* log-mel of an all-zero window */
+    if (parts & RESET_RING) {
+        unsigned int *h = reinterpret_cast<unsigned int *>(st.hist) + (long long)s * hist_words;
+        for (int i = threadIdx.x; i < hist_words; i += blockDim.x) h[i] = 0;                   /* PcmBufClass_reset, PcmBufClass.c:19-28 */
+    }
 }
 
 }  // namespace nnsp
@@ -1036,6 +1046,18 @@ struct nnsp_b200_cascade {
     int host_fmt = NNSP_B200_HOST_PCM16;       /* int16 PCM or raw 32-bit AUDADC words (conditioned on the device) */
     uint32_t *d_raw = nullptr;
     int32_t *d_nfr = nullptr;                  /* ragged host-buffer calls: the per-stream counts, two buffers of [S] like d_pcm */
+    /* nnsp_b200_cascade_reset_streams: the pending mode of every stream (-1: none) and the streams that have one. The next
+     * call takes them as a list sorted by stream, entries (stream << 1 | fresh), written into pinned staging rs_host[b]
+     * and copied to rs_dev[...] on the stream that reads it. Both staging buffers alternate between the calls that carry
+     * resets; rs_copied[b][j] marks the end of the copies out of rs_host[b] on pipeline stream j (0: c->stream for device
+     * calls). A device-buffer call uses rs_dev[its pipe index] (rewritten after the chain two calls back, like the log-mel
+     * rows); a host-buffer call puts slice [s0, s1)'s entries at rs_dev[0] + s0, always on the slice's own stream. */
+    std::vector<int8_t> rs_mode;
+    std::vector<int> rs_ids;
+    int *rs_host[2] = { nullptr, nullptr }, *rs_dev[2] = { nullptr, nullptr };
+    cudaEvent_t rs_copied[2][3] = {};
+    bool rs_copy_valid[2][3] = {};
+    unsigned rs_flushes = 0;
 };
 
 constexpr int CS_MAX_SLICES = 8;
@@ -1090,21 +1112,63 @@ static int cascade_ensure_logmel(nnsp_b200_cascade *c, int T)
     return NNSP_B200_OK;
 }
 
+/* cascade_reset_kernel over every stream (list null, all `fresh`) or over the n entries of the device list */
+static int cascade_launch_reset(nnsp_b200_cascade *c, const int *list, int n, int fresh, int parts, cudaStream_t st)
+{
+    const int hist_frames = c->cd.dmax + 2, lm_rows = c->cd.dmax > 0 ? c->cd.dmax : 1;
+    ResetModels rm{};
+    for (int i = 0; i < 3; i++) rm.m[i] = c->dm[i].d;
+    for (int i = 0; i < c->cd.len_seq; i++) rm.seq[i] = c->cd.seq[i];
+    cascade_reset_kernel<<<list ? n : c->S, 128, 0, st>>>(rm, c->st, c->stale, c->S, hist_frames * (NNSP_B200_FRAME / 2),
+                                                          lm_rows * NNSP_B200_NMEL, fresh, list, parts);
+    NNSP_LAUNCH_CHECK();
+    return NNSP_B200_OK;
+}
+
+/* The pending resets as a list sorted by stream in the pinned staging buffer of this call (*list, *n, *b = which one;
+ * n == 0: none), and the pending set cleared. The buffer was last written by the reset-carrying call before last: the
+ * host waits until the device has run that call's list copies, the only host wait resets add. Those copies sit in
+ * stream order behind what was queued before them on their stream -- on a pipelined device call the wait for the chain
+ * two calls back, on a host call the same slice of the ticket before -- so a caller that resets before every call runs
+ * at most about two calls ahead of the device; calls without pending resets never wait here. */
+static int cascade_take_resets(nnsp_b200_cascade *c, const int **list, int *n, int *b)
+{
+    *n = (int)c->rs_ids.size();
+    if (*n == 0) return NNSP_B200_OK;
+    *b = (int)(c->rs_flushes++ & 1u);
+    for (int j = 0; j < 3; j++)
+        if (c->rs_copy_valid[*b][j]) { NNSP_CUDA(cudaEventSynchronize(c->rs_copied[*b][j])); c->rs_copy_valid[*b][j] = false; }
+    std::sort(c->rs_ids.begin(), c->rs_ids.end());
+    int *h = c->rs_host[*b];
+    for (int k = 0; k < *n; k++) {
+        const int s = c->rs_ids[(size_t)k];
+        h[k] = (s << 1) | (c->rs_mode[(size_t)s] == NNSP_B200_RESET_FRESH ? 1 : 0);
+        c->rs_mode[(size_t)s] = -1;
+    }
+    c->rs_ids.clear();
+    *list = h;
+    return NNSP_B200_OK;
+}
+
 /* st_nn (with ev_feat): pipelined call -- everything behind the front end goes to st_nn, the PCM history is rolled out
- * of place on st right behind the front end (c->st.hist is swapped by the caller afterwards) */
+ * of place on st right behind the front end (c->st.hist is swapped by the caller afterwards).
+ * rlist (device, rn entries of cascade_take_resets, null: none): streams reset before the call -- the PCM ring on st
+ * before the front end reads it, the rest on the stream of the chain before the chain reads it. */
 static int cascade_launch(nnsp_b200_cascade *c, const int16_t *pcm, long long stride, int T, int s0, int ns,
                           nnsp_b200_cascade_result *results, const nnsp_b200_taps *taps, cudaStream_t st, bool timed,
                           int slice = 0, int32_t *logmel = nullptr, cudaStream_t st_nn = nullptr, cudaEvent_t ev_feat = nullptr,
-                          cudaEvent_t ev_prev_nn = nullptr, const int32_t *nfr = nullptr)
+                          cudaEvent_t ev_prev_nn = nullptr, const int32_t *nfr = nullptr, const int *rlist = nullptr, int rn = 0)
 {
     const int hist_frames = c->cd.dmax + 2;
     if (!logmel) logmel = c->logmel;
     const bool piped = st_nn != nullptr;
+    int rc;
+    if (rlist && (rc = cascade_launch_reset(c, rlist, rn, 0, piped ? RESET_RING : RESET_RING | RESET_STATE, st))) return rc;
     FeatLaunch fl{ pcm, stride, c->st.hist, hist_frames, s0, ns, T, logmel };
     fl.nfr = nfr;
     cudaEvent_t *tl = c->tl[c->tl_count % 8];
     if (timed) NNSP_CUDA(cudaEventRecord(tl[0], st));
-    int rc = launch_feature(c->tables, fl, c->device, st);
+    rc = launch_feature(c->tables, fl, c->device, st);
     if (rc) return rc;
     if (timed) NNSP_CUDA(cudaEventRecord(tl[1], st));
     if (piped) {
@@ -1115,6 +1179,8 @@ static int cascade_launch(nnsp_b200_cascade *c, const int16_t *pcm, long long st
         if ((rc = launch_hist_roll(pcm, stride / 2, c->st.hist, c->hist2, hist_frames, NNSP_B200_FRAME / 2, s0, ns, T, st, nfr))) return rc;
         st = st_nn;
         if (timed) NNSP_CUDA(cudaEventRecord(tl[2], st));
+        /* behind the previous call's chain (stream order) and this call's front end (ev_feat), before anything reads it */
+        if (rlist && (rc = cascade_launch_reset(c, rlist, rn, 0, RESET_STATE, st))) return rc;
     }
     CascadeArgs a{};
     for (int i = 0; i < 3; i++) { a.model[i] = c->dm[i].d; a.wimg[i] = c->dm[i].wimg; a.bimg[i] = c->dm[i].bimg; }
@@ -1360,14 +1426,15 @@ int nnsp_b200_cascade_create(const nnsp_b200_model *const models[3], const int *
     TRY(cudaMalloc(&c->ra.age0, S * sizeof(int)));
     TRY(cudaMalloc(&c->ra.lmfix, S * 2 * NNSP_B200_NMEL * sizeof(int32_t)));
     TRY(cudaMemset(c->ra.lmfix, 0, S * 2 * NNSP_B200_NMEL * sizeof(int32_t)));
+    for (int b = 0; b < 2; b++) {
+        TRY(cudaHostAlloc(&c->rs_host[b], S * sizeof(int), cudaHostAllocDefault));
+        TRY(cudaMalloc(&c->rs_dev[b], S * sizeof(int)));
+        for (auto &e : c->rs_copied[b]) TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+    }
 #undef TRY
+    c->rs_mode.assign(S, (int8_t)-1);
     if (cudaDeviceSynchronize() != cudaSuccess) return fail(NNSP_B200_ERR_CUDA);   /* uploads went through the default stream */
-    ResetModels rm{};
-    for (int i = 0; i < 3; i++) rm.m[i] = c->dm[i].d;
-    for (int i = 0; i < len_seq; i++) rm.seq[i] = seq[i];
-    cascade_reset_kernel<<<c->S, 128, 0, c->stream>>>(rm, c->st, c->stale, c->S, hist_frames * (NNSP_B200_FRAME / 2),
-                                                      lm_rows * NNSP_B200_NMEL, 1);
-    g_launches.fetch_add(1);
+    if ((rc = cascade_launch_reset(c, nullptr, 0, 1, RESET_RING | RESET_STATE, c->stream))) return fail(rc);
     if (cudaStreamSynchronize(c->stream) != cudaSuccess) { nnsp_set_error("cascade reset kernel failed: %s", cudaGetErrorString(cudaGetLastError())); return fail(NNSP_B200_ERR_CUDA); }
     *out = c;
     return NNSP_B200_OK;
@@ -1408,14 +1475,30 @@ int nnsp_b200_cascade_reset(nnsp_b200_cascade *c)
     NNSP_CUDA(cudaDeviceSynchronize());
     c->nn_pending[0] = c->nn_pending[1] = false;
     c->host_inflight = false;
-    const int hist_frames = c->cd.dmax + 2, lm_rows = c->cd.dmax > 0 ? c->cd.dmax : 1;
-    ResetModels rm{};
-    for (int i = 0; i < 3; i++) rm.m[i] = c->dm[i].d;
-    for (int i = 0; i < c->cd.len_seq; i++) rm.seq[i] = c->cd.seq[i];
-    cascade_reset_kernel<<<c->S, 128, 0, c->stream>>>(rm, c->st, c->stale, c->S,
-                                                      hist_frames * (NNSP_B200_FRAME / 2), lm_rows * NNSP_B200_NMEL, 0);
-    NNSP_LAUNCH_CHECK();
+    /* resets still pending stay pending: applied at the next call, after this one, they leave what they would have left
+     * before it (a reset stream's state does not depend on the state it had) */
+    const int rc = cascade_launch_reset(c, nullptr, 0, 0, RESET_RING | RESET_STATE, c->stream);
+    if (rc) return rc;
     NNSP_CUDA(cudaStreamSynchronize(c->stream));
+    return NNSP_B200_OK;
+}
+
+int nnsp_b200_cascade_reset_streams(nnsp_b200_cascade *c, const int32_t *streams, int n, int mode)
+{
+    if (!c || n < 0 || (n > 0 && !streams) || (mode != NNSP_B200_RESET_INSTANCE && mode != NNSP_B200_RESET_FRESH)) {
+        nnsp_set_error("cascade_reset_streams: bad arguments (n = %d, mode = %d)", n, mode);
+        return NNSP_B200_ERR_ARG;
+    }
+    for (int i = 0; i < n; i++)                                       /* checked before anything is recorded */
+        if (streams[i] < 0 || streams[i] >= c->S) {
+            nnsp_set_error("cascade_reset_streams: streams[%d] = %d is outside [0, %d)", i, (int)streams[i], c->S);
+            return NNSP_B200_ERR_ARG;
+        }
+    for (int i = 0; i < n; i++) {
+        int8_t &m = c->rs_mode[(size_t)streams[i]];
+        if (m < 0) c->rs_ids.push_back(streams[i]);
+        if (m < mode) m = (int8_t)mode;                               /* FRESH after or before INSTANCE leaves FRESH */
+    }
     return NNSP_B200_OK;
 }
 
@@ -1443,11 +1526,23 @@ static int cascade_exec_dev(nnsp_b200_cascade *c, const int16_t *pcm_dev, long l
     }
     if ((rc = cascade_ensure_logmel(c, n_frames))) return rc;
     if ((rc = cascade_ensure_split(c, n_frames))) return rc;
+    const int *rl = nullptr;                            /* pending resets: uploaded on c->stream behind the waits below */
+    int rn = 0, rb = 0;
+    auto upload_resets = [&](int *dst) -> int {
+        NNSP_CUDA(cudaMemcpyAsync(dst, rl, (size_t)rn * sizeof(int), cudaMemcpyHostToDevice, c->stream));
+        NNSP_CUDA(cudaEventRecord(c->rs_copied[rb][0], c->stream));
+        c->rs_copy_valid[rb][0] = true;
+        rl = dst;
+        return NNSP_B200_OK;
+    };
+    if ((rc = cascade_take_resets(c, &rl, &rn, &rb))) return rc;
     if (cascade_use_split(c, taps)) {
         const int i = (int)(c->pipe++ & 1u);
         if (c->nn_pending[i]) NNSP_CUDA(cudaStreamWaitEvent(c->stream, c->ev_nn[i], 0));   /* log-mel buffer i / PCM history in use two calls ago */
+        if (rn && (rc = upload_resets(c->rs_dev[i]))) return rc;      /* rs_dev[i] too: its last readers ran in that chain */
         rc = cascade_launch(c, pcm_dev, stream_stride, n_frames, 0, c->S, results_dev, nullptr, c->stream, true, 0,
-                            i ? c->logmel2 : c->logmel, c->nn_stream, c->ev_feat[i], c->nn_pending[i ^ 1] ? c->ev_nn[i ^ 1] : nullptr, nfr);
+                            i ? c->logmel2 : c->logmel, c->nn_stream, c->ev_feat[i], c->nn_pending[i ^ 1] ? c->ev_nn[i ^ 1] : nullptr, nfr,
+                            rn ? rl : nullptr, rn);
         if (rc) return rc;
         NNSP_CUDA(cudaEventRecord(c->ev_nn[i], c->nn_stream));
         c->nn_pending[i] = true;
@@ -1455,8 +1550,9 @@ static int cascade_exec_dev(nnsp_b200_cascade *c, const int16_t *pcm_dev, long l
         return NNSP_B200_OK;
     }
     if ((rc = cascade_join_nn(c, c->stream))) return rc;
+    if (rn && (rc = upload_resets(c->rs_dev[0]))) return rc;
     return cascade_launch(c, pcm_dev, stream_stride, n_frames, 0, c->S, results_dev, taps, c->stream, true, 0, nullptr, nullptr,
-                          nullptr, nullptr, nfr);
+                          nullptr, nullptr, nfr, rn ? rl : nullptr, rn);
 }
 
 int nnsp_b200_cascade_exec(nnsp_b200_cascade *c, const int16_t *pcm_dev, long long stream_stride, int n_frames,
@@ -1517,6 +1613,9 @@ static int cascade_enqueue_host(nnsp_b200_cascade *c, const int16_t *pcm, long l
         NNSP_CUDA(cudaDeviceSynchronize());
         NNSP_CUDA(cudaMalloc(&c->d_nfr, (size_t)2 * c->S * sizeof(int32_t)));
     }
+    const int *rl = nullptr;                                          /* pending resets, sorted by stream */
+    int rn = 0, rb = 0;
+    if ((rc = cascade_take_resets(c, &rl, &rn, &rb))) return rc;
     c->host_inflight = true;
     const int nsl = c->S >= 4096 ? 8 : (c->S >= 256 ? 4 : 1);
     const int buf = (int)(c->host_calls++ & 1);
@@ -1558,8 +1657,16 @@ static int cascade_enqueue_host(nnsp_b200_cascade *c, const int16_t *pcm, long l
                 NNSP_CUDA(cudaMemcpyAsync(dnfr + s0, nfr + s0, (size_t)(s1 - s0) * sizeof(int32_t), cudaMemcpyHostToDevice, st));
         } else
             NNSP_CUDA(cudaStreamWaitEvent(st, c->ev_h2d[buf][k], 0));
+        /* the slice's own resets, at rs_dev[0] + s0: only this slice's kernels, all on st, ever use those entries */
+        const int r0 = rn ? (int)(std::lower_bound(rl, rl + rn, s0 << 1) - rl) : 0;
+        const int r1 = rn ? (int)(std::lower_bound(rl, rl + rn, s1 << 1) - rl) : 0;
+        if (r1 > r0) {
+            NNSP_CUDA(cudaMemcpyAsync(c->rs_dev[0] + s0, rl + r0, (size_t)(r1 - r0) * sizeof(int), cudaMemcpyHostToDevice, st));
+            NNSP_CUDA(cudaEventRecord(c->rs_copied[rb][k % 3], st));   /* re-recorded by later slices on st: the last copy */
+            c->rs_copy_valid[rb][k % 3] = true;
+        }
         rc = cascade_launch(c, dpcm, dstride, T, s0, s1 - s0, results ? c->d_res : nullptr, nullptr, st, false, k,
-                            nullptr, nullptr, nullptr, nullptr, dnfr);
+                            nullptr, nullptr, nullptr, nullptr, dnfr, r1 > r0 ? c->rs_dev[0] + s0 : nullptr, r1 - r0);
         if (rc) return rc;
         NNSP_CUDA(cudaEventRecord(c->ev_read[buf][k], st));         /* every reader of the slice's PCM has joined st by now */
         c->read_valid[buf][k] = true;
@@ -1709,6 +1816,11 @@ void nnsp_b200_cascade_destroy(nnsp_b200_cascade *c)
     for (auto &row : c->gs) for (auto g : row) if (g) cudaStreamDestroy(g);
     for (auto e : c->ev_fork) if (e) cudaEventDestroy(e);
     for (auto &row : c->ev_join) for (auto e : row) if (e) cudaEventDestroy(e);
+    for (int b = 0; b < 2; b++) {
+        if (c->rs_host[b]) cudaFreeHost(c->rs_host[b]);
+        cudaFree(c->rs_dev[b]);
+        for (auto e : c->rs_copied[b]) if (e) cudaEventDestroy(e);
+    }
     delete c;
 }
 

@@ -22,12 +22,13 @@
 namespace {
 
 struct Command {
-    enum Kind { EXEC, RESET, QUIT } kind;
+    enum Kind { EXEC, RESET, QUIT, RESET_STREAMS } kind;
     const int16_t *pcm;
     long long stride;
-    int n_frames;
+    int n_frames;                    /* RESET_STREAMS: the mode */
     void *results;
-    long long seq;
+    long long seq;                   /* RESET_STREAMS: complete once recorded and the call before it is complete */
+    std::vector<int32_t> streams;    /* RESET_STREAMS: the member's own streams, in its numbering */
 };
 
 struct Member {
@@ -75,6 +76,7 @@ int member_wait(Member *m, long long ticket)
 void worker(Member *m)
 {
     long long inflight_seq = 0, inflight_ticket = 0;
+    long long passed_seq = 0;        /* a reset recorded while a call was in flight: complete when that call is */
     auto fail = [&](int rc) {
         std::lock_guard<std::mutex> lk(m->mu);
         if (m->status == NNSP_B200_OK) {
@@ -88,10 +90,11 @@ void worker(Member *m)
         if (rc) fail(rc);
         {
             std::lock_guard<std::mutex> lk(m->mu);
-            m->done_seq = inflight_seq;
+            m->done_seq = passed_seq > inflight_seq ? passed_seq : inflight_seq;
         }
         m->cv_done.notify_all();
         inflight_seq = 0;
+        passed_seq = 0;
     };
     for (;;) {
         Command c;
@@ -107,6 +110,14 @@ void worker(Member *m)
             m->queue.pop_front();
         }
         if (c.kind == Command::QUIT) { finish_inflight(); return; }
+        if (c.kind == Command::RESET_STREAMS) {                 /* recorded on the handle, applied by its next call */
+            const int rc = nnsp_b200_cascade_reset_streams(m->cascade, c.streams.data(), (int)c.streams.size(), c.n_frames);
+            if (rc) fail(rc);
+            if (inflight_seq) { passed_seq = c.seq; continue; }
+            { std::lock_guard<std::mutex> lk(m->mu); m->done_seq = c.seq; }
+            m->cv_done.notify_all();
+            continue;
+        }
         if (c.kind == Command::RESET) {
             finish_inflight();
             const int rc = m->cascade ? nnsp_b200_cascade_reset(m->cascade) : nnsp_b200_batch_reset(m->batch);
@@ -207,7 +218,7 @@ int nnsp_b200_group_exec_host_async(nnsp_b200_group *g, const int16_t *pcm, long
                                     void *results, long long *ticket)
 {
     if (!g || !pcm || n_frames <= 0) return NNSP_B200_ERR_ARG;
-    Command c{ Command::EXEC, pcm, stream_stride, n_frames, results, 0 };
+    Command c{ Command::EXEC, pcm, stream_stride, n_frames, results, 0, {} };
     return post(g, c, ticket);
 }
 
@@ -234,7 +245,7 @@ int nnsp_b200_group_reset(nnsp_b200_group *g)
 {
     if (!g) return NNSP_B200_ERR_ARG;
     long long t = 0;
-    Command c{ Command::RESET, nullptr, 0, 0, nullptr, 0 };
+    Command c{ Command::RESET, nullptr, 0, 0, nullptr, 0, {} };
     post(g, c, &t);
     return nnsp_b200_group_wait(g, t);
 }
@@ -258,12 +269,36 @@ int nnsp_b200_group_set_stream_params(nnsp_b200_group *g, int first_stream, int 
     return NNSP_B200_OK;
 }
 
+int nnsp_b200_group_reset_streams(nnsp_b200_group *g, const int32_t *streams, int n, int mode)
+{
+    if (!g || !g->is_cascade || n < 0 || (n > 0 && !streams) || (mode != NNSP_B200_RESET_INSTANCE && mode != NNSP_B200_RESET_FRESH)) {
+        nnsp_set_error("group_reset_streams: a cascade group, n >= 0 and a known mode are required");
+        return NNSP_B200_ERR_ARG;
+    }
+    for (int i = 0; i < n; i++)
+        if (streams[i] < 0 || streams[i] >= g->n_streams) {
+            nnsp_set_error("group_reset_streams: streams[%d] = %d is outside [0, %d)", i, (int)streams[i], g->n_streams);
+            return NNSP_B200_ERR_ARG;
+        }
+    /* every member gets the command (its own streams, maybe none) and the sequence number, so that waiting for the
+     * group's latest command (nnsp_b200_group_set_stream_params, group_wait) also waits until it is recorded */
+    const long long seq = ++g->seq;
+    for (Member *m : g->members) {
+        Command c{ Command::RESET_STREAMS, nullptr, 0, mode, nullptr, seq, {} };
+        for (int i = 0; i < n; i++)
+            if (streams[i] >= m->first && streams[i] < m->first + m->count) c.streams.push_back(streams[i] - m->first);
+        { std::lock_guard<std::mutex> lk(m->mu); m->queue.push_back(std::move(c)); }
+        m->cv_cmd.notify_one();
+    }
+    return NNSP_B200_OK;
+}
+
 void nnsp_b200_group_destroy(nnsp_b200_group *g)
 {
     if (!g) return;
     for (Member *m : g->members) {
         if (m->thread.joinable()) {
-            { std::lock_guard<std::mutex> lk(m->mu); m->queue.push_back(Command{ Command::QUIT, nullptr, 0, 0, nullptr, 0 }); }
+            { std::lock_guard<std::mutex> lk(m->mu); m->queue.push_back(Command{ Command::QUIT, nullptr, 0, 0, nullptr, 0, {} }); }
             m->cv_cmd.notify_one();
             m->thread.join();
         }
