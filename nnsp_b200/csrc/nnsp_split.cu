@@ -176,7 +176,7 @@ struct SegArgs {
     const DevTables *tables;
     int l0, l1;
     int w_base, w_bytes;            /* fragments of layers [l0, l1): uint2 offset in the image, byte count */
-    int off_bias, off_lut, off_w, off_fp, off_wb, off_log, nbuf;   /* shared-memory layout (seg_layout) */
+    int off_bias, off_lut, off_w, off_fp, off_row, off_wb, off_log, nbuf;   /* shared-memory layout (seg_layout) */
     StreamSel sel;
     int T, first, n_inf, nchunks;
     long long tile_bytes;           /* bytes of one tile's plane region (>= n_inf * 32 * pa) */
@@ -396,6 +396,12 @@ seg_kernel(SegArgs a)
     const int nsel = sel_count(a.sel);
     const int nitems = ((nsel + 15) >> 4) * a.nchunks;
     const size_t tile_base = sel_tile_base(a.sel);
+    /* MODE 2 staging: 16-byte pieces of 8 features as in MODE 1. Thread (px, pj, pr) stages features 8 px .. 8 px + 7 of
+     * rows j = pj, pj + JP, ... of tile row pr, so it standardises with the same 8 (mean, stdR) pairs throughout; consecutive
+     * threads write consecutive pieces of a row, then the next row. */
+    constexpr int JP = SEG_THREADS / 80;
+    static_assert(JP >= 1 && SEG_FROWS % JP == 0, "staging threads");
+    const int px = tid % 5, pr = tid / (5 * JP), pj = tid / 5 - pr * JP;
     __syncthreads();
 
     for (int item = blockIdx.x; item < nitems; item += gridDim.x) {
@@ -463,52 +469,69 @@ seg_kernel(SegArgs a)
             } else {
                 /* cascade: frame f of the instance is raw frame f - dback (PcmBufClass_getData look-back,
                  * PcmBufClass.c:38-85): its log-mel row comes from this call or from the carried history and is
-                 * standardised with this model's statistics (feature_module.c:67-73) */
-                constexpr int NQ = 16 * SEG_FROWS * 10;              /* pieces of 4 features */
-                for (int e0 = 0; e0 < NQ; e0 += 4 * SEG_THREADS) {
-                    int4 v[4];
-                    int from_ctx[4];
-#pragma unroll
-                    for (int u = 0; u < 4; u++) {
-                        const int e = e0 + u * SEG_THREADS + tid;
-                        v[u] = make_int4(0, 0, 0, 0);
-                        from_ctx[u] = 1;
-                        if (e < NQ) {
-                            const int r = e / (SEG_FROWS * 10), rem = e - r * (SEG_FROWS * 10), j = rem / 10, x = rem - j * 10;
-                            if (r < nvalid) {
-                                const long long s = sids[r];
-                                const int f = s_ts[r] + 2 * k0 - 5 + j;              /* frame of the call */
-                                const int life = f - s_tb[r];                        /* frames since the instance's life in this call began */
-                                if (life < 0) {                                      /* before that: the instance's stored context rows 1..5 */
-                                    const uint2 c = *reinterpret_cast<const uint2 *>(a.ctx + s * 240 + (6 + life) * 40 + x * 4);
-                                    v[u] = make_int4((int16_t)(c.x & 0xffff), (int32_t)c.x >> 16, (int16_t)(c.y & 0xffff), (int32_t)c.y >> 16);
-                                } else if (f < s_te[r]) {                            /* frames past the row's own end stage as zeros */
-                                    const int la = life + s_ag[r], fr = f - a.dback;
-                                    const int32_t *row = (la < 2) ? a.lmfix + (s * 2 + la) * NNSP_B200_NMEL     /* STFT buffer still partly zero */
-                                                       : (fr >= 0) ? a.logmel + (s * T + fr) * NNSP_B200_NMEL
-                                                                   : a.lmhist + (s * a.dmax + a.dmax + fr) * NNSP_B200_NMEL;
-                                    v[u] = __ldg(reinterpret_cast<const int4 *>(row + x * 4));
-                                    from_ctx[u] = 0;
-                                }
-                            }
+                 * standardised with this model's statistics (feature_module.c:67-73). The source of each staged row is
+                 * resolved once per item: a log-mel row (int32), a stored context row (int16, already standardised,
+                 * tagged by bit 0) or none (0: the row stages as zeros) */
+                uintptr_t *s_row = reinterpret_cast<uintptr_t *>(smem + a.off_row);    /* [16][SEG_FROWS] */
+                for (int j = tid >> 4; j < SEG_FROWS; j += SEG_THREADS >> 4) {
+                    const int r = tid & 15;
+                    uintptr_t src = 0;
+                    if (r < nvalid) {
+                        const long long s = sids[r];
+                        const int f = s_ts[r] + 2 * k0 - 5 + j;                      /* frame of the call */
+                        const int life = f - s_tb[r];                                /* frames since the instance's life in this call began */
+                        if (life < 0) {                                              /* before that: the instance's stored context rows 1..5 */
+                            src = reinterpret_cast<uintptr_t>(a.ctx + s * 240 + (6 + life) * 40) | 1;
+                        } else if (f < s_te[r]) {                                    /* frames past the row's own end stage as zeros */
+                            const int la = life + s_ag[r], fr = f - a.dback;
+                            src = reinterpret_cast<uintptr_t>((la < 2) ? a.lmfix + (s * 2 + la) * NNSP_B200_NMEL   /* STFT buffer still partly zero */
+                                                            : (fr >= 0) ? a.logmel + (s * T + fr) * NNSP_B200_NMEL
+                                                                        : a.lmhist + (s * a.dmax + a.dmax + fr) * NNSP_B200_NMEL);
                         }
                     }
+                    s_row[r * SEG_FROWS + j] = src;
+                }
+                __syncthreads();
+                if (tid < 80 * JP) {
+                    int32_t mn[8], sd[8];                                    /* the thread's features: registers, not a shared load per value */
 #pragma unroll
-                    for (int u = 0; u < 4; u++) {
-                        const int e = e0 + u * SEG_THREADS + tid;
-                        if (e < NQ) {
-                            const int r = e / (SEG_FROWS * 10), rem = e - r * (SEG_FROWS * 10), j = rem / 10, x = rem - j * 10;
-                            int w[4] = { v[u].x, v[u].y, v[u].z, v[u].w };
-                            if (!from_ctx[u]) {
+                    for (int c = 0; c < 8; c++) { mn[c] = M.mean[8 * px + c]; sd[c] = M.stdR[8 * px + c]; }
+                    const int rs = M.feat_rshift;
+                    const uintptr_t *rows = s_row + pr * SEG_FROWS + pj;
+                    uint8_t *dst = fplanes + pr * SEG_PC + pj * 40 + px * 8;
+                    constexpr int NP = SEG_FROWS / JP;                       /* pieces per thread */
+#pragma unroll 1
+                    for (int m0 = 0; m0 < NP; m0 += 4) {
+                        int4 v[4][2];                                        /* log-mel values */
+                        uint4 w[4];                                          /* 8 int16 features, pairwise: context rows, zeros */
+                        bool lm[4];
 #pragma unroll
-                                for (int c = 0; c < 4; c++) w[c] = standardise(w[c], M.mean[4 * x + c], M.stdR[4 * x + c], M.feat_rshift);
+                        for (int u = 0; u < 4; u++) {
+                            const bool in = NP % 4 == 0 || m0 + u < NP;
+                            const uintptr_t src = in ? rows[(m0 + u) * JP] : 0;
+                            const bool cx = src & 1;
+                            const int4 *p = reinterpret_cast<const int4 *>(src & ~(uintptr_t)1) + (cx ? px : 2 * px);
+                            lm[u] = src && !cx;
+                            v[u][0] = lm[u] ? __ldg(p) : make_int4(0, 0, 0, 0);
+                            v[u][1] = lm[u] ? __ldg(p + 1) : make_int4(0, 0, 0, 0);
+                            w[u] = cx ? __ldg(reinterpret_cast<const uint4 *>(p)) : make_uint4(0, 0, 0, 0);
+                        }
+#pragma unroll
+                        for (int u = 0; u < 4; u++) {
+                            if (NP % 4 != 0 && m0 + u >= NP) break;
+                            if (lm[u]) {
+                                const int32_t e[8] = { v[u][0].x, v[u][0].y, v[u][0].z, v[u][0].w, v[u][1].x, v[u][1].y, v[u][1].z, v[u][1].w };
+                                int32_t z[8];
+#pragma unroll
+                                for (int c = 0; c < 8; c++) z[c] = standardise(e[c], mn[c], sd[c], rs);
+                                w[u].x = __byte_perm(z[0], z[1], 0x5410); w[u].y = __byte_perm(z[2], z[3], 0x5410);
+                                w[u].z = __byte_perm(z[4], z[5], 0x5410); w[u].w = __byte_perm(z[6], z[7], 0x5410);
                             }
-                            const uint32_t hi = ((uint32_t)(w[0] >> 8) & 0xff) | (((uint32_t)(w[1] >> 8) & 0xff) << 8) |
-                                                (((uint32_t)(w[2] >> 8) & 0xff) << 16) | (((uint32_t)(w[3] >> 8) & 0xff) << 24);
-                            const uint32_t lo = ((uint32_t)w[0] & 0xff) | (((uint32_t)w[1] & 0xff) << 8) |
-                                                (((uint32_t)w[2] & 0xff) << 16) | (((uint32_t)w[3] & 0xff) << 24);
-                            *reinterpret_cast<uint32_t *>(fplanes + r * SEG_PC + j * 40 + x * 4) = hi;
-                            *reinterpret_cast<uint32_t *>(fplanes + (16 + r) * SEG_PC + j * 40 + x * 4) = lo;
+                            uint2 hi, lo;
+                            lo.x = __byte_perm(w[u].x, w[u].y, 0x6420); hi.x = __byte_perm(w[u].x, w[u].y, 0x7531);
+                            lo.y = __byte_perm(w[u].z, w[u].w, 0x6420); hi.y = __byte_perm(w[u].z, w[u].w, 0x7531);
+                            *reinterpret_cast<uint2 *>(dst + (m0 + u) * JP * 40) = hi;
+                            *reinterpret_cast<uint2 *>(dst + 16 * SEG_PC + (m0 + u) * JP * 40) = lo;
                         }
                     }
                 }
@@ -977,9 +1000,10 @@ __global__ void feat_tap_kernel(const int16_t *__restrict__ feat16, int16_t *fea
 /* ======================================================================================================== */
 /* host                                                                                                      */
 /* ======================================================================================================== */
-struct SegLayout { int off_bias, off_lut, off_w, off_fp, off_wb, off_log, nbuf, w_base, w_bytes; size_t total; };
+struct SegLayout { int off_bias, off_lut, off_w, off_fp, off_row, off_wb, off_log, nbuf, w_base, w_bytes; size_t total; };
 
-static SegLayout seg_layout(const MmaModel *D, int l0, int l1, bool from_feat)
+/* row_tab: the per-item source table of the log-mel staging (seg_kernel<2>) */
+static SegLayout seg_layout(const MmaModel *D, int l0, int l1, bool from_feat, bool row_tab)
 {
     SegLayout s{};
     auto a16 = [](size_t v) { return (v + 15) & ~(size_t)15; };
@@ -993,6 +1017,7 @@ static SegLayout seg_layout(const MmaModel *D, int l0, int l1, bool from_feat)
     off = (off + 127) & ~(size_t)127;
     s.off_w = (int)off; off += (size_t)s.w_bytes;
     s.off_fp = (int)off; if (from_feat) off += 2 * 16 * SEG_PC;
+    s.off_row = (int)off; if (row_tab) off += 16 * SEG_FROWS * sizeof(uintptr_t);
     s.nbuf = (from_feat && l1 - l0 == 1) ? 1 : 2;
     s.off_wb = (int)off; off += (size_t)SEG_WARPS * s.nbuf * 32 * D->pa;
     s.off_log = (int)off; if (l1 == D->numlayers) off += (size_t)SEG_WARPS * 16 * (D->no + 4) * 4;
@@ -1020,7 +1045,8 @@ int split_supported(const MmaDeviceModel &mm)
     for (int l0 = 0; l0 < D->numlayers;) {                           /* every fc run must fit shared memory */
         int l1 = l0;
         while (l1 < D->numlayers && D->layer[l1].type == LAYER_FC) l1++;
-        if (l1 > l0 && seg_layout(D, l0, l1, l0 == 0).total > (size_t)SPLIT_MAX_DYN_SMEM) return 0;
+        /* with the staging table: any model may run in a cascade */
+        if (l1 > l0 && seg_layout(D, l0, l1, l0 == 0, l0 == 0).total > (size_t)SPLIT_MAX_DYN_SMEM) return 0;
         l0 = (l1 > l0) ? l1 : l0 + 1;
     }
     return 1;
@@ -1196,11 +1222,11 @@ int launch_split_layers(const MmaDeviceModel &mm, const SplitGroup &q, int devic
             li = l1;
         } else
         if (l1 > li) {                                           /* a run of fc layers */
-            const SegLayout lay = seg_layout(D, li, l1, from_feat);
+            const SegLayout lay = seg_layout(D, li, l1, from_feat, from_feat && q.mode == 2);
             SegArgs a{};
             a.model = mm.d; a.frag = (const uint2 *)mm.frag; a.bias32 = mm.bias32; a.tables = q.tables;
             a.l0 = li; a.l1 = l1; a.w_base = lay.w_base; a.w_bytes = lay.w_bytes;
-            a.off_bias = lay.off_bias; a.off_lut = lay.off_lut; a.off_w = lay.off_w; a.off_fp = lay.off_fp;
+            a.off_bias = lay.off_bias; a.off_lut = lay.off_lut; a.off_w = lay.off_w; a.off_fp = lay.off_fp; a.off_row = lay.off_row;
             a.off_wb = lay.off_wb; a.off_log = lay.off_log; a.nbuf = lay.nbuf;
             a.sel = sel; a.T = q.T; a.first = q.first; a.n_inf = q.n_inf; a.nchunks = nchunks;
             a.tile_bytes = tile_bytes; a.dec_stride = q.dec_stride;
