@@ -225,6 +225,50 @@ int nnsp_b200_cascade_reset(nnsp_b200_cascade *c);
 #define NNSP_B200_RESET_INSTANCE 0
 #define NNSP_B200_RESET_FRESH    1
 int nnsp_b200_cascade_reset_streams(nnsp_b200_cascade *c, const int32_t *streams, int n, int mode);
+/* Sessions: the whole state of a stream as a record, to continue it in another slot, another handle or process, or on
+ * another GPU (export, import into the new slot, FRESH reset of the old one). Record i of a call covers streams[i];
+ * every record of a handle is nnsp_b200_cascade_stream_state_bytes long, which depends on its look-back depths. It
+ * starts with this header; the body behind it is versioned and opaque: the controller scalars (sequence position,
+ * both time-out counters, the instance's age in frames), the NNSPClass scalars, the context rows, LSTM h and c at
+ * NNSP_B200_MAX_WIDTH, context row 5 of every instance, the PCM ring and the log-mel history (DESIGN.md sections 3,
+ * 4.3). Per-stream parameters (nnsp_b200_cascade_set_stream_params) are NOT in the record: they stay configuration of
+ * the slot, and a caller with custom thresholds sets them on the destination slot. */
+#define NNSP_B200_STREAM_MAGIC   0x5353504eu   /* "NPSS" little endian */
+#define NNSP_B200_STREAM_VERSION 1u
+typedef struct {
+    uint32_t magic;            /* NNSP_B200_STREAM_MAGIC                                                       */
+    uint32_t version;          /* NNSP_B200_STREAM_VERSION                                                     */
+    uint32_t record_bytes;     /* nnsp_b200_cascade_stream_state_bytes of the writing handle                   */
+    int32_t  len_seq;          /* the cascade sequence of the writing handle ...                               */
+    int32_t  seq[3];           /* ... entries past len_seq are -1                                               */
+    int16_t  frs_vbufBk_kws;   /* the handle's look-back depths (nnsp_b200_cascade_params)                      */
+    int16_t  frs_vbufBk_s2i;
+    uint64_t model_fnv1a[3];   /* 64-bit FNV-1a of the NNSPM1 blob (nnsp_b200_model_to_blob) of the model at seq[k],
+                                  which covers its accumulator mode; 0 past len_seq                               */
+    uint64_t reserved;         /* 0                                                                             */
+} nnsp_b200_stream_header;     /* 64 bytes */
+size_t nnsp_b200_cascade_stream_state_bytes(const nnsp_b200_cascade *c);
+/* Export: synchronous. Waits for every call issued on the handle (asynchronous host tickets included, whose results
+ * are then complete), applies the resets and imports still pending, and writes the record of streams[i] to
+ * records + i * stream_state_bytes: the state the stream's next call would start from. A stream may be listed twice;
+ * n == 0 does nothing. The next call starts on an idle device, without the overlap it would have had with the
+ * previous call (DESIGN.md section 4.3). An id outside [0, n_streams) or n < 0 returns NNSP_B200_ERR_ARG. */
+int nnsp_b200_cascade_export_streams(nnsp_b200_cascade *c, const int32_t *streams, int n, void *records);
+/* Import: like nnsp_b200_cascade_reset_streams, the records are checked and copied before the call returns and nothing
+ * waits for the device; the listed slots start the NEXT exec call of any kind (device, ragged, host, host-async,
+ * tapped) from the imported state, calls issued before are not affected. Pending operations on one slot compose in
+ * call order as if each had been applied when issued: import then INSTANCE reset loads the record and then applies
+ * nnCntrlClass_reset to it (its position and context row 5 kept); import then FRESH is FRESH; a reset then an import,
+ * or two imports, leave the last import; nnsp_b200_cascade_reset counts as an INSTANCE reset of every stream.
+ * Returns NNSP_B200_ERR_ARG and records nothing for n < 0, an id outside [0, n_streams), a slot listed twice, or a
+ * record with a bad magic, version or record_bytes, or whose sequence, look-back depths or model fingerprints differ
+ * from this handle's. The body fields that the kernels use as an index or a loop bound are range-checked too, so
+ * that no corrupted or foreign record reaches the device: the sequence position (< len_seq), the instance's age
+ * (<= 2), both time-out counters (< 32767, the longest time-out a parameter can set), the stride-2 gate
+ * NNSPClass.slides (0 or 1) and the last S2I argmax (0 .. 6). Like reset_streams, a call that carries imports uploads
+ * them from double-buffered pinned staging and waits on the host before it reuses a staging buffer until the device
+ * has run the kernels that read that buffer's records two import-carrying calls back. */
+int nnsp_b200_cascade_import_streams(nnsp_b200_cascade *c, const int32_t *streams, int n, const void *records);
 /* ParamCntrlClass belongs to a controller instance (nnCntrlClass.h:12-29), i.e. to a stream: params[i] becomes the
  * parameter set of stream first_stream + i (thresholds, counts, time-outs; the two look-back depths must equal the
  * handle's, they size its history buffers). Waits for the handle's work in flight; takes effect with the next call and
@@ -302,6 +346,14 @@ int nnsp_b200_group_set_stream_params(nnsp_b200_group *g, int first_stream, int 
  * NNSP_B200_ERR_ARG). Checked and copied before it returns, queued in order with the group's calls in each member's
  * command queue: the listed streams start the next call issued after it from the reset state. Does not wait. */
 int nnsp_b200_group_reset_streams(nnsp_b200_group *g, const int32_t *streams, int n, int mode);
+/* Sessions in the group's stream numbering (cascade groups; a batch group returns NNSP_B200_ERR_ARG and its state
+ * bytes are 0). The records are those of the member handles, all the same size. Export is a command to every member,
+ * in order with the group's calls, and waits for it: the members gather in parallel, each into the records of its own
+ * streams. Import is checked and copied before it returns and queued in order with the calls like reset_streams. A move
+ * of stream a to slot b, also across members and so across GPUs: export [a], import into [b], FRESH reset of [a]. */
+size_t nnsp_b200_group_stream_state_bytes(const nnsp_b200_group *g);
+int nnsp_b200_group_export_streams(nnsp_b200_group *g, const int32_t *streams, int n, void *records);
+int nnsp_b200_group_import_streams(nnsp_b200_group *g, const int32_t *streams, int n, const void *records);
 int nnsp_b200_group_exec_host(nnsp_b200_group *g, const int16_t *pcm, long long stream_stride, int n_frames, void *results);
 int nnsp_b200_group_exec_host_async(nnsp_b200_group *g, const int16_t *pcm, long long stream_stride, int n_frames,
                                     void *results, long long *ticket);

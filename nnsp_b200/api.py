@@ -258,6 +258,15 @@ class NNSPBatch:
             pass
 
 
+def _records_in(records, n, size):
+    """a stream-record buffer (bytes or any numpy array) as contiguous bytes of n records"""
+    b = np.frombuffer(records, np.uint8) if isinstance(records, (bytes, bytearray, memoryview)) \
+        else np.ascontiguousarray(records).view(np.uint8).ravel()
+    if b.size != n * size:
+        raise ValueError("%d bytes of stream records for %d streams of %d bytes each" % (b.size, n, size))
+    return b
+
+
 class Cascade:
     """n_streams independent nnCntrlClass controllers (VAD -> KWS -> S2I by default)."""
 
@@ -294,6 +303,26 @@ class Cascade:
         s = np.ascontiguousarray(streams, np.int32).ravel()
         check(lib().nnsp_b200_cascade_reset_streams(self.h, s.ctypes.data_as(C.c_void_p), len(s), 1 if fresh else 0),
               "cascade_reset_streams")
+
+    def stream_state_bytes(self):
+        return int(lib().nnsp_b200_cascade_stream_state_bytes(self.h))
+
+    def export_streams(self, streams):
+        """The records of the listed streams (bytes, stream_state_bytes() each, in list order): waits for every call issued,
+        applies pending resets and imports, and returns the state each stream's next call would start from."""
+        s = np.ascontiguousarray(streams, np.int32).ravel()
+        out = np.empty(len(s) * self.stream_state_bytes(), np.uint8)
+        check(lib().nnsp_b200_cascade_export_streams(self.h, s.ctypes.data_as(C.c_void_p), len(s), out.ctypes.data_as(C.c_void_p)),
+              "cascade_export_streams")
+        return out.tobytes()
+
+    def import_streams(self, streams, records):
+        """Load records (bytes or a numpy buffer, as export_streams returns them) into the listed slots before the next call
+        of any kind, without waiting for the device. Per-stream parameters are the slot's and are not changed."""
+        s = np.ascontiguousarray(streams, np.int32).ravel()
+        b = _records_in(records, len(s), self.stream_state_bytes())
+        check(lib().nnsp_b200_cascade_import_streams(self.h, s.ctypes.data_as(C.c_void_p), len(s), b.ctypes.data_as(C.c_void_p)),
+              "cascade_import_streams")
 
     def set_stream_params(self, first_stream, params):
         """params: [n][10] int16, rows in the field order of ParamCntrlClass (what params_array() returns for the handle)"""
@@ -467,6 +496,24 @@ class Group:
         s = np.ascontiguousarray(streams, np.int32).ravel()
         check(lib().nnsp_b200_group_reset_streams(self.h, s.ctypes.data_as(C.c_void_p), len(s), 1 if fresh else 0),
               "group_reset_streams")
+
+    def stream_state_bytes(self):
+        return int(lib().nnsp_b200_group_stream_state_bytes(self.h))
+
+    def export_streams(self, streams):
+        """cascade groups: Cascade.export_streams in the group's stream numbering, in order with the group's calls"""
+        s = np.ascontiguousarray(streams, np.int32).ravel()
+        out = np.empty(len(s) * self.stream_state_bytes(), np.uint8)
+        check(lib().nnsp_b200_group_export_streams(self.h, s.ctypes.data_as(C.c_void_p), len(s), out.ctypes.data_as(C.c_void_p)),
+              "group_export_streams")
+        return out.tobytes()
+
+    def import_streams(self, streams, records):
+        """cascade groups: Cascade.import_streams in the group's stream numbering, queued in order with the group's calls"""
+        s = np.ascontiguousarray(streams, np.int32).ravel()
+        b = _records_in(records, len(s), self.stream_state_bytes())
+        check(lib().nnsp_b200_group_import_streams(self.h, s.ctypes.data_as(C.c_void_p), len(s), b.ctypes.data_as(C.c_void_p)),
+              "group_import_streams")
 
     def set_stream_params(self, first_stream, params):
         """cascade groups: params [n][10] int16 in the field order of ParamCntrlClass, global stream numbering"""

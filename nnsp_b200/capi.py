@@ -27,6 +27,16 @@ class CascadeParams(C.Structure):
         "thresh_cnts_s2i", "frs_vbufBk_kws", "thresh_timeout_kws", "thresh_prob_kws", "thresh_cnts_kws")]
 
 
+class StreamHeader(C.Structure):
+    """nnsp_b200_stream_header: the head of every stream record (Cascade.export_streams)"""
+    _fields_ = [("magic", C.c_uint32), ("version", C.c_uint32), ("record_bytes", C.c_uint32), ("len_seq", C.c_int32),
+                ("seq", C.c_int32 * 3), ("frs_vbufBk_kws", C.c_int16), ("frs_vbufBk_s2i", C.c_int16),
+                ("model_fnv1a", C.c_uint64 * 3), ("reserved", C.c_uint64)]
+
+
+STREAM_MAGIC, STREAM_VERSION = 0x5353504E, 1
+
+
 class NnspError(RuntimeError):
     pass
 
@@ -48,7 +58,9 @@ nnsp_b200_group_create_batch nnsp_b200_group_create_cascade nnsp_b200_group_size
 nnsp_b200_group_exec_host nnsp_b200_group_exec_host_async nnsp_b200_group_wait nnsp_b200_group_destroy
 nnsp_b200_batch_set_host_format nnsp_b200_cascade_set_host_format nnsp_b200_wav_info nnsp_b200_wav_read_frames nnsp_b200_wav_load_streams nnsp_b200_cascade_timeline
 nnsp_b200_cascade_exec_ragged nnsp_b200_cascade_exec_host_ragged_async nnsp_b200_scan_kernel_launches
-nnsp_b200_cascade_reset_streams nnsp_b200_group_reset_streams""".split()
+nnsp_b200_cascade_reset_streams nnsp_b200_group_reset_streams
+nnsp_b200_cascade_stream_state_bytes nnsp_b200_cascade_export_streams nnsp_b200_cascade_import_streams
+nnsp_b200_group_stream_state_bytes nnsp_b200_group_export_streams nnsp_b200_group_import_streams""".split()
 
 
 def lib():
@@ -102,6 +114,10 @@ def lib():
         L.nnsp_b200_cascade_reset.argtypes = [vp]
         L.nnsp_b200_cascade_set_stream_params.argtypes = [vp, ci, ci, vp]
         L.nnsp_b200_cascade_reset_streams.argtypes = [vp, vp, ci, ci]
+        L.nnsp_b200_cascade_stream_state_bytes.argtypes = [vp]
+        L.nnsp_b200_cascade_stream_state_bytes.restype = C.c_size_t
+        L.nnsp_b200_cascade_export_streams.argtypes = [vp, vp, ci, vp]
+        L.nnsp_b200_cascade_import_streams.argtypes = [vp, vp, ci, vp]
         L.nnsp_b200_cascade_exec.argtypes = [vp, vp, ll, ci, vp, C.POINTER(Taps)]
         L.nnsp_b200_cascade_exec_host.argtypes = [vp, vp, ll, ci, vp]
         L.nnsp_b200_cascade_exec_host_async.argtypes = [vp, vp, ll, ci, vp, C.POINTER(ll)]
@@ -138,6 +154,10 @@ def lib():
     L.nnsp_b200_group_reset.argtypes = [vp]
     L.nnsp_b200_group_set_stream_params.argtypes = [vp, ci, ci, vp]
     L.nnsp_b200_group_reset_streams.argtypes = [vp, vp, ci, ci]
+    L.nnsp_b200_group_stream_state_bytes.argtypes = [vp]
+    L.nnsp_b200_group_stream_state_bytes.restype = C.c_size_t
+    L.nnsp_b200_group_export_streams.argtypes = [vp, vp, ci, vp]
+    L.nnsp_b200_group_import_streams.argtypes = [vp, vp, ci, vp]
     L.nnsp_b200_group_exec_host.argtypes = [vp, vp, ll, ci, vp]
     L.nnsp_b200_group_exec_host_async.argtypes = [vp, vp, ll, ci, vp, C.POINTER(ll)]
     L.nnsp_b200_group_wait.argtypes = [vp, ll]

@@ -945,21 +945,60 @@ __global__ void __launch_bounds__(256) cascade_ctx_kernel(CascadePostArgs a)
 
 struct ResetModels { const DevModel *m[3]; int seq[CS_MAXSEQ]; };
 
+/* A stream's record (nnsp_b200_cascade_export_streams): the 64-byte nnsp_b200_stream_header, then the state at these
+ * byte offsets, every part a multiple of 8 bytes at an 8-byte aligned offset; the PCM ring (hist_words 32-bit words)
+ * at REC_RING, the log-mel history (lm_words) behind it. In the records a call stages for its imports, the header's
+ * `reserved` word holds the destination stream instead (REC_DEST). */
+constexpr int REC_DEST = 56, REC_SCAL = 64, REC_CASC = 96, REC_PAD = 104, REC_CTX = 112, REC_H = 592, REC_C = 848,
+              REC_STALE = 1360, REC_RING = 1600;
+static_assert(REC_H == REC_CTX + 240 * 2 && REC_C == REC_H + NNSP_B200_MAX_WIDTH * 2 &&
+              REC_STALE == REC_C + NNSP_B200_MAX_WIDTH * 4 && REC_RING == REC_STALE + 120 * 2, "record layout");
+__host__ __device__ constexpr long long rec_bytes_of(int hist_words, int lm_words) { return REC_RING + 4LL * (hist_words + lm_words); }
+
+__device__ __forceinline__ void copy8(void *dst, const void *src, int nbytes)
+{
+    uint2 *d = reinterpret_cast<uint2 *>(dst);
+    const uint2 *q = reinterpret_cast<const uint2 *>(src);
+    for (int i = threadIdx.x; i < nbytes / 8; i += blockDim.x) d[i] = q[i];
+}
+
+/* Entries of a device list of pending operations: (stream << 2 | op) for the resets, (record << 2 | op) for the ops that
+ * load a staged record, which names its stream at REC_DEST. OP_INSTANCE / OP_FRESH are NNSP_B200_RESET_INSTANCE / _FRESH. */
+constexpr int OP_INSTANCE = 0, OP_FRESH = 1, OP_LOAD = 2, OP_LOAD_INSTANCE = 3;
+
 /* nnCntrlClass_reset (nnCntrlClass.c:130-150): every instance reset, ring cleared, timeout counters
  * zeroed; current_pos_seq is NOT rewound (only nnCntrlClass_init sets it, :125) and every instance keeps
  * its context row 5. fresh != 0 (create = init + reset on zeroed structs) also rewinds and clears those.
- * list == null: streams 0 .. S-1, one per CTA, all with `fresh`; else the streams list[0 .. gridDim.x), each entry
- * (stream << 1 | fresh). `parts` says what is written: the PCM ring, which the front end reads, and the controller /
+ * list == null: streams 0 .. S-1, one per CTA, all with `fresh`; else the entries list[0 .. gridDim.x) (OP_*):
+ * OP_LOAD writes the record recs[entry >> 2] into its stream, OP_LOAD_INSTANCE does that and then the reset.
+ * `parts` says what is written: the PCM ring, which the front end reads, and the controller /
  * instance state with the log-mel history, which the chain reads -- a pipelined call resets them on different streams. */
 constexpr int RESET_RING = 1, RESET_STATE = 2;
 __global__ void cascade_reset_kernel(ResetModels rm, StreamState st, int16_t *stale, int S,
-                                     int hist_words, int lm_words, int fresh, const int *list, int parts)
+                                     int hist_words, int lm_words, int fresh, const int *list, int parts, const uint8_t *recs)
 {
-    int s = blockIdx.x;
-    if (list) { const int e = list[blockIdx.x]; s = e >> 1; fresh = e & 1; }
+    int s = blockIdx.x, op = fresh;
+    const uint8_t *rec = nullptr;
+    if (list) {
+        const int e = list[blockIdx.x];
+        op = e & 3;
+        if (op & OP_LOAD) { rec = recs + (e >> 2) * rec_bytes_of(hist_words, lm_words); s = *reinterpret_cast<const int *>(rec + REC_DEST); }
+        else s = e >> 2;
+    }
     if (s >= S) return;
     const int HS = NNSP_B200_MAX_WIDTH;
-    if (parts & RESET_STATE) {
+    if ((parts & RESET_STATE) && rec) {
+        copy8(st.scal + (long long)s * SC_N, rec + REC_SCAL, SC_N * 2);
+        copy8(st.casc + (long long)s * CS_N, rec + REC_CASC, CS_N * 2);
+        copy8(st.ctx + (long long)s * 240, rec + REC_CTX, 240 * 2);
+        copy8(st.h + (long long)s * HS, rec + REC_H, HS * 2);
+        copy8(st.c + (long long)s * HS, rec + REC_C, HS * 4);
+        copy8(stale + (long long)s * 120, rec + REC_STALE, 120 * 2);
+        copy8(st.lmhist + (long long)s * lm_words, rec + REC_RING + 4LL * hist_words, lm_words * 4);
+    }
+    if ((parts & RESET_STATE) && op != OP_LOAD) {
+        const bool fresh = op == OP_FRESH;
+        __syncthreads();                                                  /* the position a load just wrote */
         const int pos = fresh ? 0 : st.casc[(long long)s * CS_N + CS_POS];
         const DevModel *M = rm.m[rm.seq[pos]];
         __syncthreads();
@@ -976,8 +1015,28 @@ __global__ void cascade_reset_kernel(ResetModels rm, StreamState st, int16_t *st
     }
     if (parts & RESET_RING) {
         unsigned int *h = reinterpret_cast<unsigned int *>(st.hist) + (long long)s * hist_words;
-        for (int i = threadIdx.x; i < hist_words; i += blockDim.x) h[i] = 0;                   /* PcmBufClass_reset, PcmBufClass.c:19-28 */
+        if (op == OP_LOAD) copy8(h, rec + REC_RING, hist_words * 4);
+        else for (int i = threadIdx.x; i < hist_words; i += blockDim.x) h[i] = 0;              /* PcmBufClass_reset, PcmBufClass.c:19-28 */
     }
+}
+
+/* the records of the streams ids[0 .. gridDim.x), one per CTA, into out: header `hdr`, then the state (REC_*) */
+__global__ void cascade_export_kernel(StreamState st, const int16_t *stale, const int *ids, uint8_t *out, int hist_words,
+                                      int lm_words, nnsp_b200_stream_header hdr)
+{
+    const long long s = ids[blockIdx.x];
+    const int HS = NNSP_B200_MAX_WIDTH;
+    uint8_t *rec = out + blockIdx.x * rec_bytes_of(hist_words, lm_words);
+    copy8(rec, &hdr, (int)sizeof hdr);
+    if (threadIdx.x == 0) *reinterpret_cast<uint2 *>(rec + REC_PAD) = make_uint2(0, 0);
+    copy8(rec + REC_SCAL, st.scal + s * SC_N, SC_N * 2);
+    copy8(rec + REC_CASC, st.casc + s * CS_N, CS_N * 2);
+    copy8(rec + REC_CTX, st.ctx + s * 240, 240 * 2);
+    copy8(rec + REC_H, st.h + s * HS, HS * 2);
+    copy8(rec + REC_C, st.c + s * HS, HS * 4);
+    copy8(rec + REC_STALE, stale + s * 120, 120 * 2);
+    copy8(rec + REC_RING, st.hist + s * hist_words * 2, hist_words * 4);
+    copy8(rec + REC_RING + 4LL * hist_words, st.lmhist + s * lm_words, lm_words * 4);
 }
 
 }  // namespace nnsp
@@ -1052,12 +1111,28 @@ struct nnsp_b200_cascade {
      * resets; rs_copied[b][j] marks the end of the copies out of rs_host[b] on pipeline stream j (0: c->stream for device
      * calls). A device-buffer call uses rs_dev[its pipe index] (rewritten after the chain two calls back, like the log-mel
      * rows); a host-buffer call puts slice [s0, s1)'s entries at rs_dev[0] + s0, always on the slice's own stream. */
-    std::vector<int8_t> rs_mode;
+    std::vector<int8_t> rs_mode;               /* OP_* or -1 */
     std::vector<int> rs_ids;
+    std::vector<int> rs_taken, rs_taken_loads; /* the latest take: its streams in list order, loads before each entry (+ total) */
     int *rs_host[2] = { nullptr, nullptr }, *rs_dev[2] = { nullptr, nullptr };
     cudaEvent_t rs_copied[2][3] = {};
     bool rs_copy_valid[2][3] = {};
     unsigned rs_flushes = 0;
+    /* nnsp_b200_cascade_import_streams: the pending record of a stream whose mode is OP_LOAD / OP_LOAD_INSTANCE sits at
+     * slot ip_slot[s] of ip_pool (a stream imported and then reset FRESH keeps its slot, unused, until the take; every
+     * pending stream's slot is released when the pool is emptied). The call that takes it packs the records of its loads, in list order, into pinned
+     * rp_host[b] (b as rs_host) and copies them to rp_dev[b] on the streams of the kernels that read them; rp_read[b][j]
+     * marks the end of those kernels on pipeline stream j (0..2: c->stream / the host slices' streams, 3: nn_stream), and
+     * both buffers of b are rewritten only after them. Capacities in records, grown on demand. */
+    std::vector<uint8_t> ip_pool;
+    std::vector<int> ip_slot;
+    uint8_t *rp_host[2] = { nullptr, nullptr }, *rp_dev[2] = { nullptr, nullptr };
+    int rp_cap[2] = { 0, 0 };
+    cudaEvent_t rp_read[2][4] = {};
+    bool rp_read_valid[2][4] = {};
+    int *ex_ids = nullptr; uint8_t *ex_dev = nullptr; long long ex_cap = 0;   /* export: device ids and records, grown on demand */
+    nnsp_b200_stream_header hdr{};             /* the header of this handle's records */
+    long long rec_bytes = 0;
 };
 
 constexpr int CS_MAX_SLICES = 8;
@@ -1112,58 +1187,103 @@ static int cascade_ensure_logmel(nnsp_b200_cascade *c, int T)
     return NNSP_B200_OK;
 }
 
-/* cascade_reset_kernel over every stream (list null, all `fresh`) or over the n entries of the device list */
-static int cascade_launch_reset(nnsp_b200_cascade *c, const int *list, int n, int fresh, int parts, cudaStream_t st)
+static int cascade_hist_words(const nnsp_b200_cascade *c) { return (c->cd.dmax + 2) * (NNSP_B200_FRAME / 2); }
+static int cascade_lm_words(const nnsp_b200_cascade *c) { return (c->cd.dmax > 0 ? c->cd.dmax : 1) * NNSP_B200_NMEL; }
+
+/* cascade_reset_kernel over every stream (list null, all `fresh`) or over the n entries of the device list, whose
+ * loads read the device records `recs` */
+static int cascade_launch_reset(nnsp_b200_cascade *c, const int *list, int n, int fresh, int parts, cudaStream_t st,
+                                const uint8_t *recs = nullptr)
 {
-    const int hist_frames = c->cd.dmax + 2, lm_rows = c->cd.dmax > 0 ? c->cd.dmax : 1;
     ResetModels rm{};
     for (int i = 0; i < 3; i++) rm.m[i] = c->dm[i].d;
     for (int i = 0; i < c->cd.len_seq; i++) rm.seq[i] = c->cd.seq[i];
-    cascade_reset_kernel<<<list ? n : c->S, 128, 0, st>>>(rm, c->st, c->stale, c->S, hist_frames * (NNSP_B200_FRAME / 2),
-                                                          lm_rows * NNSP_B200_NMEL, fresh, list, parts);
+    cascade_reset_kernel<<<list ? n : c->S, 128, 0, st>>>(rm, c->st, c->stale, c->S, cascade_hist_words(c), cascade_lm_words(c),
+                                                          fresh, list, parts, recs);
     NNSP_LAUNCH_CHECK();
     return NNSP_B200_OK;
 }
 
-/* The pending resets as a list sorted by stream in the pinned staging buffer of this call (*list, *n, *b = which one;
- * n == 0: none), and the pending set cleared. The buffer was last written by the reset-carrying call before last: the
- * host waits until the device has run that call's list copies, the only host wait resets add. Those copies sit in
- * stream order behind what was queued before them on their stream -- on a pipelined device call the wait for the chain
- * two calls back, on a host call the same slice of the ticket before -- so a caller that resets before every call runs
- * at most about two calls ahead of the device; calls without pending resets never wait here. */
-static int cascade_take_resets(nnsp_b200_cascade *c, const int **list, int *n, int *b)
+/* The pending resets and imports as a list sorted by stream in the pinned staging buffer of this call (*list, *n, *b =
+ * which one; n == 0: none), the records of its *loads in rp_host[*b], and the pending set cleared. The buffers were
+ * last written by the call before last that carried any: the host waits until the device has run that call's list
+ * copies -- and, when this call loads records, the kernels that read that call's records -- the only host waits these
+ * functions add. Those sit in stream order behind what was queued before them on their stream -- on a pipelined device
+ * call the wait for the chain two calls back (a record's reader: one call back), on a host call the same slice of the
+ * ticket before -- so a caller that resets before every call runs at most about two calls ahead of the device; calls
+ * without pending operations never wait here. */
+static int cascade_take_resets(nnsp_b200_cascade *c, const int **list, int *n, int *b, int *loads)
 {
     *n = (int)c->rs_ids.size();
+    *loads = 0;
     if (*n == 0) return NNSP_B200_OK;
     *b = (int)(c->rs_flushes++ & 1u);
     for (int j = 0; j < 3; j++)
         if (c->rs_copy_valid[*b][j]) { NNSP_CUDA(cudaEventSynchronize(c->rs_copied[*b][j])); c->rs_copy_valid[*b][j] = false; }
     std::sort(c->rs_ids.begin(), c->rs_ids.end());
-    int *h = c->rs_host[*b];
-    for (int k = 0; k < *n; k++) {
-        const int s = c->rs_ids[(size_t)k];
-        h[k] = (s << 1) | (c->rs_mode[(size_t)s] == NNSP_B200_RESET_FRESH ? 1 : 0);
-        c->rs_mode[(size_t)s] = -1;
-    }
+    c->rs_taken.swap(c->rs_ids);
     c->rs_ids.clear();
+    c->rs_taken_loads.resize((size_t)*n + 1);
+    for (int k = 0; k < *n; k++) {
+        c->rs_taken_loads[(size_t)k] = *loads;
+        if (c->rs_mode[(size_t)c->rs_taken[(size_t)k]] & OP_LOAD) ++*loads;
+    }
+    c->rs_taken_loads[(size_t)*n] = *loads;
+    if (*loads) {
+        for (int j = 0; j < 4; j++)
+            if (c->rp_read_valid[*b][j]) { NNSP_CUDA(cudaEventSynchronize(c->rp_read[*b][j])); c->rp_read_valid[*b][j] = false; }
+        if (*loads > c->rp_cap[*b]) {                                  /* nothing reads either buffer any more */
+            if (c->rp_host[*b]) NNSP_CUDA(cudaFreeHost(c->rp_host[*b]));
+            if (c->rp_dev[*b]) NNSP_CUDA(cudaFree(c->rp_dev[*b]));
+            c->rp_host[*b] = nullptr; c->rp_dev[*b] = nullptr; c->rp_cap[*b] = 0;
+            NNSP_CUDA(cudaHostAlloc(&c->rp_host[*b], (size_t)*loads * c->rec_bytes, cudaHostAllocDefault));
+            NNSP_CUDA(cudaMalloc(&c->rp_dev[*b], (size_t)*loads * c->rec_bytes));
+            c->rp_cap[*b] = *loads;
+        }
+    }
+    int *h = c->rs_host[*b];
+    for (int k = 0, l = 0; k < *n; k++) {
+        const int s = c->rs_taken[(size_t)k], op = c->rs_mode[(size_t)s];
+        if (op & OP_LOAD) {
+            uint8_t *r = c->rp_host[*b] + (size_t)l * c->rec_bytes;
+            memcpy(r, c->ip_pool.data() + (size_t)c->ip_slot[(size_t)s] * c->rec_bytes, (size_t)c->rec_bytes);
+            memcpy(r + REC_DEST, &s, sizeof s);
+            h[k] = (l++ << 2) | op;
+        } else
+            h[k] = (s << 2) | op;
+        c->rs_mode[(size_t)s] = -1;
+        c->ip_slot[(size_t)s] = -1;            /* also a slot whose import a FRESH reset replaced: the pool is emptied */
+    }
+    c->ip_pool.clear();
     *list = h;
     return NNSP_B200_OK;
 }
 
+/* what a call applies before its kernels read the state: the device list, the device records of its loads (null:
+ * none) and the events to record behind the kernels that read those records on the front-end stream and the chain's */
+struct PendingOps {
+    const int *list; int n;
+    const uint8_t *recs;
+    cudaEvent_t read_ring, read_state;
+};
+
 /* st_nn (with ev_feat): pipelined call -- everything behind the front end goes to st_nn, the PCM history is rolled out
  * of place on st right behind the front end (c->st.hist is swapped by the caller afterwards).
- * rlist (device, rn entries of cascade_take_resets, null: none): streams reset before the call -- the PCM ring on st
- * before the front end reads it, the rest on the stream of the chain before the chain reads it. */
+ * ops (null: none): streams reset or loaded before the call -- the PCM ring on st before the front end reads it, the
+ * rest on the stream of the chain before the chain reads it. */
 static int cascade_launch(nnsp_b200_cascade *c, const int16_t *pcm, long long stride, int T, int s0, int ns,
                           nnsp_b200_cascade_result *results, const nnsp_b200_taps *taps, cudaStream_t st, bool timed,
                           int slice = 0, int32_t *logmel = nullptr, cudaStream_t st_nn = nullptr, cudaEvent_t ev_feat = nullptr,
-                          cudaEvent_t ev_prev_nn = nullptr, const int32_t *nfr = nullptr, const int *rlist = nullptr, int rn = 0)
+                          cudaEvent_t ev_prev_nn = nullptr, const int32_t *nfr = nullptr, const PendingOps *ops = nullptr)
 {
     const int hist_frames = c->cd.dmax + 2;
     if (!logmel) logmel = c->logmel;
     const bool piped = st_nn != nullptr;
     int rc;
-    if (rlist && (rc = cascade_launch_reset(c, rlist, rn, 0, piped ? RESET_RING : RESET_RING | RESET_STATE, st))) return rc;
+    if (ops) {
+        if ((rc = cascade_launch_reset(c, ops->list, ops->n, 0, piped ? RESET_RING : RESET_RING | RESET_STATE, st, ops->recs))) return rc;
+        if (ops->recs) NNSP_CUDA(cudaEventRecord(ops->read_ring, st));
+    }
     FeatLaunch fl{ pcm, stride, c->st.hist, hist_frames, s0, ns, T, logmel };
     fl.nfr = nfr;
     cudaEvent_t *tl = c->tl[c->tl_count % 8];
@@ -1180,7 +1300,10 @@ static int cascade_launch(nnsp_b200_cascade *c, const int16_t *pcm, long long st
         st = st_nn;
         if (timed) NNSP_CUDA(cudaEventRecord(tl[2], st));
         /* behind the previous call's chain (stream order) and this call's front end (ev_feat), before anything reads it */
-        if (rlist && (rc = cascade_launch_reset(c, rlist, rn, 0, RESET_STATE, st))) return rc;
+        if (ops) {
+            if ((rc = cascade_launch_reset(c, ops->list, ops->n, 0, RESET_STATE, st, ops->recs))) return rc;
+            if (ops->recs) NNSP_CUDA(cudaEventRecord(ops->read_state, st));
+        }
     }
     CascadeArgs a{};
     for (int i = 0; i < 3; i++) { a.model[i] = c->dm[i].d; a.wimg[i] = c->dm[i].wimg; a.bimg[i] = c->dm[i].bimg; }
@@ -1430,9 +1553,26 @@ int nnsp_b200_cascade_create(const nnsp_b200_model *const models[3], const int *
         TRY(cudaHostAlloc(&c->rs_host[b], S * sizeof(int), cudaHostAllocDefault));
         TRY(cudaMalloc(&c->rs_dev[b], S * sizeof(int)));
         for (auto &e : c->rs_copied[b]) TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+        for (auto &e : c->rp_read[b]) TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
     }
 #undef TRY
     c->rs_mode.assign(S, (int8_t)-1);
+    c->ip_slot.assign(S, -1);
+    c->rec_bytes = rec_bytes_of(cascade_hist_words(c), cascade_lm_words(c));
+    nnsp_b200_stream_header &H = c->hdr;
+    H.magic = NNSP_B200_STREAM_MAGIC; H.version = NNSP_B200_STREAM_VERSION; H.record_bytes = (uint32_t)c->rec_bytes;
+    H.len_seq = len_seq; H.frs_vbufBk_kws = P.frs_vbufBk_kws; H.frs_vbufBk_s2i = P.frs_vbufBk_s2i;
+    for (int k = 0; k < 3; k++) {
+        H.seq[k] = k < len_seq ? seq[k] : -1;
+        if (k >= len_seq) continue;
+        size_t nb = 0;
+        if ((rc = nnsp_b200_model_to_blob(models[seq[k]], nullptr, 0, &nb))) return fail(rc);
+        std::vector<unsigned char> blob(nb);
+        if ((rc = nnsp_b200_model_to_blob(models[seq[k]], blob.data(), nb, &nb))) return fail(rc);
+        uint64_t f = 0xcbf29ce484222325ull;                              /* FNV-1a, 64 bits */
+        for (unsigned char x : blob) f = (f ^ x) * 0x100000001b3ull;
+        H.model_fnv1a[k] = f;
+    }
     if (cudaDeviceSynchronize() != cudaSuccess) return fail(NNSP_B200_ERR_CUDA);   /* uploads went through the default stream */
     if ((rc = cascade_launch_reset(c, nullptr, 0, 1, RESET_RING | RESET_STATE, c->stream))) return fail(rc);
     if (cudaStreamSynchronize(c->stream) != cudaSuccess) { nnsp_set_error("cascade reset kernel failed: %s", cudaGetErrorString(cudaGetLastError())); return fail(NNSP_B200_ERR_CUDA); }
@@ -1476,7 +1616,10 @@ int nnsp_b200_cascade_reset(nnsp_b200_cascade *c)
     c->nn_pending[0] = c->nn_pending[1] = false;
     c->host_inflight = false;
     /* resets still pending stay pending: applied at the next call, after this one, they leave what they would have left
-     * before it (a reset stream's state does not depend on the state it had) */
+     * before it (a reset stream's state does not depend on the state it had). A pending import is followed by this
+     * reset: it becomes load-then-reset. */
+    for (int s : c->rs_ids)
+        if (c->rs_mode[(size_t)s] == OP_LOAD) c->rs_mode[(size_t)s] = OP_LOAD_INSTANCE;
     const int rc = cascade_launch_reset(c, nullptr, 0, 0, RESET_RING | RESET_STATE, c->stream);
     if (rc) return rc;
     NNSP_CUDA(cudaStreamSynchronize(c->stream));
@@ -1497,8 +1640,110 @@ int nnsp_b200_cascade_reset_streams(nnsp_b200_cascade *c, const int32_t *streams
     for (int i = 0; i < n; i++) {
         int8_t &m = c->rs_mode[(size_t)streams[i]];
         if (m < 0) c->rs_ids.push_back(streams[i]);
-        if (m < mode) m = (int8_t)mode;                               /* FRESH after or before INSTANCE leaves FRESH */
+        if (m >= OP_LOAD) m = (int8_t)(mode == OP_FRESH ? OP_FRESH : OP_LOAD_INSTANCE);   /* an import, then this reset */
+        else if (m < mode) m = (int8_t)mode;                          /* FRESH after or before INSTANCE leaves FRESH */
     }
+    return NNSP_B200_OK;
+}
+
+size_t nnsp_b200_cascade_stream_state_bytes(const nnsp_b200_cascade *c) { return c ? (size_t)c->rec_bytes : 0; }
+
+/* A record that may go to the device: its header matches this handle's, and every body field a kernel uses as an
+ * index or a loop bound is in range (the readers of casc / scal in nnsp_cascade.cu and nnsp_split.cu: cd.seq[pos],
+ * the fix rows of ages 0 and 1, the frame a time-out falls on, the first inference frame, the S2I argmax). */
+int nnsp_cascade_check_records(const nnsp_b200_cascade *c, const void *records, int n)
+{
+    if (n > 0 && !records) { nnsp_set_error("stream records: null pointer"); return NNSP_B200_ERR_ARG; }
+    for (int i = 0; i < n; i++) {
+        const unsigned char *r = static_cast<const unsigned char *>(records) + (size_t)i * c->rec_bytes;
+        nnsp_b200_stream_header h;
+        memcpy(&h, r, sizeof h);
+        const char *bad = nullptr;
+        if (h.magic != NNSP_B200_STREAM_MAGIC) bad = "bad magic";
+        else if (h.version != NNSP_B200_STREAM_VERSION) bad = "unknown version";
+        else if (h.record_bytes != (uint32_t)c->rec_bytes) bad = "record size differs from this handle's";
+        else if (h.len_seq != c->hdr.len_seq || memcmp(h.seq, c->hdr.seq, sizeof h.seq)) bad = "cascade sequence differs from this handle's";
+        else if (h.frs_vbufBk_kws != c->hdr.frs_vbufBk_kws || h.frs_vbufBk_s2i != c->hdr.frs_vbufBk_s2i) bad = "look-back depths differ from this handle's";
+        else if (memcmp(h.model_fnv1a, c->hdr.model_fnv1a, sizeof h.model_fnv1a)) bad = "model fingerprints differ from this handle's";
+        if (!bad) {
+            uint16_t cs[CS_N];
+            int16_t sc[SC_N];
+            memcpy(cs, r + REC_CASC, sizeof cs);
+            memcpy(sc, r + REC_SCAL, sizeof sc);
+            if (cs[CS_POS] >= c->cd.len_seq) bad = "sequence position out of range";
+            else if (cs[CS_AGE] > 2) bad = "instance age out of range";
+            else if (cs[CS_CNT_KWS] >= 32767 || cs[CS_CNT_S2I] >= 32767) bad = "time-out counter out of range";
+            else if (sc[SC_SLIDES] != 0 && sc[SC_SLIDES] != 1) bad = "NNSPClass.slides out of range";
+            else if (sc[SC_ARGMAX_LAST] < 0 || sc[SC_ARGMAX_LAST] > 6) bad = "last S2I argmax out of range";
+        }
+        if (bad) { nnsp_set_error("stream record %d: %s", i, bad); return NNSP_B200_ERR_ARG; }
+    }
+    return NNSP_B200_OK;
+}
+
+int nnsp_b200_cascade_import_streams(nnsp_b200_cascade *c, const int32_t *streams, int n, const void *records)
+{
+    if (!c || n < 0 || (n > 0 && !streams)) { nnsp_set_error("cascade_import_streams: bad arguments (n = %d)", n); return NNSP_B200_ERR_ARG; }
+    std::vector<char> seen;
+    for (int i = 0; i < n; i++) {                                     /* checked before anything is recorded */
+        if (streams[i] < 0 || streams[i] >= c->S) {
+            nnsp_set_error("cascade_import_streams: streams[%d] = %d is outside [0, %d)", i, (int)streams[i], c->S);
+            return NNSP_B200_ERR_ARG;
+        }
+        if (seen.empty()) seen.assign((size_t)c->S, 0);
+        if (seen[(size_t)streams[i]]++) { nnsp_set_error("cascade_import_streams: stream %d listed twice", (int)streams[i]); return NNSP_B200_ERR_ARG; }
+    }
+    int rc = nnsp_cascade_check_records(c, records, n);
+    if (rc) return rc;
+    for (int i = 0; i < n; i++) {
+        const size_t s = (size_t)streams[i];
+        if (c->rs_mode[s] < 0) c->rs_ids.push_back(streams[i]);
+        c->rs_mode[s] = OP_LOAD;                                      /* whatever was pending before: the last import wins */
+        if (c->ip_slot[s] < 0) {
+            c->ip_slot[s] = (int)(c->ip_pool.size() / (size_t)c->rec_bytes);
+            c->ip_pool.resize(c->ip_pool.size() + (size_t)c->rec_bytes);
+        }
+        memcpy(c->ip_pool.data() + (size_t)c->ip_slot[s] * c->rec_bytes, static_cast<const unsigned char *>(records) + (size_t)i * c->rec_bytes,
+               (size_t)c->rec_bytes);
+    }
+    return NNSP_B200_OK;
+}
+
+int nnsp_b200_cascade_export_streams(nnsp_b200_cascade *c, const int32_t *streams, int n, void *records)
+{
+    if (!c || n < 0 || (n > 0 && (!streams || !records))) { nnsp_set_error("cascade_export_streams: bad arguments (n = %d)", n); return NNSP_B200_ERR_ARG; }
+    for (int i = 0; i < n; i++)
+        if (streams[i] < 0 || streams[i] >= c->S) {
+            nnsp_set_error("cascade_export_streams: streams[%d] = %d is outside [0, %d)", i, (int)streams[i], c->S);
+            return NNSP_B200_ERR_ARG;
+        }
+    if (n == 0) return NNSP_B200_OK;
+    int rc = nnsp_b200_cascade_sync(c);                               /* every call issued, host tickets included */
+    if (rc) return rc;
+    /* the device is idle: the pending resets and imports, both parts at once, on c->stream */
+    const int *rl = nullptr;
+    int rn = 0, rb = 0, loads = 0;
+    if ((rc = cascade_take_resets(c, &rl, &rn, &rb, &loads))) return rc;
+    if (rn) {
+        NNSP_CUDA(cudaMemcpyAsync(c->rs_dev[0], rl, (size_t)rn * sizeof(int), cudaMemcpyHostToDevice, c->stream));
+        NNSP_CUDA(cudaEventRecord(c->rs_copied[rb][0], c->stream));
+        c->rs_copy_valid[rb][0] = true;
+        if (loads) NNSP_CUDA(cudaMemcpyAsync(c->rp_dev[rb], c->rp_host[rb], (size_t)loads * c->rec_bytes, cudaMemcpyHostToDevice, c->stream));
+        if ((rc = cascade_launch_reset(c, c->rs_dev[0], rn, 0, RESET_RING | RESET_STATE, c->stream, loads ? c->rp_dev[rb] : nullptr))) return rc;
+        if (loads) { NNSP_CUDA(cudaEventRecord(c->rp_read[rb][0], c->stream)); c->rp_read_valid[rb][0] = true; }
+    }
+    if (n > c->ex_cap) {
+        cudaFree(c->ex_ids); cudaFree(c->ex_dev);
+        c->ex_ids = nullptr; c->ex_dev = nullptr; c->ex_cap = 0;
+        NNSP_CUDA(cudaMalloc(&c->ex_ids, (size_t)n * sizeof(int)));
+        NNSP_CUDA(cudaMalloc(&c->ex_dev, (size_t)n * c->rec_bytes));
+        c->ex_cap = n;
+    }
+    NNSP_CUDA(cudaMemcpyAsync(c->ex_ids, streams, (size_t)n * sizeof(int), cudaMemcpyHostToDevice, c->stream));
+    cascade_export_kernel<<<n, 128, 0, c->stream>>>(c->st, c->stale, c->ex_ids, c->ex_dev, cascade_hist_words(c), cascade_lm_words(c), c->hdr);
+    NNSP_LAUNCH_CHECK();
+    NNSP_CUDA(cudaMemcpyAsync(records, c->ex_dev, (size_t)n * c->rec_bytes, cudaMemcpyDeviceToHost, c->stream));
+    NNSP_CUDA(cudaStreamSynchronize(c->stream));
     return NNSP_B200_OK;
 }
 
@@ -1526,23 +1771,30 @@ static int cascade_exec_dev(nnsp_b200_cascade *c, const int16_t *pcm_dev, long l
     }
     if ((rc = cascade_ensure_logmel(c, n_frames))) return rc;
     if ((rc = cascade_ensure_split(c, n_frames))) return rc;
-    const int *rl = nullptr;                            /* pending resets: uploaded on c->stream behind the waits below */
-    int rn = 0, rb = 0;
-    auto upload_resets = [&](int *dst) -> int {
+    const int *rl = nullptr;                            /* pending resets and imports: uploaded on c->stream behind the waits below */
+    int rn = 0, rb = 0, loads = 0;
+    PendingOps ops{};
+    auto upload_resets = [&](int *dst, bool piped) -> int {
         NNSP_CUDA(cudaMemcpyAsync(dst, rl, (size_t)rn * sizeof(int), cudaMemcpyHostToDevice, c->stream));
         NNSP_CUDA(cudaEventRecord(c->rs_copied[rb][0], c->stream));
         c->rs_copy_valid[rb][0] = true;
-        rl = dst;
+        ops.list = dst; ops.n = rn;
+        if (loads) {
+            NNSP_CUDA(cudaMemcpyAsync(c->rp_dev[rb], c->rp_host[rb], (size_t)loads * c->rec_bytes, cudaMemcpyHostToDevice, c->stream));
+            ops.recs = c->rp_dev[rb];
+            ops.read_ring = c->rp_read[rb][0]; c->rp_read_valid[rb][0] = true;
+            if (piped) { ops.read_state = c->rp_read[rb][3]; c->rp_read_valid[rb][3] = true; }
+        }
         return NNSP_B200_OK;
     };
-    if ((rc = cascade_take_resets(c, &rl, &rn, &rb))) return rc;
+    if ((rc = cascade_take_resets(c, &rl, &rn, &rb, &loads))) return rc;
     if (cascade_use_split(c, taps)) {
         const int i = (int)(c->pipe++ & 1u);
         if (c->nn_pending[i]) NNSP_CUDA(cudaStreamWaitEvent(c->stream, c->ev_nn[i], 0));   /* log-mel buffer i / PCM history in use two calls ago */
-        if (rn && (rc = upload_resets(c->rs_dev[i]))) return rc;      /* rs_dev[i] too: its last readers ran in that chain */
+        if (rn && (rc = upload_resets(c->rs_dev[i], true))) return rc;    /* rs_dev[i] too: its last readers ran in that chain */
         rc = cascade_launch(c, pcm_dev, stream_stride, n_frames, 0, c->S, results_dev, nullptr, c->stream, true, 0,
                             i ? c->logmel2 : c->logmel, c->nn_stream, c->ev_feat[i], c->nn_pending[i ^ 1] ? c->ev_nn[i ^ 1] : nullptr, nfr,
-                            rn ? rl : nullptr, rn);
+                            rn ? &ops : nullptr);
         if (rc) return rc;
         NNSP_CUDA(cudaEventRecord(c->ev_nn[i], c->nn_stream));
         c->nn_pending[i] = true;
@@ -1550,9 +1802,9 @@ static int cascade_exec_dev(nnsp_b200_cascade *c, const int16_t *pcm_dev, long l
         return NNSP_B200_OK;
     }
     if ((rc = cascade_join_nn(c, c->stream))) return rc;
-    if (rn && (rc = upload_resets(c->rs_dev[0]))) return rc;
+    if (rn && (rc = upload_resets(c->rs_dev[0], false))) return rc;
     return cascade_launch(c, pcm_dev, stream_stride, n_frames, 0, c->S, results_dev, taps, c->stream, true, 0, nullptr, nullptr,
-                          nullptr, nullptr, nfr, rn ? rl : nullptr, rn);
+                          nullptr, nullptr, nfr, rn ? &ops : nullptr);
 }
 
 int nnsp_b200_cascade_exec(nnsp_b200_cascade *c, const int16_t *pcm_dev, long long stream_stride, int n_frames,
@@ -1613,9 +1865,9 @@ static int cascade_enqueue_host(nnsp_b200_cascade *c, const int16_t *pcm, long l
         NNSP_CUDA(cudaDeviceSynchronize());
         NNSP_CUDA(cudaMalloc(&c->d_nfr, (size_t)2 * c->S * sizeof(int32_t)));
     }
-    const int *rl = nullptr;                                          /* pending resets, sorted by stream */
-    int rn = 0, rb = 0;
-    if ((rc = cascade_take_resets(c, &rl, &rn, &rb))) return rc;
+    const int *rl = nullptr;                                          /* pending resets and imports, sorted by stream */
+    int rn = 0, rb = 0, loads = 0;
+    if ((rc = cascade_take_resets(c, &rl, &rn, &rb, &loads))) return rc;
     c->host_inflight = true;
     const int nsl = c->S >= 4096 ? 8 : (c->S >= 256 ? 4 : 1);
     const int buf = (int)(c->host_calls++ & 1);
@@ -1657,16 +1909,27 @@ static int cascade_enqueue_host(nnsp_b200_cascade *c, const int16_t *pcm, long l
                 NNSP_CUDA(cudaMemcpyAsync(dnfr + s0, nfr + s0, (size_t)(s1 - s0) * sizeof(int32_t), cudaMemcpyHostToDevice, st));
         } else
             NNSP_CUDA(cudaStreamWaitEvent(st, c->ev_h2d[buf][k], 0));
-        /* the slice's own resets, at rs_dev[0] + s0: only this slice's kernels, all on st, ever use those entries */
-        const int r0 = rn ? (int)(std::lower_bound(rl, rl + rn, s0 << 1) - rl) : 0;
-        const int r1 = rn ? (int)(std::lower_bound(rl, rl + rn, s1 << 1) - rl) : 0;
+        /* the slice's own resets, at rs_dev[0] + s0: only this slice's kernels, all on st, ever use those entries; its
+         * records, p0 .. p1 - 1 of the call's, at the same place in rp_dev[rb] */
+        const int *taken = c->rs_taken.data();
+        const int r0 = rn ? (int)(std::lower_bound(taken, taken + rn, s0) - taken) : 0;
+        const int r1 = rn ? (int)(std::lower_bound(taken, taken + rn, s1) - taken) : 0;
+        PendingOps ops{ c->rs_dev[0] + s0, r1 - r0, nullptr, nullptr, nullptr };
         if (r1 > r0) {
             NNSP_CUDA(cudaMemcpyAsync(c->rs_dev[0] + s0, rl + r0, (size_t)(r1 - r0) * sizeof(int), cudaMemcpyHostToDevice, st));
             NNSP_CUDA(cudaEventRecord(c->rs_copied[rb][k % 3], st));   /* re-recorded by later slices on st: the last copy */
             c->rs_copy_valid[rb][k % 3] = true;
+            const int p0 = c->rs_taken_loads[(size_t)r0], p1 = c->rs_taken_loads[(size_t)r1];
+            if (p1 > p0) {
+                NNSP_CUDA(cudaMemcpyAsync(c->rp_dev[rb] + (size_t)p0 * c->rec_bytes, c->rp_host[rb] + (size_t)p0 * c->rec_bytes,
+                                          (size_t)(p1 - p0) * c->rec_bytes, cudaMemcpyHostToDevice, st));
+                ops.recs = c->rp_dev[rb];
+                ops.read_ring = c->rp_read[rb][k % 3];
+                c->rp_read_valid[rb][k % 3] = true;
+            }
         }
         rc = cascade_launch(c, dpcm, dstride, T, s0, s1 - s0, results ? c->d_res : nullptr, nullptr, st, false, k,
-                            nullptr, nullptr, nullptr, nullptr, dnfr, r1 > r0 ? c->rs_dev[0] + s0 : nullptr, r1 - r0);
+                            nullptr, nullptr, nullptr, nullptr, dnfr, r1 > r0 ? &ops : nullptr);
         if (rc) return rc;
         NNSP_CUDA(cudaEventRecord(c->ev_read[buf][k], st));         /* every reader of the slice's PCM has joined st by now */
         c->read_valid[buf][k] = true;
@@ -1820,7 +2083,11 @@ void nnsp_b200_cascade_destroy(nnsp_b200_cascade *c)
         if (c->rs_host[b]) cudaFreeHost(c->rs_host[b]);
         cudaFree(c->rs_dev[b]);
         for (auto e : c->rs_copied[b]) if (e) cudaEventDestroy(e);
+        if (c->rp_host[b]) cudaFreeHost(c->rp_host[b]);
+        cudaFree(c->rp_dev[b]);
+        for (auto e : c->rp_read[b]) if (e) cudaEventDestroy(e);
     }
+    cudaFree(c->ex_ids); cudaFree(c->ex_dev);
     delete c;
 }
 

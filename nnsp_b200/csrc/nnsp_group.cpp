@@ -10,10 +10,12 @@
  * Host code only (C++ threads over the library's own C ABI): no CUDA call is made here, and no collective exists. */
 #include <condition_variable>
 #include <cstdio>
+#include <cstring>
 #include <deque>
 #include <mutex>
 #include <new>
 #include <thread>
+#include <utility>
 #include <vector>
 
 #include "nnsp_b200.h"
@@ -22,13 +24,15 @@
 namespace {
 
 struct Command {
-    enum Kind { EXEC, RESET, QUIT, RESET_STREAMS } kind;
+    enum Kind { EXEC, RESET, QUIT, RESET_STREAMS, IMPORT_STREAMS, EXPORT_STREAMS } kind;
     const int16_t *pcm;
     long long stride;
     int n_frames;                    /* RESET_STREAMS: the mode */
-    void *results;
-    long long seq;                   /* RESET_STREAMS: complete once recorded and the call before it is complete */
-    std::vector<int32_t> streams;    /* RESET_STREAMS: the member's own streams, in its numbering */
+    void *results;                   /* EXPORT_STREAMS: the caller's records */
+    long long seq;                   /* RESET_ / IMPORT_STREAMS: complete once recorded and the call before it is complete */
+    std::vector<int32_t> streams;    /* *_STREAMS: the member's own streams, in its numbering */
+    std::vector<int32_t> where;      /* EXPORT_STREAMS: the record of streams[i] is record where[i] of the caller's */
+    std::vector<unsigned char> records;   /* IMPORT_STREAMS: the records of streams, a copy */
 };
 
 struct Member {
@@ -106,14 +110,33 @@ void worker(Member *m)
                 lk.lock();
             }
             m->cv_cmd.wait(lk, [&] { return !m->queue.empty(); });
-            c = m->queue.front();
+            c = std::move(m->queue.front());
             m->queue.pop_front();
         }
         if (c.kind == Command::QUIT) { finish_inflight(); return; }
-        if (c.kind == Command::RESET_STREAMS) {                 /* recorded on the handle, applied by its next call */
-            const int rc = nnsp_b200_cascade_reset_streams(m->cascade, c.streams.data(), (int)c.streams.size(), c.n_frames);
+        if (c.kind == Command::RESET_STREAMS || c.kind == Command::IMPORT_STREAMS) {   /* recorded on the handle, applied by its next call */
+            const int rc = c.kind == Command::RESET_STREAMS
+                               ? nnsp_b200_cascade_reset_streams(m->cascade, c.streams.data(), (int)c.streams.size(), c.n_frames)
+                               : nnsp_b200_cascade_import_streams(m->cascade, c.streams.data(), (int)c.streams.size(), c.records.data());
             if (rc) fail(rc);
             if (inflight_seq) { passed_seq = c.seq; continue; }
+            { std::lock_guard<std::mutex> lk(m->mu); m->done_seq = c.seq; }
+            m->cv_done.notify_all();
+            continue;
+        }
+        if (c.kind == Command::EXPORT_STREAMS) {                /* synchronous: the member's device is idle afterwards */
+            finish_inflight();
+            const size_t rb = nnsp_b200_cascade_stream_state_bytes(m->cascade), n = c.streams.size();
+            unsigned char *out = static_cast<unsigned char *>(c.results);
+            int rc = NNSP_B200_OK;
+            if (n && c.where[n - 1] - c.where[0] + 1 == (int32_t)n)   /* the member's records are one range of the caller's */
+                rc = nnsp_b200_cascade_export_streams(m->cascade, c.streams.data(), (int)n, out + rb * (size_t)c.where[0]);
+            else if (n) {
+                std::vector<unsigned char> tmp(rb * n);
+                rc = nnsp_b200_cascade_export_streams(m->cascade, c.streams.data(), (int)n, tmp.data());
+                for (size_t i = 0; !rc && i < n; i++) memcpy(out + rb * (size_t)c.where[i], tmp.data() + rb * i, rb);
+            }
+            if (rc) fail(rc);
             { std::lock_guard<std::mutex> lk(m->mu); m->done_seq = c.seq; }
             m->cv_done.notify_all();
             continue;
@@ -218,7 +241,7 @@ int nnsp_b200_group_exec_host_async(nnsp_b200_group *g, const int16_t *pcm, long
                                     void *results, long long *ticket)
 {
     if (!g || !pcm || n_frames <= 0) return NNSP_B200_ERR_ARG;
-    Command c{ Command::EXEC, pcm, stream_stride, n_frames, results, 0, {} };
+    Command c{ Command::EXEC, pcm, stream_stride, n_frames, results, 0, {}, {}, {} };
     return post(g, c, ticket);
 }
 
@@ -245,7 +268,7 @@ int nnsp_b200_group_reset(nnsp_b200_group *g)
 {
     if (!g) return NNSP_B200_ERR_ARG;
     long long t = 0;
-    Command c{ Command::RESET, nullptr, 0, 0, nullptr, 0, {} };
+    Command c{ Command::RESET, nullptr, 0, 0, nullptr, 0, {}, {}, {} };
     post(g, c, &t);
     return nnsp_b200_group_wait(g, t);
 }
@@ -284,9 +307,69 @@ int nnsp_b200_group_reset_streams(nnsp_b200_group *g, const int32_t *streams, in
      * group's latest command (nnsp_b200_group_set_stream_params, group_wait) also waits until it is recorded */
     const long long seq = ++g->seq;
     for (Member *m : g->members) {
-        Command c{ Command::RESET_STREAMS, nullptr, 0, mode, nullptr, seq, {} };
+        Command c{ Command::RESET_STREAMS, nullptr, 0, mode, nullptr, seq, {}, {}, {} };
         for (int i = 0; i < n; i++)
             if (streams[i] >= m->first && streams[i] < m->first + m->count) c.streams.push_back(streams[i] - m->first);
+        { std::lock_guard<std::mutex> lk(m->mu); m->queue.push_back(std::move(c)); }
+        m->cv_cmd.notify_one();
+    }
+    return NNSP_B200_OK;
+}
+
+size_t nnsp_b200_group_stream_state_bytes(const nnsp_b200_group *g)
+{
+    return (g && g->is_cascade) ? nnsp_b200_cascade_stream_state_bytes(g->members[0]->cascade) : 0;
+}
+
+/* the checks of nnsp_b200_cascade_export_streams / _import_streams over the group's numbering (cascade groups) */
+static int group_check_ids(const nnsp_b200_group *g, const int32_t *streams, int n, bool unique, const char *fn)
+{
+    if (!g || !g->is_cascade || n < 0 || (n > 0 && !streams)) {
+        nnsp_set_error("%s: a cascade group and n >= 0 are required", fn);
+        return NNSP_B200_ERR_ARG;
+    }
+    std::vector<char> seen(unique ? (size_t)g->n_streams : 0);
+    for (int i = 0; i < n; i++) {
+        if (streams[i] < 0 || streams[i] >= g->n_streams) {
+            nnsp_set_error("%s: streams[%d] = %d is outside [0, %d)", fn, i, (int)streams[i], g->n_streams);
+            return NNSP_B200_ERR_ARG;
+        }
+        if (unique && seen[(size_t)streams[i]]++) { nnsp_set_error("%s: stream %d listed twice", fn, (int)streams[i]); return NNSP_B200_ERR_ARG; }
+    }
+    return NNSP_B200_OK;
+}
+
+int nnsp_b200_group_export_streams(nnsp_b200_group *g, const int32_t *streams, int n, void *records)
+{
+    int rc = group_check_ids(g, streams, n, false, "group_export_streams");
+    if (rc) return rc;
+    if (n > 0 && !records) { nnsp_set_error("group_export_streams: null records"); return NNSP_B200_ERR_ARG; }
+    const long long seq = ++g->seq;
+    for (Member *m : g->members) {
+        Command c{ Command::EXPORT_STREAMS, nullptr, 0, 0, records, seq, {}, {}, {} };
+        for (int i = 0; i < n; i++)
+            if (streams[i] >= m->first && streams[i] < m->first + m->count) { c.streams.push_back(streams[i] - m->first); c.where.push_back(i); }
+        { std::lock_guard<std::mutex> lk(m->mu); m->queue.push_back(std::move(c)); }
+        m->cv_cmd.notify_one();
+    }
+    return nnsp_b200_group_wait(g, seq);
+}
+
+int nnsp_b200_group_import_streams(nnsp_b200_group *g, const int32_t *streams, int n, const void *records)
+{
+    int rc = group_check_ids(g, streams, n, true, "group_import_streams");
+    if (rc) return rc;
+    if ((rc = nnsp_cascade_check_records(g->members[0]->cascade, records, n))) return rc;   /* every member takes the same records */
+    const size_t rb = nnsp_b200_cascade_stream_state_bytes(g->members[0]->cascade);
+    const unsigned char *in = static_cast<const unsigned char *>(records);
+    const long long seq = ++g->seq;                                   /* in order with the calls, like RESET_STREAMS */
+    for (Member *m : g->members) {
+        Command c{ Command::IMPORT_STREAMS, nullptr, 0, 0, nullptr, seq, {}, {}, {} };
+        for (int i = 0; i < n; i++)
+            if (streams[i] >= m->first && streams[i] < m->first + m->count) {
+                c.streams.push_back(streams[i] - m->first);
+                c.records.insert(c.records.end(), in + rb * (size_t)i, in + rb * (size_t)(i + 1));
+            }
         { std::lock_guard<std::mutex> lk(m->mu); m->queue.push_back(std::move(c)); }
         m->cv_cmd.notify_one();
     }
@@ -298,7 +381,7 @@ void nnsp_b200_group_destroy(nnsp_b200_group *g)
     if (!g) return;
     for (Member *m : g->members) {
         if (m->thread.joinable()) {
-            { std::lock_guard<std::mutex> lk(m->mu); m->queue.push_back(Command{ Command::QUIT, nullptr, 0, 0, nullptr, 0, {} }); }
+            { std::lock_guard<std::mutex> lk(m->mu); m->queue.push_back(Command{ Command::QUIT, nullptr, 0, 0, nullptr, 0, {}, {}, {} }); }
             m->cv_cmd.notify_one();
             m->thread.join();
         }

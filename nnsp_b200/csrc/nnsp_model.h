@@ -50,6 +50,9 @@ size_t nnsp_interleave_arm(const int8_t *src_rowmajor, int rows, int cols, int8_
 
 void nnsp_set_error(const char *fmt, ...);
 
+/* nnsp_cascade.cu: NNSP_B200_ERR_ARG unless all n records may be imported into handle c (nnsp_b200_cascade_import_streams) */
+int nnsp_cascade_check_records(const nnsp_b200_cascade *c, const void *records, int n);
+
 #ifdef __cplusplus
 }
 #endif
