@@ -736,6 +736,9 @@ struct CascadePostArgs {
     nnsp_b200_cascade_result *results;
     CascadeDev cd;
     const int32_t *nfr;              /* ragged call: stream s ends at frame stream_frames(nfr, s, T) */
+    int32_t *lm_next;                /* pipelined call shorter than the log-mel history, or ragged (else null): the next
+                                        call's history, whose newest rows feat_kernel wrote; cascade_ctx_kernel adds the
+                                        rows of st.lmhist that stay */
 };
 
 /* log-mel row the instance of stream s reads at frame f of the call (f >= its tb): a fix row during its first two frames */
@@ -913,13 +916,20 @@ __global__ void __launch_bounds__(32 * CPOST_WARPS) cascade_post_kernel(CascadeP
 
 /* context of the instances that lived through the call (t0 == T + 1): the newest six standardised rows of (the rows the
  * instance had when its life in this call began ++ the rows of its frames tb .. Ts-1, read with its look-back); a warp
- * per stream */
+ * per stream. With lm_next, first the rows of the log-mel history that stay in the next one: next rows
+ * [0, dmax - Ts) <- st.lmhist rows [Ts, dmax). This runs after the call's resets and imports (head of the chain). */
 __global__ void __launch_bounds__(256) cascade_ctx_kernel(CascadePostArgs a)
 {
     const int si = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
     if (si >= a.ns) return;
     const long long s = a.s0 + si;
     const int T = a.T;
+    if (a.lm_next) {
+        const int words = a.cd.dmax * NNSP_B200_NMEL, Ts = stream_frames(a.nfr, s, T);
+        const int32_t *hi = a.st.lmhist + s * words + Ts * NNSP_B200_NMEL;
+        int32_t *ho = a.lm_next + s * words;
+        for (int i = lane; i < words - Ts * NNSP_B200_NMEL; i += 32) ho[i] = hi[i];
+    }
     if (a.ra.t0[s] != T + 1) return;
     const CascadeDev &cd = a.cd;
     const int id = cd.seq[a.st.casc[s * CS_N + CS_POS]];
@@ -1088,14 +1098,17 @@ struct nnsp_b200_cascade {
     int32_t *dec = nullptr;
     long long split_cap_T = 0;
     cudaStream_t gs[4][3] = {};                /* per pipeline stream (3 host-call streams + the device-call stream): one per model group */
-    /* device-buffer calls are pipelined like the batched path: front end + PCM history roll of call N+1 on `stream`,
-     * controller / network work of call N on `nn_stream`; log-mel rows and PCM history are double buffered */
+    /* device-buffer calls are pipelined like the batched path: front end of call N+1 on `stream`, controller / network
+     * work of call N on `nn_stream`; log-mel rows are double buffered. The PCM and log-mel histories are triple
+     * buffered: call N+1's front end writes the next histories into the buffers that call N-1's chain read, which it
+     * waits for anyway (for its log-mel rows), while call N's chain may still read the ones call N read. */
     cudaStream_t nn_stream = nullptr;
     cudaEvent_t ev_feat[2] = { nullptr, nullptr }, ev_nn[2] = { nullptr, nullptr };
     bool nn_pending[2] = { false, false }, last_piped = false;
     unsigned pipe = 0;
     int32_t *logmel2 = nullptr;                /* second log-mel buffer */
-    int16_t *hist2 = nullptr;                  /* second PCM history buffer */
+    int16_t *hist2 = nullptr, *hist3 = nullptr;   /* the next PCM history (written by the pipelined call), the spare */
+    int32_t *lmhist2 = nullptr, *lmhist3 = nullptr;   /* the same for the log-mel history */
     cudaEvent_t ev_fork[4] = {}, ev_join[4][3] = {};
     /* asynchronous host-buffer calls: one completion event per pipeline stream, a ring of CS_HOST_RING calls */
     cudaEvent_t host_ev[CS_HOST_RING][3] = {};
@@ -1267,14 +1280,14 @@ struct PendingOps {
     cudaEvent_t read_ring, read_state;
 };
 
-/* st_nn (with ev_feat): pipelined call -- everything behind the front end goes to st_nn, the PCM history is rolled out
- * of place on st right behind the front end (c->st.hist is swapped by the caller afterwards).
+/* st_nn (with ev_feat): pipelined call -- everything behind the front end goes to st_nn; the front end writes the next
+ * PCM and log-mel histories out of place into c->hist2 / c->lmhist2 (the caller rotates the buffers afterwards).
  * ops (null: none): streams reset or loaded before the call -- the PCM ring on st before the front end reads it, the
  * rest on the stream of the chain before the chain reads it. */
 static int cascade_launch(nnsp_b200_cascade *c, const int16_t *pcm, long long stride, int T, int s0, int ns,
                           nnsp_b200_cascade_result *results, const nnsp_b200_taps *taps, cudaStream_t st, bool timed,
                           int slice = 0, int32_t *logmel = nullptr, cudaStream_t st_nn = nullptr, cudaEvent_t ev_feat = nullptr,
-                          cudaEvent_t ev_prev_nn = nullptr, const int32_t *nfr = nullptr, const PendingOps *ops = nullptr)
+                          const int32_t *nfr = nullptr, const PendingOps *ops = nullptr)
 {
     const int hist_frames = c->cd.dmax + 2;
     if (!logmel) logmel = c->logmel;
@@ -1286,6 +1299,10 @@ static int cascade_launch(nnsp_b200_cascade *c, const int16_t *pcm, long long st
     }
     FeatLaunch fl{ pcm, stride, c->st.hist, hist_frames, s0, ns, T, logmel };
     fl.nfr = nfr;
+    if (piped) {
+        fl.hist_out = c->hist2;
+        if (c->cd.dmax > 0) { fl.lm_out = c->lmhist2; fl.lm_rows = c->cd.dmax; }
+    }
     cudaEvent_t *tl = c->tl[c->tl_count % 8];
     if (timed) NNSP_CUDA(cudaEventRecord(tl[0], st));
     rc = launch_feature(c->tables, fl, c->device, st);
@@ -1294,9 +1311,6 @@ static int cascade_launch(nnsp_b200_cascade *c, const int16_t *pcm, long long st
     if (piped) {
         NNSP_CUDA(cudaEventRecord(ev_feat, st));
         NNSP_CUDA(cudaStreamWaitEvent(st_nn, ev_feat, 0));
-        /* the spare history buffer is the one the previous call's replay may still read: roll into it only then */
-        if (ev_prev_nn) NNSP_CUDA(cudaStreamWaitEvent(st, ev_prev_nn, 0));
-        if ((rc = launch_hist_roll(pcm, stride / 2, c->st.hist, c->hist2, hist_frames, NNSP_B200_FRAME / 2, s0, ns, T, st, nfr))) return rc;
         st = st_nn;
         if (timed) NNSP_CUDA(cudaEventRecord(tl[2], st));
         /* behind the previous call's chain (stream order) and this call's front end (ev_feat), before anything reads it */
@@ -1326,6 +1340,7 @@ static int cascade_launch(nnsp_b200_cascade *c, const int16_t *pcm, long long st
         for (int i = 0; i < 3; i++) p.model[i] = c->mm[i].d;
         p.st = c->st; p.stale = c->stale; p.logmel = logmel; p.dec = c->dec; p.dec_stride = n_inf_max; p.ra = c->ra;
         p.s0 = s0; p.ns = ns; p.T = T; p.results = results; p.cd = c->cd; p.nfr = nfr;
+        if (piped && c->cd.dmax > 0 && (nfr || T < c->cd.dmax)) p.lm_next = c->lmhist2;
         for (int r = 0; r < c->rounds; r++) {
             int *ctl_r = ctl + CTL_ROUND * r, *ctl_prev = ctl + CTL_ROUND * (r - 1);
             const int *queued = r ? c->pend[r & 1] + s0 : nullptr;        /* streams the previous round's walk queued */
@@ -1405,7 +1420,7 @@ static int cascade_launch(nnsp_b200_cascade *c, const int16_t *pcm, long long st
         c->ev_valid = true; c->last_piped = piped; c->tl_count++;
     }
     if (!piped && (rc = launch_hist_update(pcm, stride / 2, c->st.hist, hist_frames, NNSP_B200_FRAME / 2, s0, ns, T, st, nfr))) return rc;
-    if (c->cd.dmax > 0)
+    if (!piped && c->cd.dmax > 0)
         rc = launch_hist_update(logmel, (long long)T * NNSP_B200_NMEL, c->st.lmhist, c->cd.dmax, NNSP_B200_NMEL, s0, ns, T, st, nfr);
     return rc;
 }
@@ -1530,7 +1545,10 @@ int nnsp_b200_cascade_create(const nnsp_b200_model *const models[3], const int *
     TRY(cudaMalloc(&c->st.casc, S * CS_N * sizeof(uint16_t)));
     TRY(cudaMalloc(&c->st.hist, S * hist_frames * NNSP_B200_FRAME * sizeof(int16_t)));
     TRY(cudaMalloc(&c->hist2, S * hist_frames * NNSP_B200_FRAME * sizeof(int16_t)));
+    TRY(cudaMalloc(&c->hist3, S * hist_frames * NNSP_B200_FRAME * sizeof(int16_t)));
     TRY(cudaMalloc(&c->st.lmhist, S * lm_rows * NNSP_B200_NMEL * sizeof(int32_t)));
+    TRY(cudaMalloc(&c->lmhist2, S * lm_rows * NNSP_B200_NMEL * sizeof(int32_t)));
+    TRY(cudaMalloc(&c->lmhist3, S * lm_rows * NNSP_B200_NMEL * sizeof(int32_t)));
     TRY(cudaMalloc(&c->stale, S * 120 * sizeof(int16_t)));
     TRY(cudaMalloc(&c->thr, S * sizeof(CascThr)));
     c->cd.thr = c->thr;
@@ -1793,18 +1811,20 @@ static int cascade_exec_dev(nnsp_b200_cascade *c, const int16_t *pcm_dev, long l
         if (c->nn_pending[i]) NNSP_CUDA(cudaStreamWaitEvent(c->stream, c->ev_nn[i], 0));   /* log-mel buffer i / PCM history in use two calls ago */
         if (rn && (rc = upload_resets(c->rs_dev[i], true))) return rc;    /* rs_dev[i] too: its last readers ran in that chain */
         rc = cascade_launch(c, pcm_dev, stream_stride, n_frames, 0, c->S, results_dev, nullptr, c->stream, true, 0,
-                            i ? c->logmel2 : c->logmel, c->nn_stream, c->ev_feat[i], c->nn_pending[i ^ 1] ? c->ev_nn[i ^ 1] : nullptr, nfr,
-                            rn ? &ops : nullptr);
+                            i ? c->logmel2 : c->logmel, c->nn_stream, c->ev_feat[i], nfr, rn ? &ops : nullptr);
         if (rc) return rc;
         NNSP_CUDA(cudaEventRecord(c->ev_nn[i], c->nn_stream));
         c->nn_pending[i] = true;
-        int16_t *t = c->st.hist; c->st.hist = c->hist2; c->hist2 = t;      /* the rolled history is the live one from here on */
+        int16_t *t = c->st.hist; c->st.hist = c->hist2; c->hist2 = c->hist3; c->hist3 = t;   /* the written histories are the live ones from here on */
+        if (c->cd.dmax > 0) {                  /* without a look-back the one-row log-mel history is never written */
+            int32_t *u = c->st.lmhist; c->st.lmhist = c->lmhist2; c->lmhist2 = c->lmhist3; c->lmhist3 = u;
+        }
         return NNSP_B200_OK;
     }
     if ((rc = cascade_join_nn(c, c->stream))) return rc;
     if (rn && (rc = upload_resets(c->rs_dev[0], false))) return rc;
     return cascade_launch(c, pcm_dev, stream_stride, n_frames, 0, c->S, results_dev, taps, c->stream, true, 0, nullptr, nullptr,
-                          nullptr, nullptr, nfr, rn ? &ops : nullptr);
+                          nullptr, nfr, rn ? &ops : nullptr);
 }
 
 int nnsp_b200_cascade_exec(nnsp_b200_cascade *c, const int16_t *pcm_dev, long long stream_stride, int n_frames,
@@ -1929,7 +1949,7 @@ static int cascade_enqueue_host(nnsp_b200_cascade *c, const int16_t *pcm, long l
             }
         }
         rc = cascade_launch(c, dpcm, dstride, T, s0, s1 - s0, results ? c->d_res : nullptr, nullptr, st, false, k,
-                            nullptr, nullptr, nullptr, nullptr, dnfr, r1 > r0 ? &ops : nullptr);
+                            nullptr, nullptr, nullptr, dnfr, r1 > r0 ? &ops : nullptr);
         if (rc) return rc;
         NNSP_CUDA(cudaEventRecord(c->ev_read[buf][k], st));         /* every reader of the slice's PCM has joined st by now */
         c->read_valid[buf][k] = true;
@@ -2061,7 +2081,7 @@ void nnsp_b200_cascade_destroy(nnsp_b200_cascade *c)
     for (int i = 0; i < 3; i++) if (c->have[i]) free_model(&c->dm[i]);
     cudaFree(c->st.ctx); cudaFree(c->st.h); cudaFree(c->st.c); cudaFree(c->st.scal); cudaFree(c->st.casc);
     cudaFree(c->st.hist); cudaFree(c->st.lmhist); cudaFree(c->stale); cudaFree(c->thr); cudaFree(c->vseq);
-    cudaFree(c->logmel); cudaFree(c->logmel2); cudaFree(c->hist2); cudaFree(c->d_pcm); cudaFree(c->d_res); cudaFree(c->d_raw); cudaFree(c->d_nfr);
+    cudaFree(c->logmel); cudaFree(c->logmel2); cudaFree(c->hist2); cudaFree(c->hist3); cudaFree(c->lmhist2); cudaFree(c->lmhist3); cudaFree(c->d_pcm); cudaFree(c->d_res); cudaFree(c->d_raw); cudaFree(c->d_nfr);
     if (c->nn_stream) cudaStreamDestroy(c->nn_stream);
     for (auto e : c->ev_feat) if (e) cudaEventDestroy(e);
     for (auto e : c->ev_nn) if (e) cudaEventDestroy(e);

@@ -267,7 +267,7 @@ __global__ void __launch_bounds__(FEAT_THREADS, FEAT_CTAS_PER_SM)
 feat_kernel(const DevTables *__restrict__ tables, const int16_t *__restrict__ pcm, long long stride,
             const int16_t *__restrict__ hist, int hist_frames, int s0, int ns, int T,
             int32_t *__restrict__ logmel, const int32_t *__restrict__ norm, int16_t *__restrict__ feat16,
-            const int32_t *__restrict__ nfr)
+            const int32_t *__restrict__ nfr, int16_t *__restrict__ hist_out, int32_t *__restrict__ lm_out, int lm_rows)
 {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     FeatSmem &sm = *reinterpret_cast<FeatSmem *>(smem_raw);
@@ -284,8 +284,9 @@ feat_kernel(const DevTables *__restrict__ tables, const int16_t *__restrict__ pc
         bool valid = f < F;
         const long long fc = valid ? f : 0;
         const int s = s0 + (int)(fc / T), t = (int)(fc % T);
+        const int Ts = RAGGED ? stream_frames(nfr, s, T) : T;               /* frames of stream s in this call */
         if (RAGGED) {
-            valid = valid && t < stream_frames(nfr, s, T);
+            valid = valid && t < Ts;
             if (!__any_sync(0xffffffffu, valid)) continue;              /* warp-uniform: neither frame is live */
         }
         /* the 480-sample window starts two frames back: word L + 16a of it comes from this call's PCM or, for
@@ -294,12 +295,35 @@ feat_kernel(const DevTables *__restrict__ tables, const int16_t *__restrict__ pc
         const unsigned int *pw = reinterpret_cast<const unsigned int *>(pcm + (long long)s * stride + base) + L;
         const unsigned int *hw = reinterpret_cast<const unsigned int *>(hist + (long long)s * hist_len + hist_len + base) + L;
         const int pth = (2 - t) * (NNSP_B200_FRAME / 2);                   /* pairs below pth precede the call */
+        /* hist_out (pipelined cascade calls): a frame among the stream's newest hist_frames also goes into the next
+         * call's PCM history, at frame hist_frames - (Ts - t). Its own 160 samples are window words 160..239 (a = 10..14),
+         * which always come from this call's PCM. */
+        unsigned int *ho = nullptr;
+        if (hist_out && valid && t >= Ts - hist_frames)
+            ho = reinterpret_cast<unsigned int *>(hist_out + (long long)s * hist_len + hist_len + base - Ts * NNSP_B200_FRAME) + L;
         auto load_pair = [&](int a, int p) -> uint32_t {
             if (RAGGED && !valid) return 0u;
-            return (p < pth) ? __ldg(hw + 16 * a) : __ldg(pw + 16 * a);
+            const uint32_t v = (p < pth) ? __ldg(hw + 16 * a) : __ldg(pw + 16 * a);
+            if (a >= 10 && ho) ho[16 * a] = v;
+            return v;
         };
+        /* lm_out: the same for the log-mel row, into the next call's lm_rows-row log-mel history (row lm_rows - (Ts - t)) */
+        int32_t *lo = nullptr;
+        if (lm_out && valid && t >= Ts - lm_rows) lo = lm_out + ((long long)s * lm_rows + lm_rows - (Ts - t)) * NNSP_B200_NMEL;
         const long long row = ((long long)s * T + t) * NNSP_B200_NMEL;
-        frame_logmel<false>(sm.tb, fs, L, load_pair, logmel + row, valid, FeatDump{}, snorm, feat16 + row);
+        frame_logmel<false>(sm.tb, fs, L, load_pair, logmel + row, valid, FeatDump{}, snorm, feat16 + row, lo);
+    }
+    /* the frames of the old history that stay among a stream's newest hist_frames (it has fewer frames in this call):
+     * hist_out frames [0, hist_frames - Ts) <- hist frames [Ts, hist_frames), a warp per stream */
+    if (hist_out && (RAGGED || T < hist_frames)) {
+        const int wpf = NNSP_B200_FRAME / 2, words = hist_frames * wpf;
+        for (int w = blockIdx.x * FEAT_WARPS + warp; w < ns; w += gridDim.x * FEAT_WARPS) {
+            const long long s = s0 + w;
+            const int Ts = RAGGED ? stream_frames(nfr, s, T) : T;
+            const unsigned int *hi = reinterpret_cast<const unsigned int *>(hist) + s * words + Ts * wpf;
+            unsigned int *ho = reinterpret_cast<unsigned int *>(hist_out) + s * words;
+            for (int i = lane; i < words - Ts * wpf; i += 32) ho[i] = hi[i];
+        }
     }
 }
 
@@ -343,10 +367,10 @@ int launch_feature(const DevTables *tb, const FeatLaunch &a, int device, cudaStr
     const size_t smem = sizeof(FeatSmem) + (pad > 0 ? pad : 0);
     if (a.nfr)
         feat_kernel<true><<<(unsigned)blocks, FEAT_THREADS, smem, st>>>(tb, a.pcm, a.stride, a.hist, a.hist_frames, a.s0, a.ns, a.T,
-                                                                       a.logmel, a.norm, a.feat16, a.nfr);
+                                                                       a.logmel, a.norm, a.feat16, a.nfr, a.hist_out, a.lm_out, a.lm_rows);
     else
         feat_kernel<false><<<(unsigned)blocks, FEAT_THREADS, smem, st>>>(tb, a.pcm, a.stride, a.hist, a.hist_frames, a.s0, a.ns, a.T,
-                                                                        a.logmel, a.norm, a.feat16, nullptr);
+                                                                        a.logmel, a.norm, a.feat16, nullptr, a.hist_out, a.lm_out, a.lm_rows);
     NNSP_LAUNCH_CHECK();
     return NNSP_B200_OK;
 }
@@ -382,34 +406,6 @@ __global__ void hist_kernel(const unsigned int *__restrict__ src, long long stri
         }
         for (int i = lane; i < tw; i += 32) h[kw + i] = p[i];
     }
-}
-
-/* out of place: hist_out <- newest hist_frames frames of (hist_in ++ src[0..T)) */
-template <bool RAGGED>
-__global__ void hist_roll_kernel(const unsigned int *__restrict__ src, long long stride_words, const unsigned int *__restrict__ hist_in,
-                                 unsigned int *__restrict__ hist_out, int hist_frames, int wpf, int s0, int ns, int T_call,
-                                 const int32_t *__restrict__ nfr)
-{
-    const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
-    if (warp >= ns) return;
-    const long long s = s0 + warp;
-    const int T = RAGGED ? stream_frames(nfr, s, T_call) : T_call;            /* 0: hist_out is hist_in */
-    const int words = hist_frames * wpf, keep = (hist_frames - T) * wpf;       /* words of the old history that survive */
-    const unsigned int *hi = hist_in + s * words, *p = src + s * stride_words;
-    unsigned int *ho = hist_out + s * words;
-    for (int i = lane; i < words; i += 32)
-        ho[i] = (i < keep) ? hi[i + T * wpf] : p[(long long)(T - hist_frames) * wpf + i];
-}
-
-int launch_hist_roll(const void *src, long long stride_words, const void *hist_in, void *hist_out, int hist_frames,
-                     int words_per_frame, int s0, int ns, int T, cudaStream_t st, const int32_t *nfr)
-{
-    if (ns <= 0 || T <= 0 || hist_frames <= 0) return NNSP_B200_OK;
-    const int threads = 256, blocks = (ns * 32 + threads - 1) / threads;
-    (nfr ? hist_roll_kernel<true> : hist_roll_kernel<false>)<<<blocks, threads, 0, st>>>((const unsigned int *)src, stride_words, (const unsigned int *)hist_in,
-                                                 (unsigned int *)hist_out, hist_frames, words_per_frame, s0, ns, T, nfr);
-    NNSP_LAUNCH_CHECK();
-    return NNSP_B200_OK;
 }
 
 int launch_hist_update(const void *src, long long stride_words, void *hist, int hist_frames, int words_per_frame,

@@ -127,12 +127,13 @@ __device__ __forceinline__ int xpad(int p) { return p + (p >> 4); }
  * compile-time constant after unrolling, so callers can address with immediates).
  * Every lane of the WARP must call this together (full-warp __syncwarp inside). */
 /* norm (optional, shared memory): mean[40], stdR[40], rshift of a model. When given, the standardised row
- * (feature_module.c:67-73) is written to out_feat as int16 instead of the log-mel row to out_logmel. */
+ * (feature_module.c:67-73) is written to out_feat as int16 instead of the log-mel row to out_logmel.
+ * out_copy (optional, log-mel mode): a second place the log-mel row is written to. */
 template <bool DUMP, typename LoadPair>
 __device__ __forceinline__ void frame_logmel(const FeatSmemTables &tb, FrameScratch &fs, int L,
                                              LoadPair load_pair, int32_t *__restrict__ out_logmel,
                                              bool store, FeatDump dump, const int32_t *norm = nullptr,
-                                             int16_t *__restrict__ out_feat = nullptr)
+                                             int16_t *__restrict__ out_feat = nullptr, int32_t *__restrict__ out_copy = nullptr)
 {
     int32_t xr[16], xi[16];
     /* window, Q15 x Q15 >> 15 (spectrogram_module.c:62-66); zero padding 480..511 (:68-71) */
@@ -264,7 +265,10 @@ __device__ __forceinline__ void frame_logmel(const FeatSmemTables &tb, FrameScra
             if (store) {
                 const int32_t lm = log10_q15(mel, tb.log_lut);
                 if (norm) out_feat[b] = standardise(lm, norm[b], norm[40 + b], norm[80]);
-                else out_logmel[b] = lm;
+                else {
+                    out_logmel[b] = lm;
+                    if (out_copy) out_copy[b] = lm;
+                }
             }
         }
     }
