@@ -8,13 +8,13 @@
  * context row 5 of every instance (feature_module.c:39-42 refills rows 0..4 only).
  *
  * Per exec call:
- *   feat_kernel    : log-mel of every raw (undelayed) frame of the call, full 3-frame window
+ *   feat_kernel    : log-mel of every raw (undelayed) frame of the call, full 3-frame window; also the
+ *                    newest d_max+2 PCM frames and d_max log-mel rows, the next call's histories
  *   cascade_kernel : per stream (one warp), frame by frame: pick the active model and its look-back d,
  *                    take the log-mel row of frame t-d (this call or the log-mel history), or -- for the
  *                    first two frames after an activation, whose window is partly the zeroed
  *                    dataBuffer -- recompute it on the spot; standardise, network, post-processing,
- *                    controller transition, reset-on-exit
- *   hist kernels   : newest d_max+2 PCM frames and d_max log-mel rows for the next call */
+ *                    controller transition, reset-on-exit */
 #include <algorithm>
 #include <cstdlib>
 #include <cuda_runtime.h>
@@ -736,9 +736,6 @@ struct CascadePostArgs {
     nnsp_b200_cascade_result *results;
     CascadeDev cd;
     const int32_t *nfr;              /* ragged call: stream s ends at frame stream_frames(nfr, s, T) */
-    int32_t *lm_next;                /* pipelined call shorter than the log-mel history, or ragged (else null): the next
-                                        call's history, whose newest rows feat_kernel wrote; cascade_ctx_kernel adds the
-                                        rows of st.lmhist that stay */
 };
 
 /* log-mel row the instance of stream s reads at frame f of the call (f >= its tb): a fix row during its first two frames */
@@ -916,20 +913,13 @@ __global__ void __launch_bounds__(32 * CPOST_WARPS) cascade_post_kernel(CascadeP
 
 /* context of the instances that lived through the call (t0 == T + 1): the newest six standardised rows of (the rows the
  * instance had when its life in this call began ++ the rows of its frames tb .. Ts-1, read with its look-back); a warp
- * per stream. With lm_next, first the rows of the log-mel history that stay in the next one: next rows
- * [0, dmax - Ts) <- st.lmhist rows [Ts, dmax). This runs after the call's resets and imports (head of the chain). */
+ * per stream */
 __global__ void __launch_bounds__(256) cascade_ctx_kernel(CascadePostArgs a)
 {
     const int si = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
     if (si >= a.ns) return;
     const long long s = a.s0 + si;
     const int T = a.T;
-    if (a.lm_next) {
-        const int words = a.cd.dmax * NNSP_B200_NMEL, Ts = stream_frames(a.nfr, s, T);
-        const int32_t *hi = a.st.lmhist + s * words + Ts * NNSP_B200_NMEL;
-        int32_t *ho = a.lm_next + s * words;
-        for (int i = lane; i < words - Ts * NNSP_B200_NMEL; i += 32) ho[i] = hi[i];
-    }
     if (a.ra.t0[s] != T + 1) return;
     const CascadeDev &cd = a.cd;
     const int id = cd.seq[a.st.casc[s * CS_N + CS_POS]];
@@ -981,9 +971,9 @@ constexpr int OP_INSTANCE = 0, OP_FRESH = 1, OP_LOAD = 2, OP_LOAD_INSTANCE = 3;
  * its context row 5. fresh != 0 (create = init + reset on zeroed structs) also rewinds and clears those.
  * list == null: streams 0 .. S-1, one per CTA, all with `fresh`; else the entries list[0 .. gridDim.x) (OP_*):
  * OP_LOAD writes the record recs[entry >> 2] into its stream, OP_LOAD_INSTANCE does that and then the reset.
- * `parts` says what is written: the PCM ring, which the front end reads, and the controller /
- * instance state with the log-mel history, which the chain reads -- a pipelined call resets them on different streams. */
-constexpr int RESET_RING = 1, RESET_STATE = 2;
+ * `parts` says what is written: the histories (PCM ring and log-mel rows), which the front end reads and rewrites, and
+ * the controller / instance state, which the chain reads -- a pipelined call resets them on different streams. */
+constexpr int RESET_HIST = 1, RESET_STATE = 2;
 __global__ void cascade_reset_kernel(ResetModels rm, StreamState st, int16_t *stale, int S,
                                      int hist_words, int lm_words, int fresh, const int *list, int parts, const uint8_t *recs)
 {
@@ -1004,7 +994,6 @@ __global__ void cascade_reset_kernel(ResetModels rm, StreamState st, int16_t *st
         copy8(st.h + (long long)s * HS, rec + REC_H, HS * 2);
         copy8(st.c + (long long)s * HS, rec + REC_C, HS * 4);
         copy8(stale + (long long)s * 120, rec + REC_STALE, 120 * 2);
-        copy8(st.lmhist + (long long)s * lm_words, rec + REC_RING + 4LL * hist_words, lm_words * 4);
     }
     if ((parts & RESET_STATE) && op != OP_LOAD) {
         const bool fresh = op == OP_FRESH;
@@ -1020,13 +1009,17 @@ __global__ void cascade_reset_kernel(ResetModels rm, StreamState st, int16_t *st
         for (int i = threadIdx.x; i < HS; i += blockDim.x) { st.h[(long long)s * HS + i] = 0; st.c[(long long)s * HS + i] = 0; }
         for (int i = threadIdx.x; i < SC_N; i += blockDim.x) st.scal[(long long)s * SC_N + i] = (i == SC_SLIDES) ? 1 : 0;
         for (int i = threadIdx.x; i < CS_N; i += blockDim.x) st.casc[(long long)s * CS_N + i] = (i == CS_POS) ? (uint16_t)pos : (uint16_t)0;
-        int32_t *lm = st.lmhist + (long long)s * lm_words;
-        for (int i = threadIdx.x; i < lm_words; i += blockDim.x) lm[i] = LOGMEL_OF_ZERO;       /* log-mel of an all-zero window */
     }
-    if (parts & RESET_RING) {
+    if (parts & RESET_HIST) {                   /* OP_LOAD_INSTANCE: the reset overwrites all the load would write here */
         unsigned int *h = reinterpret_cast<unsigned int *>(st.hist) + (long long)s * hist_words;
-        if (op == OP_LOAD) copy8(h, rec + REC_RING, hist_words * 4);
-        else for (int i = threadIdx.x; i < hist_words; i += blockDim.x) h[i] = 0;              /* PcmBufClass_reset, PcmBufClass.c:19-28 */
+        int32_t *lm = st.lmhist + (long long)s * lm_words;
+        if (op == OP_LOAD) {
+            copy8(h, rec + REC_RING, hist_words * 4);
+            copy8(lm, rec + REC_RING + 4LL * hist_words, lm_words * 4);
+        } else {
+            for (int i = threadIdx.x; i < hist_words; i += blockDim.x) h[i] = 0;              /* PcmBufClass_reset, PcmBufClass.c:19-28 */
+            for (int i = threadIdx.x; i < lm_words; i += blockDim.x) lm[i] = LOGMEL_OF_ZERO;  /* log-mel of an all-zero window */
+        }
     }
 }
 
@@ -1099,15 +1092,17 @@ struct nnsp_b200_cascade {
     long long split_cap_T = 0;
     cudaStream_t gs[4][3] = {};                /* per pipeline stream (3 host-call streams + the device-call stream): one per model group */
     /* device-buffer calls are pipelined like the batched path: front end of call N+1 on `stream`, controller / network
-     * work of call N on `nn_stream`; log-mel rows are double buffered. The PCM and log-mel histories are triple
-     * buffered: call N+1's front end writes the next histories into the buffers that call N-1's chain read, which it
-     * waits for anyway (for its log-mel rows), while call N's chain may still read the ones call N read. */
+     * work of call N on `nn_stream`; log-mel rows are double buffered */
     cudaStream_t nn_stream = nullptr;
     cudaEvent_t ev_feat[2] = { nullptr, nullptr }, ev_nn[2] = { nullptr, nullptr };
     bool nn_pending[2] = { false, false }, last_piped = false;
     unsigned pipe = 0;
     int32_t *logmel2 = nullptr;                /* second log-mel buffer */
-    int16_t *hist2 = nullptr, *hist3 = nullptr;   /* the next PCM history (written by the pipelined call), the spare */
+    /* Every call's front end writes the next PCM and log-mel histories into hist2 / lmhist2, and the three buffers of
+     * each rotate once per call (cascade_next_hist). Three, because a pipelined call N+1's front end then writes the
+     * buffers that call N-1's chain read, which it waits for anyway (for its log-mel rows), while call N's chain may
+     * still read the ones call N read. */
+    int16_t *hist2 = nullptr, *hist3 = nullptr;       /* the next PCM history, the spare */
     int32_t *lmhist2 = nullptr, *lmhist3 = nullptr;   /* the same for the log-mel history */
     cudaEvent_t ev_fork[4] = {}, ev_join[4][3] = {};
     /* asynchronous host-buffer calls: one completion event per pipeline stream, a ring of CS_HOST_RING calls */
@@ -1277,32 +1272,30 @@ static int cascade_take_resets(nnsp_b200_cascade *c, const int **list, int *n, i
 struct PendingOps {
     const int *list; int n;
     const uint8_t *recs;
-    cudaEvent_t read_ring, read_state;
+    cudaEvent_t read_hist, read_state;
 };
 
-/* st_nn (with ev_feat): pipelined call -- everything behind the front end goes to st_nn; the front end writes the next
- * PCM and log-mel histories out of place into c->hist2 / c->lmhist2 (the caller rotates the buffers afterwards).
- * ops (null: none): streams reset or loaded before the call -- the PCM ring on st before the front end reads it, the
+/* The front end writes the next PCM and log-mel histories of streams s0 .. s0+ns-1 out of place into c->hist2 /
+ * c->lmhist2 (the caller rotates the buffers once per call: cascade_next_hist).
+ * st_nn (with ev_feat): pipelined call -- everything behind the front end goes to st_nn.
+ * ops (null: none): streams reset or loaded before the call -- the histories on st before the front end reads them, the
  * rest on the stream of the chain before the chain reads it. */
 static int cascade_launch(nnsp_b200_cascade *c, const int16_t *pcm, long long stride, int T, int s0, int ns,
                           nnsp_b200_cascade_result *results, const nnsp_b200_taps *taps, cudaStream_t st, bool timed,
                           int slice = 0, int32_t *logmel = nullptr, cudaStream_t st_nn = nullptr, cudaEvent_t ev_feat = nullptr,
                           const int32_t *nfr = nullptr, const PendingOps *ops = nullptr)
 {
-    const int hist_frames = c->cd.dmax + 2;
     if (!logmel) logmel = c->logmel;
     const bool piped = st_nn != nullptr;
     int rc;
     if (ops) {
-        if ((rc = cascade_launch_reset(c, ops->list, ops->n, 0, piped ? RESET_RING : RESET_RING | RESET_STATE, st, ops->recs))) return rc;
-        if (ops->recs) NNSP_CUDA(cudaEventRecord(ops->read_ring, st));
+        if ((rc = cascade_launch_reset(c, ops->list, ops->n, 0, piped ? RESET_HIST : RESET_HIST | RESET_STATE, st, ops->recs))) return rc;
+        if (ops->recs) NNSP_CUDA(cudaEventRecord(ops->read_hist, st));
     }
-    FeatLaunch fl{ pcm, stride, c->st.hist, hist_frames, s0, ns, T, logmel };
+    FeatLaunch fl{ pcm, stride, c->st.hist, c->cd.dmax + 2, s0, ns, T, logmel };
     fl.nfr = nfr;
-    if (piped) {
-        fl.hist_out = c->hist2;
-        if (c->cd.dmax > 0) { fl.lm_out = c->lmhist2; fl.lm_rows = c->cd.dmax; }
-    }
+    fl.hist_out = c->hist2;
+    if (c->cd.dmax > 0) { fl.lm_hist = c->st.lmhist; fl.lm_out = c->lmhist2; fl.lm_rows = c->cd.dmax; }
     cudaEvent_t *tl = c->tl[c->tl_count % 8];
     if (timed) NNSP_CUDA(cudaEventRecord(tl[0], st));
     rc = launch_feature(c->tables, fl, c->device, st);
@@ -1340,7 +1333,6 @@ static int cascade_launch(nnsp_b200_cascade *c, const int16_t *pcm, long long st
         for (int i = 0; i < 3; i++) p.model[i] = c->mm[i].d;
         p.st = c->st; p.stale = c->stale; p.logmel = logmel; p.dec = c->dec; p.dec_stride = n_inf_max; p.ra = c->ra;
         p.s0 = s0; p.ns = ns; p.T = T; p.results = results; p.cd = c->cd; p.nfr = nfr;
-        if (piped && c->cd.dmax > 0 && (nfr || T < c->cd.dmax)) p.lm_next = c->lmhist2;
         for (int r = 0; r < c->rounds; r++) {
             int *ctl_r = ctl + CTL_ROUND * r, *ctl_prev = ctl + CTL_ROUND * (r - 1);
             const int *queued = r ? c->pend[r & 1] + s0 : nullptr;        /* streams the previous round's walk queued */
@@ -1419,10 +1411,16 @@ static int cascade_launch(nnsp_b200_cascade *c, const int16_t *pcm, long long st
         NNSP_CUDA(cudaEventRecord(tl[3], st));
         c->ev_valid = true; c->last_piped = piped; c->tl_count++;
     }
-    if (!piped && (rc = launch_hist_update(pcm, stride / 2, c->st.hist, hist_frames, NNSP_B200_FRAME / 2, s0, ns, T, st, nfr))) return rc;
-    if (!piped && c->cd.dmax > 0)
-        rc = launch_hist_update(logmel, (long long)T * NNSP_B200_NMEL, c->st.lmhist, c->cd.dmax, NNSP_B200_NMEL, s0, ns, T, st, nfr);
-    return rc;
+    return NNSP_B200_OK;
+}
+
+/* after a call (never per slice: every slice of a host call reads the same buffers, and slice k always covers the same
+ * streams on the same CUDA stream): the histories its front end wrote are the live ones. Without a look-back the
+ * one-row log-mel history is never written and does not rotate. */
+static void cascade_next_hist(nnsp_b200_cascade *c)
+{
+    int16_t *t = c->st.hist; c->st.hist = c->hist2; c->hist2 = c->hist3; c->hist3 = t;
+    if (c->cd.dmax > 0) { int32_t *u = c->st.lmhist; c->st.lmhist = c->lmhist2; c->lmhist2 = c->lmhist3; c->lmhist3 = u; }
 }
 
 static int cascade_join_nn(nnsp_b200_cascade *c, cudaStream_t st)
@@ -1592,7 +1590,7 @@ int nnsp_b200_cascade_create(const nnsp_b200_model *const models[3], const int *
         H.model_fnv1a[k] = f;
     }
     if (cudaDeviceSynchronize() != cudaSuccess) return fail(NNSP_B200_ERR_CUDA);   /* uploads went through the default stream */
-    if ((rc = cascade_launch_reset(c, nullptr, 0, 1, RESET_RING | RESET_STATE, c->stream))) return fail(rc);
+    if ((rc = cascade_launch_reset(c, nullptr, 0, 1, RESET_HIST | RESET_STATE, c->stream))) return fail(rc);
     if (cudaStreamSynchronize(c->stream) != cudaSuccess) { nnsp_set_error("cascade reset kernel failed: %s", cudaGetErrorString(cudaGetLastError())); return fail(NNSP_B200_ERR_CUDA); }
     *out = c;
     return NNSP_B200_OK;
@@ -1638,7 +1636,7 @@ int nnsp_b200_cascade_reset(nnsp_b200_cascade *c)
      * reset: it becomes load-then-reset. */
     for (int s : c->rs_ids)
         if (c->rs_mode[(size_t)s] == OP_LOAD) c->rs_mode[(size_t)s] = OP_LOAD_INSTANCE;
-    const int rc = cascade_launch_reset(c, nullptr, 0, 0, RESET_RING | RESET_STATE, c->stream);
+    const int rc = cascade_launch_reset(c, nullptr, 0, 0, RESET_HIST | RESET_STATE, c->stream);
     if (rc) return rc;
     NNSP_CUDA(cudaStreamSynchronize(c->stream));
     return NNSP_B200_OK;
@@ -1747,7 +1745,7 @@ int nnsp_b200_cascade_export_streams(nnsp_b200_cascade *c, const int32_t *stream
         NNSP_CUDA(cudaEventRecord(c->rs_copied[rb][0], c->stream));
         c->rs_copy_valid[rb][0] = true;
         if (loads) NNSP_CUDA(cudaMemcpyAsync(c->rp_dev[rb], c->rp_host[rb], (size_t)loads * c->rec_bytes, cudaMemcpyHostToDevice, c->stream));
-        if ((rc = cascade_launch_reset(c, c->rs_dev[0], rn, 0, RESET_RING | RESET_STATE, c->stream, loads ? c->rp_dev[rb] : nullptr))) return rc;
+        if ((rc = cascade_launch_reset(c, c->rs_dev[0], rn, 0, RESET_HIST | RESET_STATE, c->stream, loads ? c->rp_dev[rb] : nullptr))) return rc;
         if (loads) { NNSP_CUDA(cudaEventRecord(c->rp_read[rb][0], c->stream)); c->rp_read_valid[rb][0] = true; }
     }
     if (n > c->ex_cap) {
@@ -1800,7 +1798,7 @@ static int cascade_exec_dev(nnsp_b200_cascade *c, const int16_t *pcm_dev, long l
         if (loads) {
             NNSP_CUDA(cudaMemcpyAsync(c->rp_dev[rb], c->rp_host[rb], (size_t)loads * c->rec_bytes, cudaMemcpyHostToDevice, c->stream));
             ops.recs = c->rp_dev[rb];
-            ops.read_ring = c->rp_read[rb][0]; c->rp_read_valid[rb][0] = true;
+            ops.read_hist = c->rp_read[rb][0]; c->rp_read_valid[rb][0] = true;
             if (piped) { ops.read_state = c->rp_read[rb][3]; c->rp_read_valid[rb][3] = true; }
         }
         return NNSP_B200_OK;
@@ -1808,23 +1806,22 @@ static int cascade_exec_dev(nnsp_b200_cascade *c, const int16_t *pcm_dev, long l
     if ((rc = cascade_take_resets(c, &rl, &rn, &rb, &loads))) return rc;
     if (cascade_use_split(c, taps)) {
         const int i = (int)(c->pipe++ & 1u);
-        if (c->nn_pending[i]) NNSP_CUDA(cudaStreamWaitEvent(c->stream, c->ev_nn[i], 0));   /* log-mel buffer i / PCM history in use two calls ago */
+        if (c->nn_pending[i]) NNSP_CUDA(cudaStreamWaitEvent(c->stream, c->ev_nn[i], 0));   /* log-mel buffer i / the histories written next: in use two calls ago */
         if (rn && (rc = upload_resets(c->rs_dev[i], true))) return rc;    /* rs_dev[i] too: its last readers ran in that chain */
         rc = cascade_launch(c, pcm_dev, stream_stride, n_frames, 0, c->S, results_dev, nullptr, c->stream, true, 0,
                             i ? c->logmel2 : c->logmel, c->nn_stream, c->ev_feat[i], nfr, rn ? &ops : nullptr);
         if (rc) return rc;
         NNSP_CUDA(cudaEventRecord(c->ev_nn[i], c->nn_stream));
         c->nn_pending[i] = true;
-        int16_t *t = c->st.hist; c->st.hist = c->hist2; c->hist2 = c->hist3; c->hist3 = t;   /* the written histories are the live ones from here on */
-        if (c->cd.dmax > 0) {                  /* without a look-back the one-row log-mel history is never written */
-            int32_t *u = c->st.lmhist; c->st.lmhist = c->lmhist2; c->lmhist2 = c->lmhist3; c->lmhist3 = u;
-        }
-        return NNSP_B200_OK;
+    } else {
+        if ((rc = cascade_join_nn(c, c->stream))) return rc;
+        if (rn && (rc = upload_resets(c->rs_dev[0], false))) return rc;
+        rc = cascade_launch(c, pcm_dev, stream_stride, n_frames, 0, c->S, results_dev, taps, c->stream, true, 0, nullptr, nullptr,
+                            nullptr, nfr, rn ? &ops : nullptr);
+        if (rc) return rc;
     }
-    if ((rc = cascade_join_nn(c, c->stream))) return rc;
-    if (rn && (rc = upload_resets(c->rs_dev[0], false))) return rc;
-    return cascade_launch(c, pcm_dev, stream_stride, n_frames, 0, c->S, results_dev, taps, c->stream, true, 0, nullptr, nullptr,
-                          nullptr, nfr, rn ? &ops : nullptr);
+    cascade_next_hist(c);
+    return NNSP_B200_OK;
 }
 
 int nnsp_b200_cascade_exec(nnsp_b200_cascade *c, const int16_t *pcm_dev, long long stream_stride, int n_frames,
@@ -1944,7 +1941,7 @@ static int cascade_enqueue_host(nnsp_b200_cascade *c, const int16_t *pcm, long l
                 NNSP_CUDA(cudaMemcpyAsync(c->rp_dev[rb] + (size_t)p0 * c->rec_bytes, c->rp_host[rb] + (size_t)p0 * c->rec_bytes,
                                           (size_t)(p1 - p0) * c->rec_bytes, cudaMemcpyHostToDevice, st));
                 ops.recs = c->rp_dev[rb];
-                ops.read_ring = c->rp_read[rb][k % 3];
+                ops.read_hist = c->rp_read[rb][k % 3];
                 c->rp_read_valid[rb][k % 3] = true;
             }
         }
@@ -1957,6 +1954,7 @@ static int cascade_enqueue_host(nnsp_b200_cascade *c, const int16_t *pcm, long l
             NNSP_CUDA(cudaMemcpyAsync(results + (size_t)s0 * T, c->d_res + (size_t)s0 * T,
                                       (size_t)(s1 - s0) * T * sizeof(nnsp_b200_cascade_result), cudaMemcpyDeviceToHost, st));
     }
+    cascade_next_hist(c);
     return NNSP_B200_OK;
 }
 

@@ -2,17 +2,18 @@
  *
  * Two kernels per exec call:
  *   feat_kernel : log-mel of every (stream, frame) of the call; frames are independent, so the
- *                 grid covers S*T frames with one half-warp each (nnsp_feat.cuh)
+ *                 grid covers S*T frames with one half-warp each (nnsp_feat.cuh); it also writes
+ *                 the last two PCM frames into the next call's history, for its windows
  *   nn_kernel   : per stream (one warp), the T frames in order: standardise the new row into
  *                 the 6x40 context, every 2nd frame run the network and the post-processing,
  *                 update the NNSPClass scalars and LSTM state (nnsp_net.cuh)
- * plus a tiny hist_kernel that keeps the last two PCM frames for the next call's windows.
  * sm_100a only; no CPU path exists. */
 #include <cuda_runtime.h>
 #include <mutex>
 #include <new>
 #include <stdlib.h>
 #include <string.h>
+#include <utility>
 
 #include "nnsp_feat.cuh"
 #include "nnsp_host.h"
@@ -267,7 +268,8 @@ __global__ void __launch_bounds__(FEAT_THREADS, FEAT_CTAS_PER_SM)
 feat_kernel(const DevTables *__restrict__ tables, const int16_t *__restrict__ pcm, long long stride,
             const int16_t *__restrict__ hist, int hist_frames, int s0, int ns, int T,
             int32_t *__restrict__ logmel, const int32_t *__restrict__ norm, int16_t *__restrict__ feat16,
-            const int32_t *__restrict__ nfr, int16_t *__restrict__ hist_out, int32_t *__restrict__ lm_out, int lm_rows)
+            const int32_t *__restrict__ nfr, int16_t *__restrict__ hist_out, const int32_t *__restrict__ lm_hist,
+            int32_t *__restrict__ lm_out, int lm_rows)
 {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     FeatSmem &sm = *reinterpret_cast<FeatSmem *>(smem_raw);
@@ -295,9 +297,9 @@ feat_kernel(const DevTables *__restrict__ tables, const int16_t *__restrict__ pc
         const unsigned int *pw = reinterpret_cast<const unsigned int *>(pcm + (long long)s * stride + base) + L;
         const unsigned int *hw = reinterpret_cast<const unsigned int *>(hist + (long long)s * hist_len + hist_len + base) + L;
         const int pth = (2 - t) * (NNSP_B200_FRAME / 2);                   /* pairs below pth precede the call */
-        /* hist_out (pipelined cascade calls): a frame among the stream's newest hist_frames also goes into the next
-         * call's PCM history, at frame hist_frames - (Ts - t). Its own 160 samples are window words 160..239 (a = 10..14),
-         * which always come from this call's PCM. */
+        /* hist_out: a frame among the stream's newest hist_frames also goes into the next call's PCM history, at frame
+         * hist_frames - (Ts - t). Its own 160 samples are window words 160..239 (a = 10..14), which always come from this
+         * call's PCM. */
         unsigned int *ho = nullptr;
         if (hist_out && valid && t >= Ts - hist_frames)
             ho = reinterpret_cast<unsigned int *>(hist_out + (long long)s * hist_len + hist_len + base - Ts * NNSP_B200_FRAME) + L;
@@ -313,18 +315,20 @@ feat_kernel(const DevTables *__restrict__ tables, const int16_t *__restrict__ pc
         const long long row = ((long long)s * T + t) * NNSP_B200_NMEL;
         frame_logmel<false>(sm.tb, fs, L, load_pair, logmel + row, valid, FeatDump{}, snorm, feat16 + row, lo);
     }
-    /* the frames of the old history that stay among a stream's newest hist_frames (it has fewer frames in this call):
-     * hist_out frames [0, hist_frames - Ts) <- hist frames [Ts, hist_frames), a warp per stream */
-    if (hist_out && (RAGGED || T < hist_frames)) {
-        const int wpf = NNSP_B200_FRAME / 2, words = hist_frames * wpf;
+    /* the frames of an old history that stay among a stream's newest `frames` (it has fewer frames in this call):
+     * out frames [0, frames - Ts) <- in frames [Ts, frames), frames of wpf words, a warp per stream */
+    auto keep_old = [&](const void *in, void *out, int frames, int wpf) {
+        const int words = frames * wpf;
         for (int w = blockIdx.x * FEAT_WARPS + warp; w < ns; w += gridDim.x * FEAT_WARPS) {
             const long long s = s0 + w;
             const int Ts = RAGGED ? stream_frames(nfr, s, T) : T;
-            const unsigned int *hi = reinterpret_cast<const unsigned int *>(hist) + s * words + Ts * wpf;
-            unsigned int *ho = reinterpret_cast<unsigned int *>(hist_out) + s * words;
+            const unsigned int *hi = static_cast<const unsigned int *>(in) + s * words + Ts * wpf;
+            unsigned int *ho = static_cast<unsigned int *>(out) + s * words;
             for (int i = lane; i < words - Ts * wpf; i += 32) ho[i] = hi[i];
         }
-    }
+    };
+    if (hist_out && (RAGGED || T < hist_frames)) keep_old(hist, hist_out, hist_frames, NNSP_B200_FRAME / 2);
+    if (lm_out && (RAGGED || T < lm_rows)) keep_old(lm_hist, lm_out, lm_rows, NNSP_B200_NMEL);
 }
 
 int launch_feature(const DevTables *tb, const FeatLaunch &a, int device, cudaStream_t st)
@@ -367,54 +371,10 @@ int launch_feature(const DevTables *tb, const FeatLaunch &a, int device, cudaStr
     const size_t smem = sizeof(FeatSmem) + (pad > 0 ? pad : 0);
     if (a.nfr)
         feat_kernel<true><<<(unsigned)blocks, FEAT_THREADS, smem, st>>>(tb, a.pcm, a.stride, a.hist, a.hist_frames, a.s0, a.ns, a.T,
-                                                                       a.logmel, a.norm, a.feat16, a.nfr, a.hist_out, a.lm_out, a.lm_rows);
+                                                                       a.logmel, a.norm, a.feat16, a.nfr, a.hist_out, a.lm_hist, a.lm_out, a.lm_rows);
     else
         feat_kernel<false><<<(unsigned)blocks, FEAT_THREADS, smem, st>>>(tb, a.pcm, a.stride, a.hist, a.hist_frames, a.s0, a.ns, a.T,
-                                                                        a.logmel, a.norm, a.feat16, nullptr, a.hist_out, a.lm_out, a.lm_rows);
-    NNSP_LAUNCH_CHECK();
-    return NNSP_B200_OK;
-}
-
-/* keep the newest hist_frames frames of (previous history ++ this call) for the next call; a "frame" is
- * wpf 32-bit words (80 for PCM, 40 for log-mel rows). A ragged cascade call appends stream s's own frame count. */
-template <bool RAGGED>
-__global__ void hist_kernel(const unsigned int *__restrict__ src, long long stride_words, unsigned int *__restrict__ hist,
-                            int hist_frames, int wpf, int s0, int ns, int T_call, const int32_t *__restrict__ nfr)
-{
-    const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
-    if (warp >= ns) return;
-    const int s = s0 + warp;
-    const int T = RAGGED ? stream_frames(nfr, s, T_call) : T_call;
-    if (RAGGED && T == 0) return;
-    const int words = hist_frames * wpf;
-    const int keep = hist_frames - T;                                  /* frames of old history that survive (T < hist_frames) */
-    unsigned int *h = hist + (long long)s * words;
-    const unsigned int *p = src + (long long)s * stride_words;
-    if (keep <= 0) {
-        const unsigned int *q = p + (long long)(T - hist_frames) * wpf;
-        for (int i = lane; i < words; i += 32) h[i] = q[i];
-    } else {
-        /* shift old frames down by T, append the T new ones; chunked so reads precede overlapping writes */
-        const int kw = keep * wpf, tw = T * wpf;
-        for (int i0 = 0; i0 < kw; i0 += 32) {
-            const int i = i0 + lane;
-            unsigned int v = 0;
-            if (i < kw) v = h[i + tw];
-            __syncwarp();
-            if (i < kw) h[i] = v;
-            __syncwarp();
-        }
-        for (int i = lane; i < tw; i += 32) h[kw + i] = p[i];
-    }
-}
-
-int launch_hist_update(const void *src, long long stride_words, void *hist, int hist_frames, int words_per_frame,
-                       int s0, int ns, int T, cudaStream_t st, const int32_t *nfr)
-{
-    if (ns <= 0 || T <= 0 || hist_frames <= 0) return NNSP_B200_OK;
-    const int threads = 256, blocks = (ns * 32 + threads - 1) / threads;
-    (nfr ? hist_kernel<true> : hist_kernel<false>)<<<blocks, threads, 0, st>>>((const unsigned int *)src, stride_words, (unsigned int *)hist, hist_frames,
-                                            words_per_frame, s0, ns, T, nfr);
+                                                                        a.logmel, a.norm, a.feat16, nullptr, a.hist_out, a.lm_hist, a.lm_out, a.lm_rows);
     NNSP_LAUNCH_CHECK();
     return NNSP_B200_OK;
 }
@@ -692,6 +652,7 @@ struct nnsp_b200_batch {
     unsigned pipe = 0;
     int32_t *norm_dev = nullptr;            /* mean[40], stdR[40], rshift for feat_kernel's standardising mode */
     StreamState st{};
+    int16_t *hist2 = nullptr;               /* the next PCM history: every front end writes it, and the two swap after each call */
     int16_t thresh_prob = 0, th_count = 0;
     int32_t *logmel = nullptr; long long logmel_frames = 0;       /* capacity in frames per stream */
     int16_t *d_pcm = nullptr; long long d_pcm_frames = 0;
@@ -759,7 +720,8 @@ static int batch_ensure_split(nnsp_b200_batch *b, int n_inf)
 }
 
 /* st: stream of the front end (and of everything else unless st_nn is given); st_nn + ev_feat: the network kernels go
- * to st_nn once ev_feat (recorded on st behind the front end and the history roll) has fired */
+ * to st_nn once ev_feat (recorded on st behind the front end) has fired. The front end writes the next PCM history into
+ * b->hist2; the caller swaps it with b->st.hist once per call. */
 static int batch_launch(nnsp_b200_batch *b, const int16_t *pcm, long long stride, int T, int s0, int ns,
                         nnsp_b200_result *results, const nnsp_b200_taps *taps, cudaStream_t st, bool timed,
                         int fbuf = 0, cudaStream_t st_nn = nullptr, cudaEvent_t ev_feat = nullptr)
@@ -767,6 +729,7 @@ static int batch_launch(nnsp_b200_batch *b, const int16_t *pcm, long long stride
     const int path = batch_nn_path(b);
     int16_t *feat16 = b->feat16[fbuf];
     FeatLaunch fl{ pcm, stride, b->st.hist, 2, s0, ns, T, b->logmel };
+    fl.hist_out = b->hist2;
     if (path == 3) { fl.logmel = nullptr; fl.norm = b->norm_dev; fl.feat16 = feat16; }
     if (timed) NNSP_CUDA(cudaEventRecord(b->ev[0], st));
     int rc = launch_feature(b->tables, fl, b->device, st);
@@ -774,8 +737,6 @@ static int batch_launch(nnsp_b200_batch *b, const int16_t *pcm, long long stride
     if (timed) NNSP_CUDA(cudaEventRecord(b->ev[1], st));
     const bool piped = st_nn != nullptr;
     if (piped) {
-        /* the history roll only needs the PCM and must precede the next call's front end: it stays on st */
-        if ((rc = launch_hist_update(pcm, stride / 2, b->st.hist, 2, NNSP_B200_FRAME / 2, s0, ns, T, st))) return rc;
         NNSP_CUDA(cudaEventRecord(ev_feat, st));
         NNSP_CUDA(cudaStreamWaitEvent(st_nn, ev_feat, 0));
         st = st_nn;
@@ -813,10 +774,11 @@ static int batch_launch(nnsp_b200_batch *b, const int16_t *pcm, long long stride
         nn_kernel<<<blocks, NN_THREADS, b->lay.total, st>>>(a, (int)b->lay.b, (int)b->lay.lut, (int)b->lay.model, (int)b->lay.scratch);
         NNSP_LAUNCH_CHECK();
     }
-    if (timed) NNSP_CUDA(cudaEventRecord(b->ev[2], st));
-    if (!piped) rc = launch_hist_update(pcm, stride / 2, b->st.hist, 2, NNSP_B200_FRAME / 2, s0, ns, T, st);
-    if (timed) { b->ev_valid = true; b->last_piped = piped; }
-    return rc;
+    if (timed) {
+        NNSP_CUDA(cudaEventRecord(b->ev[2], st));
+        b->ev_valid = true; b->last_piped = piped;
+    }
+    return NNSP_B200_OK;
 }
 
 /* everything the network stream still has in flight must be over before `st` touches the stream state */
@@ -902,6 +864,7 @@ int nnsp_b200_batch_create(const nnsp_b200_model *m, int n_streams, int device, 
     TRY(cudaMalloc(&b->st.c, S * HS * sizeof(int32_t)));
     TRY(cudaMalloc(&b->st.scal, S * SC_N * sizeof(int16_t)));
     TRY(cudaMalloc(&b->st.hist, S * 2 * NNSP_B200_FRAME * sizeof(int16_t)));
+    TRY(cudaMalloc(&b->hist2, S * 2 * NNSP_B200_FRAME * sizeof(int16_t)));
     {
         int32_t norm[84] = { 0 };
         memcpy(norm, b->dm.h.mean, 160);
@@ -963,7 +926,10 @@ int nnsp_b200_batch_exec(nnsp_b200_batch *b, const int16_t *pcm_dev, long long s
         if ((rc = batch_join_nn(b, b->stream))) return rc;
         rc = batch_launch(b, pcm_dev, stream_stride, n_frames, 0, b->S, results_dev, taps, b->stream, true);
     }
-    if (rc == NNSP_B200_OK) b->slides = (b->slides + n_frames) % 2;
+    if (rc == NNSP_B200_OK) {
+        b->slides = (b->slides + n_frames) % 2;
+        std::swap(b->st.hist, b->hist2);
+    }
     return rc;
 }
 
@@ -1075,6 +1041,7 @@ static int batch_enqueue_host(nnsp_b200_batch *b, const int16_t *pcm, long long 
                                       (size_t)(s1 - s0) * T * sizeof(nnsp_b200_result), cudaMemcpyDeviceToHost, st));
     }
     b->slides = (b->slides + T) % 2;
+    std::swap(b->st.hist, b->hist2);                    /* once per call: every slice reads the same buffer */
     return NNSP_B200_OK;
 }
 
@@ -1142,7 +1109,7 @@ void nnsp_b200_batch_destroy(nnsp_b200_batch *b)
     cudaDeviceSynchronize();
     free_model(&b->dm);
     free_model_mma(&b->mm);
-    cudaFree(b->st.ctx); cudaFree(b->st.h); cudaFree(b->st.c); cudaFree(b->st.scal); cudaFree(b->st.hist);
+    cudaFree(b->st.ctx); cudaFree(b->st.h); cudaFree(b->st.c); cudaFree(b->st.scal); cudaFree(b->st.hist); cudaFree(b->hist2);
     cudaFree(b->logmel); cudaFree(b->d_pcm); cudaFree(b->d_res); cudaFree(b->d_raw);
     cudaFree(b->sp_planes[0]); cudaFree(b->sp_planes[1]); cudaFree(b->sp_dec);
     cudaFree(b->feat16[0]); cudaFree(b->feat16[1]); cudaFree(b->norm_dev);

@@ -57,16 +57,13 @@ struct FeatLaunch {
     int16_t *feat16 = nullptr;                /* [S][T][40] standardised rows (feature_module.c:67-73) */
     const int32_t *nfr = nullptr;             /* ragged cascade call: stream s has stream_frames(nfr, s, T) frames; the rows
                                                  of its later frames are neither computed nor written, their PCM not read */
-    int16_t *hist_out = nullptr;              /* [S][hist_frames*160], not hist: receives the newest hist_frames frames of
-                                                 (hist ++ this call) per stream, i.e. the next call's history */
-    int32_t *lm_out = nullptr; int lm_rows = 0;  /* [S][lm_rows][40]: the log-mel rows of this call's frames that are among
-                                                 each stream's newest lm_rows go there (the older rows are not written) */
+    int16_t *hist_out = nullptr;              /* [S][hist_frames*160], not hist (null: not written): receives the newest
+                                                 hist_frames frames of (hist ++ this call) per stream, the next call's history */
+    const int32_t *lm_hist = nullptr;         /* [S][lm_rows][40] log-mel rows of the frames before the call, newest last */
+    int32_t *lm_out = nullptr; int lm_rows = 0;  /* [S][lm_rows][40], not lm_hist (null: not written): the newest lm_rows
+                                                 rows of (lm_hist ++ this call's rows) per stream, the next call's history */
 };
 int launch_feature(const DevTables *tb, const FeatLaunch &a, int device, cudaStream_t st);
-/* hist <- newest hist_frames frames of (hist ++ src[0..T)); frames are words_per_frame 32-bit words. nfr (ragged
- * cascade call): stream s appends only its first stream_frames(nfr, s, T) frames, none when that is 0 */
-int launch_hist_update(const void *src, long long stride_words, void *hist, int hist_frames, int words_per_frame,
-                       int s0, int ns, int T, cudaStream_t st, const int32_t *nfr = nullptr);
 
 
 /* audio_frame_callback's conditioning (evb/src/main_nnsp.cc:58-65) of n_frames consecutive 160-sample frames, raw 32-bit

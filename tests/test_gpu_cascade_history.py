@@ -1,24 +1,31 @@
-"""The cascade's PCM history on pipelined device calls: the front end of a call writes each stream's newest frames into
-the next call's history buffer (feat_kernel), which also copies the frames of the old history that stay when a stream
-has fewer frames in the call than the history holds, and three history buffers rotate so that the next call's front
-end never writes one that a chain still in flight reads.
+"""The cascade's PCM and log-mel histories: the front end of every call writes each stream's newest frames and log-mel
+rows into the next call's history buffers (feat_kernel), and copies what stays of the old histories when a stream has
+fewer frames in the call than a history holds. The three buffers of each history rotate once per call, whichever way
+the call is issued, so that a pipelined call's front end never writes one that a chain still in flight reads, and all
+slices of a host call read the same ones.
 
-  call lengths : back-to-back calls without a host wait between them, 1, 2, 57, 81, 82, 83, 100 and 257 frames mixed,
-                 against the oracle over each stream's whole audio, with the 80-frame look-back and with none (the
-                 history is then the two frames the analysis window reaches back);
-  records      : the same calls on the pipelined path and on the sequential path (in-place history update) leave
-                 byte-identical stream records after every call, for uniform and for ragged calls (counts 0 .. 257);
-  resets       : streams reset and imported between pipelined calls continue from their new history.
-The log-mel history (the look-back rows of the delayed stages) goes the same way: feat_kernel writes the newest rows,
-cascade_ctx_kernel copies the old rows that stay."""
+  call lengths : back-to-back calls of 1, 2, 57, 81, 82, 83, 100 and 257 frames mixed, issued as pipelined device
+                 calls, on the sequential path, with taps, as asynchronous host tickets (256 streams: four slices on
+                 three CUDA streams) and as one sequence that interleaves device, host and tapped calls; every stream's
+                 records byte for byte against the pipelined device calls, and every 7th stream against the oracle over
+                 its whole audio, with the 80-frame look-back and with none (the PCM history is then the two frames the
+                 analysis window reaches back);
+  records      : the same calls on the pipelined path and on the sequential path leave byte-identical stream records
+                 after every call, for uniform and for ragged calls (counts 0 .. 257);
+  resets       : streams reset and imported between pipelined device calls and between host tickets continue from
+                 their new histories."""
 import numpy as np
 import pytest
 
 import test_gpu_cascade_ragged as R
 
-S = 37
+S = 256
 LENGTHS = (100, 1, 2, 57, 81, 82, 83, 257, 100, 3, 100)
 LOOKBACK = {"lookback80": {}, "lookback0": dict(frs_vbufBk_kws=0, frs_vbufBk_s2i=0)}
+# how the calls of LENGTHS are issued, call k as issue[k % len(issue)]: "device" (exec_device, nothing waited for
+# between the calls), "host" (exec_host_async tickets, nothing waited for between them) or "tapped" (exec with taps)
+ISSUE = {"pipelined": ("device",), "sequential": ("device",), "tapped": ("tapped",), "host": ("host",),
+         "mixed": ("device", "device", "host", "host", "tapped", "device", "host", "tapped", "tapped", "host", "device")}
 
 
 def _params(extra):
@@ -31,33 +38,59 @@ def _handle(nb, path, extra):
     return h
 
 
-def _pipelined(nb, h, pcm, lengths):
-    """every call queued before any is waited for; the records of each call"""
+def _calls(nb, h, pcm, issue, before=None):
+    """the calls of LENGTHS over pcm, issued as `issue` says, before(h, k) right before call k; the records of each"""
+    how = [issue[k % len(issue)] for k in range(len(LENGTHS))]
     bufs, pos = [], 0
-    for n in lengths:
-        bufs.append((nb.DeviceArray.from_host(np.ascontiguousarray(pcm[:, pos * 160:(pos + n) * 160])),
-                     nb.DeviceArray((S, n), nb.CASCADE_RESULT_DT)))
+    for k, n in enumerate(LENGTHS):                  # every buffer first: the calls then go back to back
+        part = np.ascontiguousarray(pcm[:, pos * 160:(pos + n) * 160])
+        if how[k] == "device":
+            bufs.append((nb.DeviceArray.from_host(part), nb.DeviceArray((S, n), nb.CASCADE_RESULT_DT)))
+        elif how[k] == "host":
+            bufs.append((nb.PinnedArray(part.shape, np.int16), nb.PinnedArray((S, n), nb.CASCADE_RESULT_DT)))
+            bufs[-1][0].array[...] = part
+        else:
+            bufs.append((part, None))
         pos += n
-    for (dp, dr), n in zip(bufs, lengths):
-        h.exec_device(dp, n * 160, n, dr)
+    out = [None] * len(LENGTHS)
+    for k, n in enumerate(LENGTHS):
+        if before:
+            before(h, k)
+        p, r = bufs[k]
+        if how[k] == "device":
+            h.exec_device(p, n * 160, n, r)
+        elif how[k] == "host":
+            h.exec_host_async(p.array, r.array)
+        else:
+            out[k] = h.exec(p, taps=True)[0]
     h.sync()
-    out = [dr.to_host() for _, dr in bufs]
-    for dp, dr in bufs:
-        dp.free(); dr.free()
+    for k, (p, r) in enumerate(bufs):
+        if how[k] != "tapped":
+            out[k] = r.to_host() if how[k] == "device" else r.array.copy()
+            p.free(); r.free()
     return out
 
 
+CASES = [pytest.param(issue, lb, id=lb if issue == "pipelined" else issue + "-" + lb) for issue in ISSUE for lb in sorted(LOOKBACK)]
+
+
 @pytest.mark.gpu
-@pytest.mark.parametrize("lookback", sorted(LOOKBACK))
-def test_pipelined_call_lengths_against_the_oracle(nb, oracle, lookback):
-    frames = sum(LENGTHS)
-    pcm = nb.synth_pcm(S, frames, first_stream=R.FIRST)
-    h = _handle(nb, "auto", LOOKBACK[lookback])
-    got = np.concatenate(_pipelined(nb, h, pcm, LENGTHS), axis=1)
+@pytest.mark.parametrize("issue,lookback", CASES)
+def test_pipelined_call_lengths_against_the_oracle(nb, oracle, issue, lookback):
+    pcm = nb.synth_pcm(S, sum(LENGTHS), first_stream=R.FIRST)
+    h = _handle(nb, "sequential" if issue == "sequential" else "auto", LOOKBACK[lookback])
+    got = _calls(nb, h, pcm, ISSUE[issue])
     h.close()
+    if issue != "pipelined":
+        ref = _handle(nb, "auto", LOOKBACK[lookback])
+        want = _calls(nb, ref, pcm, ISSUE["pipelined"])
+        ref.close()
+        for k, n in enumerate(LENGTHS):
+            assert got[k].tobytes() == want[k].tobytes(), "records of the %d-frame call %d differ from the pipelined device call's" % (n, k)
+    got = np.concatenate(got, axis=1)
     om = [oracle.model(i, False) for i in range(3)]
     par = R._params(oracle, nb, _params(LOOKBACK[lookback]))
-    for s in range(S):
+    for s in range(0, S, 7):
         want = oracle.cascade_run(om, pcm[s], params=par, taps=False)[0]
         for f in R.FIELDS:
             assert (got[s][f] == want[f]).all(), "field %s of stream %d differs from the oracle" % (f, s)
@@ -92,33 +125,29 @@ def test_records_match_the_sequential_path(nb, lookback):
     a.close(); b.close()
 
 
+def _resets_and_imports(recs):
+    def before(h, k):
+        if k == 3:
+            h.reset_streams([0, 5, 30, 100, 250])
+        if k == 5:
+            h.reset_streams([7, 8, 140], fresh=True)
+            h.import_streams([12, 2, 33, 201], recs)
+    return before
+
+
 @pytest.mark.gpu
 def test_resets_and_imports_between_pipelined_calls(nb):
-    frames = sum(LENGTHS)
-    pcm = nb.synth_pcm(S, frames, first_stream=R.FIRST)
+    pcm = nb.synth_pcm(S, sum(LENGTHS), first_stream=R.FIRST)
     donor = _handle(nb, "sequential", {})
     donor.exec(pcm[:, :150 * 160])
-    recs = donor.export_streams([3, 11, 20])
+    recs = donor.export_streams([3, 11, 20, 130])
     donor.close()
-    handles = [_handle(nb, "auto", {}), _handle(nb, "sequential", {})]
     results = []
-    for h in handles:
-        pos, out = 0, []
-        for k, n in enumerate(LENGTHS):
-            if k == 3:
-                h.reset_streams([0, 5, 30])
-            if k == 5:
-                h.reset_streams([7, 8], fresh=True)
-                h.import_streams([12, 2, 33], recs)
-            dp = nb.DeviceArray.from_host(np.ascontiguousarray(pcm[:, pos * 160:(pos + n) * 160]))
-            dr = nb.DeviceArray((S, n), nb.CASCADE_RESULT_DT)
-            h.exec_device(dp, n * 160, n, dr)
-            out.append((dp, dr))
-            pos += n
-        h.sync()
-        results.append(([dr.to_host().tobytes() for _, dr in out], h.export_streams(np.arange(S))))
-        for dp, dr in out:
-            dp.free(); dr.free()
+    for path, issue in (("auto", "pipelined"), ("sequential", "sequential"), ("auto", "host")):
+        h = _handle(nb, path, {})
+        out = _calls(nb, h, pcm, ISSUE[issue], _resets_and_imports(recs))
+        results.append(([r.tobytes() for r in out], h.export_streams(np.arange(S))))
         h.close()
-    assert results[0][0] == results[1][0]
-    assert results[0][1] == results[1][1]
+    for issue, (records, state) in zip(("sequential", "host"), results[1:]):
+        assert results[0][0] == records, "records of the %s calls differ from the pipelined ones" % issue
+        assert results[0][1] == state, "stream state after the %s calls differs from the pipelined one" % issue

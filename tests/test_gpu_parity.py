@@ -208,10 +208,12 @@ def test_back_to_back_calls_are_pipelined_correctly(nb, oracle):
 def test_async_host_calls_double_buffered(nb, oracle):
     """nnsp_b200_batch_exec_host_async / _wait_host: a server loop with two pinned PCM/result buffer pairs, one call in
     flight while the previous one is consumed; odd call lengths flip the stride-2 inference gate between calls; a
-    device-buffer call and a synchronous host call are mixed in behind the asynchronous ones."""
+    device-buffer call and a synchronous host call are mixed in behind the asynchronous ones, then 1-frame device-buffer
+    and host calls interleaved (each keeps one frame of the 2-frame PCM history the call before it wrote)."""
     S, n = 600, 7                                      # 600 streams -> 2 pipeline slices; 7 frames per call
     calls = 9
-    T = n * (calls + 2)
+    ones = (True, True, False, True, False, False)     # the 1-frame calls: device buffers (no sync between) or host
+    T = n * (calls + 2) + len(ones)
     pcm = nb.synth_pcm(S, T, first_stream=5)
     for nn_id in (1, 0):
         b = nb.NNSPBatch(_model(nb, nn_id, False), S)
@@ -230,7 +232,21 @@ def test_async_host_calls_double_buffered(nb, oracle):
         b.wait_host(1)                                 # an old ticket: already complete, returns at once
         got.append(pres[(calls - 1) & 1].array.copy())
         got.append(b.exec(pcm[:, calls * n * 160:(calls + 1) * n * 160].copy()))          # device-buffer call
-        got.append(b.exec_host(pcm[:, (calls + 1) * n * 160:].copy()))                    # synchronous host call
+        got.append(b.exec_host(pcm[:, (calls + 1) * n * 160:(calls + 2) * n * 160].copy()))   # synchronous host call
+        tail = []
+        for j, dev in enumerate(ones):
+            t = (calls + 2) * n + j
+            part = pcm[:, t * 160:(t + 1) * 160].copy()
+            if dev:
+                tail.append((nb.DeviceArray.from_host(part), nb.DeviceArray((S, 1), nb.RESULT_DT)))
+                b.exec_device(tail[-1][0], 160, 1, tail[-1][1])
+            else:
+                tail.append((None, b.exec_host(part)))
+        b.sync()
+        for dp, r in tail:
+            got.append(r if dp is None else r.to_host())
+            if dp is not None:
+                dp.free(); r.free()
         got = np.concatenate(got, axis=1)
         m_or = oracle.model(nn_id, False)
         for s in list(range(0, S, 37)) + [S - 1]:
